@@ -22,6 +22,9 @@ only collective is the all-reduce of the [9,9] i64 confusion matrix.
             events on its stream inside the timed steps; `kernels` lists every custom launch
     cpu_baseline / --impl reference   the reference's CPU path (oracle port: same per-class
             passes, band-merge loops, scikit-learn calls; torch CPU network) on the host cores
+
+--dump-outputs DIR writes what the last timed step returned as DIR/<name>.npy (see dump_outputs); the inputs
+and the network's weights are seeded, so two builds run with the same arguments can be compared array by array.
 """
 import argparse
 import concurrent.futures as cf
@@ -339,6 +342,33 @@ def roofline_of(kernels, peak, peak_kind, images_per_step, step_ms):
             "why_this_kernel": "the custom kernel with the largest share of the timed step; every custom launch of the step is listed under `kernels` with its own fraction"}
 
 
+LABEL_SAMPLE = 1 << 22      # label values --dump-outputs writes (16 MB as float32)
+
+
+def dump_outputs(out_dir, conf, conf_e2e, results, n_images):
+    """--dump-outputs: what the last timed step of each timed pass returned, as float arrays.
+        confusion.npy      [C,C] confusion matrix of the resident pass (all-reduced; counts are exact in float64)
+        confusion_e2e.npy  [C,C] the matrix run_host returned
+        labels.npy         [images, k] this rank's fitted-resolution label maps at k fixed positions
+        labels_index.npy   [k] those positions, flat indices into one [h,w] map, drawn with seed 0
+    The convolution routes and cuDNN engines are fixed per layer shape rather than timed (models/fused.py), so
+    repeated runs with the same arguments write the same arrays.
+    """
+    if len(results) != n_images:
+        raise SystemExit("bench.py: the last timed step returned %d per-image results for %d images" % (len(results), n_images))
+    maps = torch.stack([r["labels"] for r in results]).flatten(1)
+    n, hw = maps.shape
+    k = min(hw, max(1, LABEL_SAMPLE // n))
+    index = np.sort(np.random.default_rng(0).choice(hw, size=k, replace=False))
+    sample = maps[:, torch.from_numpy(index).to(maps.device)].cpu().numpy()
+    arrays = {"confusion": conf.astype(np.float64), "confusion_e2e": conf_e2e.astype(np.float64),
+              "labels": sample.astype(np.float32), "labels_index": index.astype(np.float64)}
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_ours(args, rank, world, local_rank):
     from pylc_b200 import _lib, ops
     from pylc_b200 import dist as pdist
@@ -349,7 +379,8 @@ def run_ours(args, rank, world, local_rank):
     device = torch.device("cuda", local_rank)
     torch.cuda.set_device(device)
     _lib.load()
-    torch.backends.cudnn.benchmark = True
+    # cuDNN's heuristic engines, not timed ones: a timed choice can differ between runs, and with it the TF32 sums
+    torch.backends.cudnn.benchmark = False
     dtype = {"fp32": None, "bf16": torch.bfloat16, "fp16": torch.float16}[args.backbone_dtype]
 
     model = build_model(device)
@@ -377,6 +408,7 @@ def run_ours(args, rank, world, local_rank):
     h2d = sum(im.numel() + gt.numel() for im, gt in zip(imgs, masks)) if seg.can_fit_on_device(imgs[0]) \
         else sum(f.img.numel() + f.gt.numel() for f in resident)      # bytes run_host copies per step
     clocks = ClockSampler(local_rank)
+    last_results = []
     with KernelTimer(ops) as st:
         for _ in range(args.warmup):
             seg.reset()
@@ -388,9 +420,9 @@ def run_ours(args, rank, world, local_rank):
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         torch.cuda.profiler.start()     # no-op unless run under `ncu --profile-from-start off` (tools/gpu_profile.sh)
         ev0.record()
-        for _ in range(args.steps):
+        for step in range(args.steps):
             seg.reset()
-            seg.run_resident(resident)
+            seg.run_resident(resident, results=last_results if args.dump_outputs and step == args.steps - 1 else None)
             conf_dev = pdist.all_reduce_(seg.conf.clone()) if world > 1 else seg.conf
         ev1.record()
         barrier_sync()
@@ -449,6 +481,8 @@ def run_ours(args, rank, world, local_rank):
     }
     if world == 1 and not args.no_cpu_baseline:
         line["cpu_baseline"] = cpu_baseline()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, conf_resident, conf_host, last_results, n_mine)
     print(json.dumps(line), flush=True)
     if not line["config"]["resident_equals_e2e"]:
         # both paths process the same images with ONE coverage injection (global image 0): the integer
@@ -478,7 +512,13 @@ def main():
                     "colour 3000x2000 set the metric is quoted on (default, what the driver runs); 4 = gray 6000x4000")
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"], help="weak: --images per GPU (default); "
                     "strong: ONE set of --images dealt round-robin over the ranks")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="after the timed steps, write what the last "
+                    "timed step returned to DIR/<name>.npy (float32 / float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     cfg = CONFIGS[args.config]
     n_img = cfg["n"] if args.images is None else args.images
     globals().update(N_IMAGES=n_img, W_FULL=cfg["w"], H_FULL=cfg["h"], CH=cfg["ch"], TILES_PER_IMAGE=cfg["tiles"],

@@ -1,8 +1,8 @@
 """TEST INFRASTRUCTURE ONLY.  Regenerates every golden fixture from the imported reference into a scratch directory
 (oracle/gen_golden.py, unchanged) and compares it, array by array, with the committed tests/golden/*.npz.
-Build container only (needs /root/reference):
+Needs a checkout of the reference:
 
-    python oracle/check_golden.py        # prints one line per fixture, exits non-zero on any difference
+    PYLC_REFERENCE_ROOT=<PyLC checkout> python oracle/check_golden.py   # one line per fixture, non-zero exit on any difference
 """
 import os
 import sys

@@ -1,13 +1,14 @@
 """
 TEST INFRASTRUCTURE ONLY.  Generates tests/golden/*.npz by executing the UNMODIFIED PyLC
-reference (/root/reference) on small seeded inputs.  The reference cannot travel to the GPU
-box, so the vectors are committed; re-run with
+reference on small seeded inputs.  The reference is not part of this repository, so the vectors
+are committed; regenerate them with
 
-    python oracle/gen_golden.py
+    PYLC_REFERENCE_ROOT=<PyLC checkout> python oracle/gen_golden.py
 
-in the build container to regenerate them.  Tile size 32 / stride 16 keep the fixtures small;
-the reference code paths exercised are size-independent.
+Tile size 32 / stride 16 keep the fixtures small; the reference code paths exercised are
+size-independent.  Every fixture file stays under 1 MB.
 """
+import hashlib
 import json
 import os
 import sys
@@ -187,7 +188,7 @@ def gen_reconstruct(ref, out):
             rgb = ref.tools.reconstruct(batches, meta)
         finally:
             np.argmax = real_argmax
-        out["recon_%s_tiles" % name] = tiles
+        out["recon_%s_tiles_sha256" % name] = np.array(hashlib.sha256(tiles.tobytes()).hexdigest())   # see orc.reconstruct_fixture_tiles
         out["recon_%s_geom" % name] = np.array([nr, nc, T, S, h, w, w_full, h_full, C])
         out["recon_%s_map" % name] = captured["map"][0]
         out["recon_%s_rgb" % name] = rgb

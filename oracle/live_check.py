@@ -1,14 +1,15 @@
 """TEST INFRASTRUCTURE ONLY -- live comparison of the oracle with the unmodified reference.
 
 Runs in its own process (the harness changes the working directory and puts the reference's flat module
-names -- config, utils, db, models -- at the front of sys.path): imports /root/reference through
-oracle/ref_harness.py and checks every restatement in oracle/pylc_oracle.py against the reference function
-it cites, on seeded inputs that are NOT the ones frozen in tests/golden/ (other seeds, other sizes).
+names -- config, utils, db, models -- at the front of sys.path): imports the reference checkout named by
+PYLC_REFERENCE_ROOT through oracle/ref_harness.py and checks every restatement in oracle/pylc_oracle.py against
+the reference function it cites, on seeded inputs that are NOT the ones frozen in tests/golden/ (other seeds,
+other sizes).
 
-    python oracle/live_check.py [--seed N]      exit code 0 = all equal, 1 = mismatch, 77 = reference absent
+    PYLC_REFERENCE_ROOT=<PyLC checkout> python oracle/live_check.py [--seed N]
+                                                exit code 0 = all equal, 1 = mismatch, 77 = reference absent
 
-Only tests/test_oracle_vs_reference.py runs it; it exists in the build container only (the GPU box has no
-/root/reference).
+tests/test_oracle_vs_reference.py runs it.
 """
 import argparse
 import os

@@ -17,8 +17,9 @@ exist for the expensive ones:
 Parity pinning: the reference ships no tests or golden vectors (SURVEY.md section 4).  The oracle
 is pinned instead against outputs of the unmodified reference executed in the build container
 (oracle/gen_golden.py -> tests/golden/*.npz; tests/test_oracle_golden.py) and, when
-/root/reference is present, live (tests/test_oracle_vs_reference.py).
+PYLC_REFERENCE_ROOT names a reference checkout, live (tests/test_oracle_vs_reference.py).
 """
+import hashlib
 import math
 
 import numpy as np
@@ -676,6 +677,21 @@ def augment_fixture_tile(ch, T=512):
     img = np.stack([(xx // 7 * 5 + yy // 11 * 3 + 40 * c) % 256 for c in range(ch)]).astype(np.uint8)[None]
     mask = ((xx // 60 + yy // 45) % 9).astype(np.uint8)[None]
     return img, mask
+
+
+def reconstruct_fixture_tiles(fixture, case):
+    """Logit tiles of one case of tests/golden/reconstruct.npz.  gen_golden.py draws them case after case from one
+    generator (seed 15); random floats do not compress, so the file keeps only the SHA-256 of each case's tiles and
+    the draw is repeated here and checked against it."""
+    rng = np.random.default_rng(15)
+    for name in (str(c) for c in fixture["recon_cases"]):
+        nr, nc, T, S, h, w, w_full, h_full, C = (int(v) for v in fixture["recon_%s_geom" % name])
+        tiles = (rng.standard_normal((nr * nc, C, T, T)) * 3).astype(np.float32)
+        if name == case:
+            digest = hashlib.sha256(tiles.tobytes()).hexdigest()
+            assert digest == str(fixture["recon_%s_tiles_sha256" % name]), "regenerated tiles differ from the fixture's"
+            return tiles
+    raise KeyError(case)
 
 
 # ---------------------------------------------------------------------------------------------

@@ -1,12 +1,13 @@
 """
 TEST INFRASTRUCTURE ONLY -- never imported by the product (pylc_b200/).
 
-Harness that imports the *unmodified* PyLC reference from /root/reference so that
+Harness that imports the *unmodified* PyLC reference from the checkout named by the
+PYLC_REFERENCE_ROOT environment variable (default: oracle/_ref/, ignored by git) so that
 (a) the oracle restatements in oracle/pylc_oracle.py can be validated against it and
 (b) golden input/output vectors can be generated (oracle/gen_golden.py -> tests/golden/).
 
-The reference only exists in the build container (it is not shipped to the GPU box), so
-everything here is guarded by `available()`.
+The reference is not part of this repository, so everything here is guarded by `available()`;
+without it the committed golden vectors carry the pinning.
 
 Recipe (SURVEY.md Appendix B):
   * stub modules for h5py / seaborn / matplotlib (import-only dependencies of
@@ -22,7 +23,7 @@ import sys
 import tempfile
 import types
 
-REF_ROOT = os.environ.get("PYLC_REFERENCE_ROOT", "/root/reference")
+REF_ROOT = os.environ.get("PYLC_REFERENCE_ROOT", os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref"))
 
 _state = {"loaded": False, "workdir": None}
 

@@ -23,8 +23,6 @@ state_dict.  Outputs match `net.eval()(x)` to fp32 rounding of the folded weight
 bit, so the pipeline uses it only when asked (`TiledSegmenter(fuse_network=True)`); parity tests of
 the custom kernels never depend on it.
 """
-import os
-
 import torch
 import torch.nn as nn
 import torch.nn.functional as F
@@ -44,9 +42,10 @@ def fold_conv_bn(conv, bn):
     return w.float(), b.float()
 
 
-# Per layer and input shape, the plan times its library routes once and keeps the fastest:
+# Library routes of a convolution with a ReLU; the plan picks one from the layer's geometry (`_Conv._route`):
 #   0  torch.cudnn_convolution_relu / _add_relu: one fused cuDNN call, engine chosen by cuDNN's heuristic
-#   1  F.conv2d (engine chosen by torch.backends.cudnn.benchmark when that is on) + in-place add / ReLU
+#   1  F.conv2d (engine chosen by torch.backends.cudnn.benchmark when that is on) + in-place add / ReLU: only the
+#      convolutions without a ReLU (`_Conv._plain`)
 #   2  tap split (3x3, stride 1, padding == dilation >= 6 only): the convolution as nine cuBLAS GEMMs over the flat
 #      pixel ranges that do not fall into the zero padding, summed by pylc_tap_combine_relu_f32 (`_Conv._tap_split`)
 # Measured on B200 (tools/exp/dilated_conv.py, 45 tiles): cuDNN has an sm100 kernel for the ASPP branches with
@@ -55,19 +54,20 @@ def fold_conv_bn(conv, bn):
 # (0.2 ms): 10 % of the whole network.  With dilation 18 > 32 / 2 every output pixel sees at most two taps per
 # axis, i.e. 39 % of the dense products; route 2 computes 62 % (whole flat runs, so that no window is ever copied),
 # on the TF32 tensor cores through cuBLAS.
-AUTOTUNE = os.environ.get("PYLC_CONV_AUTOTUNE", "1") != "0"
+# The route is fixed by geometry, not timed at run time: where two routes take about as long, timing picks
+# differently from process to process, their TF32 sums round differently, and so the same input would give
+# different near-tied labels from run to run.
 
 
 class _Conv(object):
     """One folded convolution with an optional fused ReLU / residual add."""
-    __slots__ = ("w", "b", "stride", "padding", "dilation", "relu", "choice", "taps")
+    __slots__ = ("w", "b", "stride", "padding", "dilation", "relu", "taps")
 
     def __init__(self, conv, bn, relu, channels_last):
         w, b = fold_conv_bn(conv, bn)
         self.w = w.contiguous(memory_format=torch.channels_last) if channels_last else w.contiguous()
         self.b = b.contiguous()
         self.stride, self.padding, self.dilation, self.relu = conv.stride, conv.padding, conv.dilation, relu
-        self.choice = {}
         self.taps = None
 
     def to(self, dtype):
@@ -132,36 +132,17 @@ class _Conv(object):
             y.add_(residual)
         return y.relu_() if self.relu else y
 
-    def _pick(self, x, residual):
-        """Time both routes on this very input (CUDA events, after a warm-up each)."""
-        best, best_ms = 0, None
-        routes = (self._fused, self._plain) + ((self._tap_split,) if self._tap_split_applies(x, residual) else ())
-        for route, fn in enumerate(routes):
-            try:
-                for _ in range(2):
-                    fn(x, residual)
-                e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                e0.record()
-                for _ in range(3):
-                    fn(x, residual)
-                e1.record()
-                e1.synchronize()
-                ms = e0.elapsed_time(e1)
-            except RuntimeError:
-                continue
-            if best_ms is None or ms < 0.97 * best_ms:      # the fused call keeps ties
-                best, best_ms = route, ms
-        return best
+    def _route(self, x, residual):
+        """Route 2 (tap split) where the dilation exceeds half the map, so that at most two taps per axis reach any
+        output pixel and cuDNN's dense kernel would do more than twice the products (dilation 18 on the 32 x 32
+        ASPP input); route 0 (one fused cuDNN call) everywhere else."""
+        if self._tap_split_applies(x, residual) and 2 * self.dilation[0] > min(x.shape[2], x.shape[3]):
+            return self._tap_split
+        return self._fused
 
     def __call__(self, x, residual=None):
         if x.is_cuda and self.relu:
-            if not AUTOTUNE:
-                return self._fused(x, residual)
-            key = (tuple(x.shape), x.dtype, residual is not None)
-            route = self.choice.get(key)
-            if route is None:
-                route = self.choice[key] = self._pick(x, residual)
-            return (self._fused, self._plain, self._tap_split)[route](x, residual)
+            return self._route(x, residual)(x, residual)
         return self._plain(x, residual)
 
 
@@ -228,7 +209,7 @@ class FusedDeepLab(object):
                 w4[:, (py * 2 + px) * 3:(py * 2 + px) * 3 + 3] = w8[:, :, py::2, px::2]
         s = _Conv.__new__(_Conv)
         s.w = w4.contiguous(memory_format=torch.channels_last)
-        s.b, s.stride, s.padding, s.dilation, s.relu, s.choice = stem.b, (1, 1), (0, 0), (1, 1), True, {}
+        s.b, s.stride, s.padding, s.dilation, s.relu, s.taps = stem.b, (1, 1), (0, 0), (1, 1), True, None
         return s
 
     def _aspp_out_folded(self, cat4, pooled):

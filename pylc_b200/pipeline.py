@@ -199,11 +199,14 @@ class TiledSegmenter(object):
     def reset(self):
         self.conf.zero_()
 
-    def run_resident(self, fitted_images):
-        """Device-only pass over images already staged in HBM (bench.py `value`)."""
+    def run_resident(self, fitted_images, results=None):
+        """Device-only pass over images already staged in HBM (bench.py `value`).  Returns the last image's
+        result; `results`, when given, is a list that receives every image's result in order."""
         out = None
         for f in fitted_images:
             out = self.segment_fitted(f, inject=self.n_inject if f.index == 0 else 0)
+            if results is not None:
+                results.append(out)
         return out
 
     def run_host(self, images, masks=None, indices=None, distributed=False, global_offset=None, global_indices=None):

@@ -31,7 +31,7 @@ def _cli(cwd, *argv):
     return out.stdout
 
 
-def test_cli_extract_profile_test_on_files(tmp_path, palettes):
+def test_cli_extract_profile_test_on_files(tmp_path, palettes, monkeypatch):
     pal = palettes["a"]
     C = len(pal)
     W, H = 2000, 1500
@@ -107,6 +107,7 @@ def test_cli_extract_profile_test_on_files(tmp_path, palettes):
     assert np.array_equal(np.load(cm[0]), want["cmatrix"])
     # and the label map itself is the reference's reconstruct of THIS network's logits (near-ties aside)
     from pylc_b200.models.model import Model
+    monkeypatch.chdir(tmp_path)                                        # Model creates ./data/save/<id>, as the CLI did
     model = Model().load(model_file)
     model.net.eval()                                                   # test.py:41
     fitted = cv2.resize(img, (w_fit, h_fit), interpolation=cv2.INTER_AREA)

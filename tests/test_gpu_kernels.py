@@ -386,7 +386,7 @@ def test_stitch_golden(ops, golden, palettes, case):
     g = golden("reconstruct")
     nr, nc, T, S, h, w, w_full, h_full, C = [int(v) for v in g["recon_%s_geom" % case]]
     pal = palettes["b" if case.startswith("b") else "a"]
-    tiles = g["recon_%s_tiles" % case]
+    tiles = orc.reconstruct_fixture_tiles(g, case)
     check_stitch(ops, tiles, nr, nc, T, S, pal, ref_map=g["recon_%s_map" % case])
     check_stitch(ops, tiles, nr, nc, T, S, pal, ref_map=g["recon_%s_map" % case], batches=4)
     # end of tools.reconstruct: NN-resample to (w_full, h_full) and colourise == reference RGB
@@ -926,7 +926,7 @@ def test_tap_split_route_equals_cudnn_convolution(ops, H, W, d, cin, cout, B):
     err_split, err_cudnn = float((got - exact).abs().max()), float((want - exact).abs().max())
     assert err_split <= 3e-3 * scale                       # TF32 inputs (10-bit mantissa), fp32 accumulation
     assert err_split <= 4 * err_cudnn + 1e-6 * scale       # no worse than the library convolution it replaces
-    # and the plan's autotuned call returns the same thing whichever route it keeps
+    # and the plan's call returns the same thing whichever route its geometry rule picks
     y = c(x)
     assert float((y - exact).abs().max()) <= 3e-3 * scale
 

@@ -271,14 +271,28 @@ def test_cli_parser_accepts_reference_command_lines():
         p.parse_args("extract --ch 2 --img x".split())                    # ch in {1, 3}
 
 
+def _live_golden():
+    """What the *_live tests compare, recorded by oracle/gen_live_golden.py."""
+    with open(os.path.join(ROOT, "tests", "golden", "host_live.json")) as f:
+        return json.load(f)
+
+
 def test_cli_parser_covers_reference_options_live():
-    """In the build container: every option of the reference's extract / augment / train / test sub-parsers exists here
-    with the same destination and choices (merge / grayscale are stubs in the reference and are not provided)."""
+    """Every option of the reference's extract / augment / train / test sub-parsers exists here with the same destination
+    and choices: against tests/golden/host_live.json, and against the reference's parser when it is present (merge /
+    grayscale are stubs in the reference and are not provided)."""
     import argparse
     import importlib
     import ref_harness
+    import host_record as hr
+    from pylc_b200.pylc import get_parser as our_parser
+    stored, ours_rec = _live_golden()["parser"], hr.record_parser(our_parser())      # tests/golden/host_live.json
+    assert set(stored["commands"]) <= set(ours_rec["commands"])
+    for cmd in ("extract", "augment", "train", "test"):
+        for opts, want in stored[cmd].items():
+            assert ours_rec[cmd].get(opts) == want, (cmd, opts)
     if not ref_harness.available():
-        pytest.skip("reference not present (GPU box)")
+        return
     ref_harness.load()
     sys.path.insert(0, ref_harness.REF_ROOT)
     try:
@@ -305,14 +319,19 @@ def test_cli_parser_covers_reference_options_live():
 
 
 def test_python_surface_covers_reference_live():
-    """SURVEY.md section 8b in the build container: every public method of the reference's path classes and every
+    """SURVEY.md section 8b, against tests/golden/host_live.json and, when present, the reference: every public method of the reference's path classes and every
     function of its path modules exists here under the same module path and name, with the reference's leading
     parameters (extra trailing parameters with defaults are extensions).  Omissions are listed, with the reason."""
     import importlib
     import inspect
     import ref_harness
+    import host_record as hr
+    stored, ours_rec = _live_golden()["surface"], hr.record_surface(hr.package_modules())   # tests/golden/host_live.json
+    for owner, members in stored.items():
+        for n, params in members.items():
+            assert n in ours_rec[owner] and ours_rec[owner][n][:len(params)] == params, (owner, n)
     if not ref_harness.available():
-        pytest.skip("reference not present (GPU box)")
+        return
     ref_harness.load()
     omitted = {
         ("Evaluator", "save_tex"): "LaTeX table helper (analysis, SURVEY.md section 2: out of scope)",
@@ -363,8 +382,11 @@ def test_parameters_table_equals_reference_live(schema):
     checkpoint.py:53-66): attribute names and default values must be the reference's, key for key."""
     import importlib
     import ref_harness
+    import host_record as hr
+    from pylc_b200.config import Parameters as OurParameters
+    assert hr.record_parameters(OurParameters, schema) == _live_golden()["parameters"][schema]   # tests/golden/host_live.json
     if not ref_harness.available():
-        pytest.skip("reference not present (GPU box)")
+        return
     ref_harness.load()
     sys.path.insert(0, ref_harness.REF_ROOT)
     try:

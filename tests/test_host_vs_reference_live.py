@@ -1,9 +1,8 @@
-"""Build-container only: the host-side helpers of the path (decode, file collation, fit, shuffles, C-vector
-statistics) executed side by side with the unmodified reference on the same files and
-arrays.  Skipped where /root/reference is absent (the GPU box); the committed golden vectors cover that side."""
-import contextlib
+"""The host-side helpers of the path (decode, file collation, fit, shuffles, C-vector statistics) on the same files and
+arrays as the unmodified reference: against the record in tests/golden/host_live.json (oracle/gen_live_golden.py), and
+side by side with the reference itself when PYLC_REFERENCE_ROOT names a PyLC checkout."""
 import importlib
-import io
+import json
 import os
 import sys
 
@@ -11,14 +10,17 @@ import cv2
 import numpy as np
 import pytest
 
-import pylc_oracle as orc
+import host_record as hr
 import ref_harness
 
-pytestmark = pytest.mark.skipif(not ref_harness.available(), reason="reference not present (GPU box)")
+GOLDEN = json.load(open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "host_live.json")))
+PACKAGE = hr.package_modules()
 
 
 @pytest.fixture(scope="module")
 def ref():
+    if not ref_harness.available():
+        return None
     ref_harness.load()
     sys.path.insert(0, ref_harness.REF_ROOT)
     try:
@@ -29,38 +31,20 @@ def ref():
     return type("Ref", (), mods)
 
 
-def run(fn, *a, **k):
-    """(outcome, value, printed text): the reference signals errors with print + exit(1)."""
-    buf = io.StringIO()
-    try:
-        with contextlib.redirect_stdout(buf):
-            val = fn(*a, **k)
-        return "ok", val, buf.getvalue()
-    except SystemExit as e:
-        return "exit", e.code, buf.getvalue()
-    except AssertionError:
-        return "assert", None, buf.getvalue()
-
-
 @pytest.fixture(scope="module")
 def files(tmp_path_factory, palettes):
     d = tmp_path_factory.mktemp("live")
-    os.makedirs(d / "img")
-    os.makedirs(d / "mask")
-    os.makedirs(d / "odd")
-    pal = palettes["a"]
-    for i, (name, ext) in enumerate([("a", ".tif"), ("b", ".png"), ("c", ".jpg")]):
-        assert cv2.imwrite(str(d / "img" / (name + ext)), orc.synth_image(i, 300, 200, 3)[..., ::-1])
-        assert cv2.imwrite(str(d / "mask" / (name + ".png")), np.ascontiguousarray(orc.synth_mask(i, 300, 200, pal)[..., ::-1]))
-    (d / "img" / "notes.txt").write_text("not an image")
-    assert cv2.imwrite(str(d / "odd" / "only.png"), orc.synth_image(5, 64, 64, 3))
-    assert cv2.imwrite(str(d / "gray.tif"), orc.synth_image(9, 300, 200, 1))
+    hr.make_files(str(d), palettes["a"])
     return d
 
 
 def test_collate_and_load_files(ref, files):
     from pylc_b200.utils import tools
     d = str(files)
+    assert hr.record_file_lists(PACKAGE, d) == GOLDEN["files"]
+    if ref is None:
+        return
+    run = hr.run
     for args in ((d + "/img", d + "/mask"), (d + "/img",), (d + "/img/a.tif", d + "/mask/a.png"),
                  (d + "/img", d + "/odd"), (d + "/missing",)):
         want, got = run(ref.tools.collate, *args), run(tools.collate, *args)
@@ -70,18 +54,17 @@ def test_collate_and_load_files(ref, files):
         assert ref.tools.get_fname(p) == tools.get_fname(p)
 
 
-@pytest.mark.parametrize("name,ch,scale,interp", [
-    ("img/a.tif", 3, None, cv2.INTER_AREA), ("img/b.png", 3, 0.5, cv2.INTER_AREA), ("img/c.jpg", 3, None, cv2.INTER_AREA),
-    ("mask/a.png", 3, 0.4, cv2.INTER_NEAREST), ("gray.tif", 1, None, cv2.INTER_AREA), ("gray.tif", 1, 0.7, cv2.INTER_AREA),
-    ("gray.tif", 3, None, cv2.INTER_AREA),      # a gray file asked for as colour: print + exit(1) in both
-    ("img/a.tif", 1, None, cv2.INTER_AREA),     # a colour file asked for as gray (the reference prompts; stdin is empty)
-])
+@pytest.mark.parametrize("name,ch,scale,interp", hr.GET_IMAGE_CASES)
 def test_get_image(ref, files, name, ch, scale, interp, monkeypatch):
     from pylc_b200.utils import tools
+    case = (name, ch, scale, interp)
+    assert hr.record_get_image(PACKAGE, str(files), case) == GOLDEN["get_image"][hr.get_image_key(case)]
+    if ref is None:
+        return
     monkeypatch.setattr("builtins.input", lambda *a: "y")
     path = str(files / name)
-    want = run(ref.tools.get_image, path, ch, scale=scale, interpolate=interp)
-    got = run(tools.get_image, path, ch, scale=scale, interpolate=interp)
+    want = hr.run(ref.tools.get_image, path, ch, scale=scale, interpolate=getattr(cv2, interp))
+    got = hr.run(tools.get_image, path, ch, scale=scale, interpolate=getattr(cv2, interp))
     assert want[0] == got[0]
     if want[0] == "ok":
         assert np.array_equal(want[1][0], got[1][0]) and tuple(want[1][1:]) == tuple(got[1][1:])
@@ -89,6 +72,10 @@ def test_get_image(ref, files, name, ch, scale, interp, monkeypatch):
 
 def test_adjust_to_tile_coshuffle_and_statistics(ref):
     from pylc_b200.utils import metrics, tools
+    assert hr.record_helpers(PACKAGE) == GOLDEN["helpers"]
+    if ref is None:
+        return
+    import pylc_oracle as orc
     for seed, (w, h, ch) in enumerate([(700, 500, 1), (650, 430, 3), (512, 512, 1)]):
         img = orc.synth_image(seed, w, h, ch)
         want, got = ref.tools.adjust_to_tile(img, 128, 64, ch), tools.adjust_to_tile(img, 128, 64, ch)

@@ -115,7 +115,7 @@ def test_reconstruct(golden, palettes, case):
     g = golden("reconstruct")
     nr, nc, T, S, h, w, w_full, h_full, C = [int(v) for v in g["recon_%s_geom" % case]]
     pal = palettes["b" if case.startswith("b") else "a"]
-    tiles = g["recon_%s_tiles" % case]
+    tiles = orc.reconstruct_fixture_tiles(g, case)
     ref_map = g["recon_%s_map" % case]
     assert orc.stitch_grid(h, w, T, S) == (nr, nc)
     # the step-by-step port is bit-equal to the reference
