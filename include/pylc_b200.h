@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define PYLC_ABI_VERSION 2
+#define PYLC_ABI_VERSION 3
 #define PYLC_MAX_CLASSES 32
 
 #define PYLC_OK 0
@@ -288,6 +288,27 @@ PYLC_API int pylc_stitch_upsample_argmax_colour(const float *const *decoder_batc
 PYLC_API int pylc_colourise_u8(const uint8_t *labels, int64_t n_px, const uint8_t *lut_rgb, int C,
                       uint8_t *rgb, pylc_stream_t stream);
 
+/*
+ * Per-pixel class probabilities and confidence from the same stitch (an extension: the reference never forms a
+ * clean probability map).  P(y, x) is the mean, over the 1, 2 or 4 tiles covering the pixel, of softmax_c of
+ * that tile's logits.  On edge blocks it is exactly the reference's merged map M; on corners (and everywhere
+ * when S == T) the softmax of the raw logits; in the interior the mean of the four softmaxes.
+ *   mode          PYLC_STITCH_REFERENCE: labels / rgb / stitched are those of pylc_stitch_argmax_colour (first
+ *                 argmax of M, stitched = M), bit for bit.
+ *                 PYLC_STITCH_MEAN: labels = first argmax of P, stitched = P.
+ *   confidence    nullable [h, w] u8, q = min(255, round-to-nearest(P[label] * 255)); the same P in both modes
+ * Other arguments as pylc_stitch_argmax_colour / pylc_stitch_upsample_argmax_colour (the fused form also
+ * returns PYLC_ERR_ALIGN for an odd `confidence` address).  An unknown mode is PYLC_ERR_ARG.
+ */
+#define PYLC_STITCH_REFERENCE 0
+#define PYLC_STITCH_MEAN 1
+PYLC_API int pylc_stitch_probs(const float *logits, const float *const *tile_batches, int tiles_per_batch,
+                      int nr, int nc, int C, int T, int S, int mode, const uint8_t *lut_rgb,
+                      uint8_t *labels, uint8_t *rgb, uint8_t *confidence, float *stitched, pylc_stream_t stream);
+PYLC_API int pylc_stitch_upsample_probs(const float *const *decoder_batches, int tiles_per_batch, int nr, int nc,
+                               int C, int T, int S, int hs, int ws, int mode, const uint8_t *lut_rgb,
+                               uint8_t *labels, uint8_t *rgb, uint8_t *confidence, float *stitched, pylc_stream_t stream);
+
 /* ---- evaluation --------------------------------------------------------------------------- */
 
 /*
@@ -317,6 +338,23 @@ PYLC_API int pylc_resample_encode_confusion(const uint8_t *labels, int h, int w,
 /* Confusion matrix of two flat u8 label vectors (aggregate mode, utils/evaluate.py:158-174). */
 PYLC_API int pylc_confusion_u8(const uint8_t *y_true, const uint8_t *y_pred, int64_t n, int C, int n_inject,
                       int64_t *conf, pylc_stream_t stream);
+
+/*
+ * Nearest-neighbour resample of the fitted confidence plane (pylc_stitch_probs) with the label map's OpenCV
+ * index maps, and the reliability table of a calibration figure.
+ *   confidence       [h, w] u8 fitted-resolution confidence
+ *   x_ofs / y_ofs    as pylc_resample_encode_confusion
+ *   y_pred_full / y_true_full  nullable [h_full, w_full] u8 predicted / true classes (pred_full / gt_full of
+ *                    pylc_resample_encode_confusion); pixels whose class is >= C are not counted
+ *   confidence_full  nullable [h_full, w_full] u8
+ *   reliability      nullable [C, 256, 2] i64, ADDED INTO: [pred][q][pred == true] += 1 per full-resolution pixel
+ *                    (no coverage injection).  Needs both label planes, else PYLC_ERR_ARG.
+ * Any width and any alignment; rows are dense (pitch = w_full).
+ */
+PYLC_API int pylc_confidence_resample(const uint8_t *confidence, int h, int w, const int32_t *x_ofs,
+                             const int32_t *y_ofs, int h_full, int w_full, const uint8_t *y_pred_full,
+                             const uint8_t *y_true_full, int C, uint8_t *confidence_full, int64_t *reliability,
+                             pylc_stream_t stream);
 
 /* ---- multi-loss --------------------------------------------------------------------------- */
 

@@ -15,7 +15,7 @@ LIB_PATH = os.path.join(_HERE, "lib", "libpylc_b200.so")
 
 MAX_CLASSES = 32
 AREA_TAPS = 6
-ABI_VERSION = 2
+ABI_VERSION = 3
 
 
 class PylcError(RuntimeError):
@@ -69,10 +69,15 @@ SIGNATURES = {
     "pylc_stitch_upsample_argmax_colour": (c_int, [_ptr, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
                                                    POINTER(c_uint8), _u8p, _u8p, _ptr, _ptr]),
     "pylc_colourise_u8": (c_int, [_u8p, c_int64, POINTER(c_uint8), c_int, _u8p, _ptr]),
+    "pylc_stitch_probs": (c_int, [_ptr, _ptr, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
+                                  POINTER(c_uint8), _u8p, _u8p, _u8p, _ptr, _ptr]),
+    "pylc_stitch_upsample_probs": (c_int, [_ptr, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
+                                           POINTER(c_uint8), _u8p, _u8p, _u8p, _ptr, _ptr]),
     "pylc_resample_encode_confusion": (c_int, [_u8p, c_int, c_int, _ptr, _ptr, c_int, c_int, _u8p, c_size_t,
                                                POINTER(c_uint8), POINTER(c_uint8), c_int, c_int, _ptr,
                                                _u8p, _u8p, _u8p, _ptr]),
     "pylc_confusion_u8": (c_int, [_u8p, _u8p, c_int64, c_int, c_int, _ptr, _ptr]),
+    "pylc_confidence_resample": (c_int, [_u8p, c_int, c_int, _ptr, _ptr, c_int, c_int, _u8p, _u8p, c_int, _u8p, _ptr, _ptr]),
     "pylc_multiloss_reduce": (c_int, [_ptr, _ptr, c_int, c_int, c_int, c_int64, _ptr, POINTER(LossCfg),
                                       _ptr, _u8p, _ptr]),
     "pylc_multiloss_finalize": (c_int, [_ptr, c_int, c_int64, POINTER(LossCfg), _ptr, _ptr]),

@@ -9,6 +9,13 @@
 //   so corners are raw logits, edges one softmax-average, the interior a double softmax.
 // Every logit is read exactly once; a CTA owns a slab of rows of one block, so the block kind
 // (how many tiles feed it) is uniform per CTA and there is no divergence.
+//
+// Probabilities (pylc_stitch_probs): P(y, x) = the mean over the covering tiles of their softmaxes.  In the
+// terms above it is softmax(L) on corners (and everywhere when S == T), exactly M on edges, and the sum of
+// the two strip sums x 1/4 in the interior, taken before the second softmax.  MODE selects the labels:
+// PYLC_STITCH_REFERENCE (0) takes the first argmax of M (the reference's labels), PYLC_STITCH_MEAN (1) that
+// of P, and then `stitched` holds P instead of M.  CONF adds the u8 plane q = min(255, rn(P[label] * 255)).
+// MODE = 0 without CONF is the code the argmax / colour entry points have always run.
 #include "common.cuh"
 
 namespace pylc {
@@ -106,30 +113,44 @@ __device__ __forceinline__ void load_cls(const float *p, size_t cstride, int C, 
         if (c < C) Vec<PX>::load(p + c * cstride, v[c]);
 }
 
-// Writes one unit: optional f32 map, first-maximum argmax (np.argmax), label bytes, optional RGB.
-template <int CMAX, int PX>
-__device__ __forceinline__ void emit_unit(const StitchArgs &a, const uint32_t *s_lut, int C, const float (&m)[CMAX][PX], size_t o) {
+// Writes one unit: optional f32 map, first-maximum argmax (np.argmax), label bytes, optional RGB and, with
+// CONF, the confidence byte of P at the label.
+template <int CMAX, int PX, bool CONF = false>
+__device__ __forceinline__ void emit_unit(const StitchArgs &a, const uint32_t *s_lut, int C, const float (&m)[CMAX][PX],
+                                          const float (&p)[CMAX][PX], uint8_t *conf, size_t o) {
     if (a.stitched) {
 #pragma unroll
         for (int c = 0; c < CMAX; ++c)
             if (c < C) Vec<PX>::store(a.stitched + (size_t)c * a.h * a.w + o, m[c]);
     }
     uint32_t lab[PX];
+    float pl[PX];
 #pragma unroll
     for (int j = 0; j < PX; ++j) {
         float best = m[0][j];
         uint32_t bi = 0;
+        if constexpr (CONF) pl[j] = p[0][j];
 #pragma unroll
         for (int c = 1; c < CMAX; ++c)
             if (c < C && m[c][j] > best) {  // strict: first maximum wins (np.argmax)
                 best = m[c][j];
                 bi = c;
+                if constexpr (CONF) pl[j] = p[c][j];
             }
         lab[j] = bi;
     }
     if (a.labels) {
         if (PX == 2) *reinterpret_cast<uint16_t *>(a.labels + o) = (uint16_t)(lab[0] | (lab[PX - 1] << 8));
         else a.labels[o] = (uint8_t)lab[0];
+    }
+    if constexpr (CONF) {
+        if (conf) {
+            uint32_t q[PX];
+#pragma unroll
+            for (int j = 0; j < PX; ++j) q[j] = min(255u, __float2uint_rn(pl[j] * 255.f));
+            if (PX == 2) *reinterpret_cast<uint16_t *>(conf + o) = (uint16_t)(q[0] | (q[PX - 1] << 8));
+            else conf[o] = (uint8_t)q[0];
+        }
     }
     if (a.rgb) {
         uint8_t *d = a.rgb + o * 3;
@@ -148,9 +169,36 @@ __device__ __forceinline__ void emit_unit(const StitchArgs &a, const uint32_t *s
     }
 }
 
+// P of a corner block (or of any block when S == T): softmax of the raw logits, e[c] * (1 / sum).
+template <int CMAX, int PX>
+__device__ __forceinline__ void softmax_copy(const float (&v)[CMAX][PX], int C, float (&p)[CMAX][PX]) {
+#pragma unroll
+    for (int c = 0; c < CMAX; ++c)
+#pragma unroll
+        for (int j = 0; j < PX; ++j) p[c][j] = v[c][j];
+    float r[PX];
+    exp_cls<CMAX, PX, true>(p, C, kLog2e, r);
+#pragma unroll
+    for (int c = 0; c < CMAX; ++c)
+#pragma unroll
+        for (int j = 0; j < PX; ++j)
+            if (c < C) p[c][j] *= r[j];
+}
+
+// P of an interior block: the two strip SUMS (each the sum of two softmaxes) added and scaled by 1/4.
+template <int CMAX, int PX>
+__device__ __forceinline__ void quarter_sum(const float (&s0)[CMAX][PX], const float (&s1)[CMAX][PX], int C, float (&p)[CMAX][PX]) {
+#pragma unroll
+    for (int c = 0; c < CMAX; ++c)
+#pragma unroll
+        for (int j = 0; j < PX; ++j)
+            if (c < C) p[c][j] = (s0[c][j] + s1[c][j]) * 0.25f;
+}
+
 // NH: tiles per strip (1 border / 2 interior columns); NV: strips (1 border / 2 interior rows)
-template <int C_T, int CMAX, int PX, int NH, int NV>
-__device__ __forceinline__ void stitch_units(const StitchArgs &a, const uint32_t *s_lut, int ky, int kx, int row0, int nrows) {
+template <int C_T, int CMAX, int PX, int NH, int NV, int MODE, bool CONF>
+__device__ __forceinline__ void stitch_units(const StitchArgs &a, const uint32_t *s_lut, uint8_t *conf, int ky, int kx, int row0,
+                                             int nrows) {
     const int C = C_T > 0 ? C_T : a.C;
     const int T = a.T, S = a.S;
     const size_t cstride = (size_t)T * T;
@@ -209,7 +257,11 @@ __device__ __forceinline__ void stitch_units(const StitchArgs &a, const uint32_t
                 combine_cls<CMAX, PX>(v[s][0], r0, v[s][1], r1, C, NV == 2 ? 1.f : 0.5f);
             }
         }
-        if (NV == 2) {
+        constexpr bool NEED_P = MODE == 1 || CONF;
+        float p[CMAX][PX];          // P where it is not M itself (interior and corner blocks)
+        if constexpr (NEED_P && NV == 2 && NH == 2) quarter_sum<CMAX, PX>(v[0][0], v[NV - 1][0], C, p);
+        if constexpr (NEED_P && NV == 1 && NH == 1) softmax_copy<CMAX, PX>(v[0][0], C, p);
+        if (NV == 2 && !(MODE == 1 && NH == 2)) {     // mean mode needs no second softmax in the interior
             float r0[PX], r1[PX];
             if (NH == 2) {   // inputs: sums of two probability vectors, in [0, 2]
                 exp_cls<CMAX, PX, false>(v[0][0], C, 0.5f * kLog2e, r0);
@@ -220,12 +272,17 @@ __device__ __forceinline__ void stitch_units(const StitchArgs &a, const uint32_t
             }
             combine_cls<CMAX, PX>(v[0][0], r0, v[NV - 1][0], r1, C, 0.5f);
         }
-        emit_unit<CMAX, PX>(a, s_lut, C, v[0][0], (size_t)(ky * S + yl) * a.w + (size_t)(kx * S + xl));
+        const size_t o = (size_t)(ky * S + yl) * a.w + (size_t)(kx * S + xl);
+        constexpr bool P_IS_M = NH + NV == 3;         // edge blocks: P is the reference's M
+        if constexpr (!NEED_P) emit_unit<CMAX, PX>(a, s_lut, C, v[0][0], v[0][0], conf, o);
+        else if constexpr (P_IS_M) emit_unit<CMAX, PX, CONF>(a, s_lut, C, v[0][0], v[0][0], conf, o);
+        else if constexpr (MODE == 1) emit_unit<CMAX, PX, CONF>(a, s_lut, C, p, p, conf, o);
+        else emit_unit<CMAX, PX, CONF>(a, s_lut, C, v[0][0], p, conf, o);
     }
 }
 
-template <int C_T, int CMAX, int PX>
-__global__ void __launch_bounds__(kThreads, 2) stitch_kernel(StitchArgs a, const __grid_constant__ ColourLut lut) {
+template <int C_T, int CMAX, int PX, int MODE = 0, bool CONF = false>
+__global__ void __launch_bounds__(kThreads, 2) stitch_kernel(StitchArgs a, const __grid_constant__ ColourLut lut, uint8_t *conf) {
     __shared__ uint32_t s_lut[PYLC_MAX_CLASSES];
     if (threadIdx.x < PYLC_MAX_CLASSES) s_lut[threadIdx.x] = lut.rgb[threadIdx.x];
     __syncthreads();
@@ -242,11 +299,11 @@ __global__ void __launch_bounds__(kThreads, 2) stitch_kernel(StitchArgs a, const
     const bool two_h = a.overlap && kx > 0 && kx < a.nc;
     const bool two_v = a.overlap && ky > 0 && ky < a.nr;
     if (two_h) {
-        if (two_v) stitch_units<C_T, CMAX, PX, 2, 2>(a, s_lut, ky, kx, slab * a.rows_per_cta, a.rows_per_cta);
-        else stitch_units<C_T, CMAX, PX, 2, 1>(a, s_lut, ky, kx, slab * a.rows_per_cta, a.rows_per_cta);
+        if (two_v) stitch_units<C_T, CMAX, PX, 2, 2, MODE, CONF>(a, s_lut, conf, ky, kx, slab * a.rows_per_cta, a.rows_per_cta);
+        else stitch_units<C_T, CMAX, PX, 2, 1, MODE, CONF>(a, s_lut, conf, ky, kx, slab * a.rows_per_cta, a.rows_per_cta);
     } else {
-        if (two_v) stitch_units<C_T, CMAX, PX, 1, 2>(a, s_lut, ky, kx, slab * a.rows_per_cta, a.rows_per_cta);
-        else stitch_units<C_T, CMAX, PX, 1, 1>(a, s_lut, ky, kx, slab * a.rows_per_cta, a.rows_per_cta);
+        if (two_v) stitch_units<C_T, CMAX, PX, 1, 2, MODE, CONF>(a, s_lut, conf, ky, kx, slab * a.rows_per_cta, a.rows_per_cta);
+        else stitch_units<C_T, CMAX, PX, 1, 1, MODE, CONF>(a, s_lut, conf, ky, kx, slab * a.rows_per_cta, a.rows_per_cta);
     }
 }
 
@@ -280,8 +337,9 @@ struct StitchUpArgs {
     float *stitched;
 };
 
-template <int C_T, int CMAX, int NH, int NV>
-__device__ __forceinline__ void stitch_up_units(const StitchUpArgs &a, const uint32_t *s_lut, float *s_src, int ky, int kx, int row0) {
+template <int C_T, int CMAX, int NH, int NV, int MODE, bool CONF>
+__device__ __forceinline__ void stitch_up_units(const StitchUpArgs &a, const uint32_t *s_lut, uint8_t *conf, float *s_src, int ky, int kx,
+                                                int row0) {
     constexpr int PX = 2;
     const int C = C_T > 0 ? C_T : a.C;
     const int T = a.T, S = a.S, hs = a.hs, ws = a.ws;
@@ -414,7 +472,11 @@ __device__ __forceinline__ void stitch_up_units(const StitchUpArgs &a, const uin
 #pragma unroll
                 for (int j = 0; j < PX; ++j) strip[s][c][j] = v[0][c][j];
         }
-        if (NV == 2) {
+        constexpr bool NEED_P = MODE == 1 || CONF;     // P as in stitch_units
+        float p[CMAX][PX];
+        if constexpr (NEED_P && NV == 2 && NH == 2) quarter_sum<CMAX, PX>(strip[0], strip[NV - 1], C, p);
+        if constexpr (NEED_P && NV == 1 && NH == 1) softmax_copy<CMAX, PX>(strip[0], C, p);
+        if (NV == 2 && !(MODE == 1 && NH == 2)) {
             float r0[PX], r1[PX];
             if (NH == 2) {
                 exp_cls<CMAX, PX, false>(strip[0], C, 0.5f * kLog2e, r0);
@@ -427,12 +489,17 @@ __device__ __forceinline__ void stitch_up_units(const StitchUpArgs &a, const uin
         }
         StitchArgs e;                    // emit_unit only reads the output pointers and the map size
         e.labels = a.labels; e.rgb = a.rgb; e.stitched = a.stitched; e.h = a.h; e.w = a.w;
-        emit_unit<CMAX, PX>(e, s_lut, C, strip[0], (size_t)(ky * S + yl) * a.w + (size_t)(kx * S + X));
+        const size_t o = (size_t)(ky * S + yl) * a.w + (size_t)(kx * S + X);
+        constexpr bool P_IS_M = NH + NV == 3;
+        if constexpr (!NEED_P) emit_unit<CMAX, PX>(e, s_lut, C, strip[0], strip[0], conf, o);
+        else if constexpr (P_IS_M) emit_unit<CMAX, PX, CONF>(e, s_lut, C, strip[0], strip[0], conf, o);
+        else if constexpr (MODE == 1) emit_unit<CMAX, PX, CONF>(e, s_lut, C, p, p, conf, o);
+        else emit_unit<CMAX, PX, CONF>(e, s_lut, C, strip[0], p, conf, o);
     }
 }
 
-template <int C_T, int CMAX>
-__global__ void __launch_bounds__(kThreads, 2) stitch_up_kernel(StitchUpArgs a, const __grid_constant__ ColourLut lut) {
+template <int C_T, int CMAX, int MODE = 0, bool CONF = false>
+__global__ void __launch_bounds__(kThreads, 2) stitch_up_kernel(StitchUpArgs a, const __grid_constant__ ColourLut lut, uint8_t *conf) {
     extern __shared__ __align__(16) float s_up[];
     __shared__ uint32_t s_lut[PYLC_MAX_CLASSES];
     if (threadIdx.x < PYLC_MAX_CLASSES) s_lut[threadIdx.x] = lut.rgb[threadIdx.x];
@@ -445,11 +512,11 @@ __global__ void __launch_bounds__(kThreads, 2) stitch_up_kernel(StitchUpArgs a, 
     const bool two_h = a.overlap && kx > 0 && kx < a.nc;
     const bool two_v = a.overlap && ky > 0 && ky < a.nr;
     if (two_h) {
-        if (two_v) stitch_up_units<C_T, CMAX, 2, 2>(a, s_lut, s_up, ky, kx, slab * kUpR);
-        else stitch_up_units<C_T, CMAX, 2, 1>(a, s_lut, s_up, ky, kx, slab * kUpR);
+        if (two_v) stitch_up_units<C_T, CMAX, 2, 2, MODE, CONF>(a, s_lut, conf, s_up, ky, kx, slab * kUpR);
+        else stitch_up_units<C_T, CMAX, 2, 1, MODE, CONF>(a, s_lut, conf, s_up, ky, kx, slab * kUpR);
     } else {
-        if (two_v) stitch_up_units<C_T, CMAX, 1, 2>(a, s_lut, s_up, ky, kx, slab * kUpR);
-        else stitch_up_units<C_T, CMAX, 1, 1>(a, s_lut, s_up, ky, kx, slab * kUpR);
+        if (two_v) stitch_up_units<C_T, CMAX, 1, 2, MODE, CONF>(a, s_lut, conf, s_up, ky, kx, slab * kUpR);
+        else stitch_up_units<C_T, CMAX, 1, 1, MODE, CONF>(a, s_lut, conf, s_up, ky, kx, slab * kUpR);
     }
 }
 
@@ -457,12 +524,31 @@ __global__ void __launch_bounds__(kThreads, 2) stitch_up_kernel(StitchUpArgs a, 
 
 using namespace pylc;
 
-extern "C" int pylc_stitch_argmax_colour(const float *logits, const float *const *tile_batches, int tiles_per_batch,
-                                         int nr, int nc, int C, int T, int S, const uint8_t *lut_rgb,
-                                         uint8_t *labels, uint8_t *rgb, float *stitched, pylc_stream_t stream) {
+// Launch of the stitch kernel instantiation for (mode, confidence); the argmax / colour entry points take
+// mode 0 without confidence, the kernels they have always launched.
+template <int MODE, bool CONF>
+static void launch_stitch(bool px2, int C, unsigned grid, cudaStream_t st, const StitchArgs &a, const ColourLut &lut,
+                          uint8_t *conf) {
+    if (px2) {
+        if (C == 9) stitch_kernel<9, 9, 2, MODE, CONF><<<grid, kThreads, 0, st>>>(a, lut, conf);
+        else if (C == 11) stitch_kernel<11, 11, 2, MODE, CONF><<<grid, kThreads, 0, st>>>(a, lut, conf);
+        else if (C <= 4) stitch_kernel<0, 4, 2, MODE, CONF><<<grid, kThreads, 0, st>>>(a, lut, conf);
+        else if (C <= 8) stitch_kernel<0, 8, 2, MODE, CONF><<<grid, kThreads, 0, st>>>(a, lut, conf);
+        else stitch_kernel<0, 12, 2, MODE, CONF><<<grid, kThreads, 0, st>>>(a, lut, conf);
+    } else {
+        if (C <= 12) stitch_kernel<0, 12, 1, MODE, CONF><<<grid, kThreads, 0, st>>>(a, lut, conf);
+        else if (C <= 16) stitch_kernel<0, 16, 1, MODE, CONF><<<grid, kThreads, 0, st>>>(a, lut, conf);
+        else stitch_kernel<0, 32, 1, MODE, CONF><<<grid, kThreads, 0, st>>>(a, lut, conf);
+    }
+}
+
+static int stitch_launch(const float *logits, const float *const *tile_batches, int tiles_per_batch, int nr, int nc, int C,
+                         int T, int S, int mode, const uint8_t *lut_rgb, uint8_t *labels, uint8_t *rgb, uint8_t *confidence,
+                         float *stitched, pylc_stream_t stream) {
     if ((!logits && !tile_batches) || nr < 1 || nc < 1 || T < 1 || S < 1) return PYLC_ERR_ARG;
     if (!logits && tiles_per_batch < 1) return PYLC_ERR_ARG;
     if (rgb && !lut_rgb) return PYLC_ERR_ARG;
+    if (mode != PYLC_STITCH_REFERENCE && mode != PYLC_STITCH_MEAN) return PYLC_ERR_ARG;
     if (C < 1 || C > PYLC_MAX_CLASSES) return PYLC_ERR_CLASSES;
     if (!(S == T || 2 * S == T)) return PYLC_ERR_GEOMETRY;  // the reference is only correct for these (tools.py:235-236)
     StitchArgs a;
@@ -478,7 +564,7 @@ extern "C" int pylc_stitch_argmax_colour(const float *logits, const float *const
     a.labels = labels; a.rgb = rgb; a.stitched = stitched;
     const bool px2 = (S % 2 == 0) && C <= 12 && ((uintptr_t)logits % 8 == 0) &&
                      (!stitched || (uintptr_t)stitched % 8 == 0) && (!labels || (uintptr_t)labels % 2 == 0) &&
-                     (!rgb || (uintptr_t)rgb % 2 == 0);
+                     (!rgb || (uintptr_t)rgb % 2 == 0) && (!confidence || (uintptr_t)confidence % 2 == 0);
     const int PX = px2 ? 2 : 1;
     a.upr = S / PX;
     // One CTA per slab of up to eight units per thread.  Measured on B200 (273 / 45 tiles, C = 9): 8 units
@@ -495,30 +581,61 @@ extern "C" int pylc_stitch_argmax_colour(const float *logits, const float *const
     else for (int i = 0; i < PYLC_MAX_CLASSES; ++i) lut.rgb[i] = 0;
     const unsigned grid = (unsigned)((long long)a.nbx * a.nby * a.slabs);
     cudaStream_t st = (cudaStream_t)stream;
-    if (px2) {
-        if (C == 9) stitch_kernel<9, 9, 2><<<grid, kThreads, 0, st>>>(a, lut);
-        else if (C == 11) stitch_kernel<11, 11, 2><<<grid, kThreads, 0, st>>>(a, lut);
-        else if (C <= 4) stitch_kernel<0, 4, 2><<<grid, kThreads, 0, st>>>(a, lut);
-        else if (C <= 8) stitch_kernel<0, 8, 2><<<grid, kThreads, 0, st>>>(a, lut);
-        else stitch_kernel<0, 12, 2><<<grid, kThreads, 0, st>>>(a, lut);
+    if (mode == PYLC_STITCH_MEAN) {
+        if (confidence) launch_stitch<1, true>(px2, C, grid, st, a, lut, confidence);
+        else launch_stitch<1, false>(px2, C, grid, st, a, lut, nullptr);
     } else {
-        if (C <= 12) stitch_kernel<0, 12, 1><<<grid, kThreads, 0, st>>>(a, lut);
-        else if (C <= 16) stitch_kernel<0, 16, 1><<<grid, kThreads, 0, st>>>(a, lut);
-        else stitch_kernel<0, 32, 1><<<grid, kThreads, 0, st>>>(a, lut);
+        if (confidence) launch_stitch<0, true>(px2, C, grid, st, a, lut, confidence);
+        else launch_stitch<0, false>(px2, C, grid, st, a, lut, nullptr);
     }
     return finish_launch();
 }
 
-extern "C" int pylc_stitch_upsample_argmax_colour(const float *const *decoder_batches, int tiles_per_batch, int nr, int nc, int C,
-                                                  int T, int S, int hs, int ws, const uint8_t *lut_rgb, uint8_t *labels,
-                                                  uint8_t *rgb, float *stitched, pylc_stream_t stream) {
+extern "C" int pylc_stitch_argmax_colour(const float *logits, const float *const *tile_batches, int tiles_per_batch,
+                                         int nr, int nc, int C, int T, int S, const uint8_t *lut_rgb,
+                                         uint8_t *labels, uint8_t *rgb, float *stitched, pylc_stream_t stream) {
+    return stitch_launch(logits, tile_batches, tiles_per_batch, nr, nc, C, T, S, PYLC_STITCH_REFERENCE, lut_rgb, labels, rgb,
+                         nullptr, stitched, stream);
+}
+
+extern "C" int pylc_stitch_probs(const float *logits, const float *const *tile_batches, int tiles_per_batch, int nr, int nc,
+                                 int C, int T, int S, int mode, const uint8_t *lut_rgb, uint8_t *labels, uint8_t *rgb,
+                                 uint8_t *confidence, float *stitched, pylc_stream_t stream) {
+    return stitch_launch(logits, tile_batches, tiles_per_batch, nr, nc, C, T, S, mode, lut_rgb, labels, rgb, confidence,
+                         stitched, stream);
+}
+
+template <int MODE, bool CONF>
+static int launch_stitch_up(int C, unsigned grid, size_t smem, cudaStream_t st, const StitchUpArgs &a, const ColourLut &lut,
+                            uint8_t *conf) {
+#define LAUNCH_UP(CT, CM)                                                                                                  \
+    do {                                                                                                                   \
+        cudaError_t e = cudaFuncSetAttribute(stitch_up_kernel<CT, CM, MODE, CONF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
+        if (e != cudaSuccess) return (int)e;                                                                               \
+        stitch_up_kernel<CT, CM, MODE, CONF><<<grid, kThreads, smem, st>>>(a, lut, conf);                                     \
+    } while (0)
+    if (C == 9) LAUNCH_UP(9, 9);
+    else if (C == 11) LAUNCH_UP(11, 11);
+    else if (C <= 4) LAUNCH_UP(0, 4);
+    else if (C <= 8) LAUNCH_UP(0, 8);
+    else LAUNCH_UP(0, 12);
+#undef LAUNCH_UP
+    return 0;
+}
+
+static int stitch_up_launch(const float *const *decoder_batches, int tiles_per_batch, int nr, int nc, int C, int T, int S,
+                            int hs, int ws, int mode, const uint8_t *lut_rgb, uint8_t *labels, uint8_t *rgb,
+                            uint8_t *confidence, float *stitched, pylc_stream_t stream) {
     if (!decoder_batches || tiles_per_batch < 1 || nr < 1 || nc < 1 || T < 1 || S < 1 || hs < 2 || ws < 2) return PYLC_ERR_ARG;
     if (rgb && !lut_rgb) return PYLC_ERR_ARG;
+    if (mode != PYLC_STITCH_REFERENCE && mode != PYLC_STITCH_MEAN) return PYLC_ERR_ARG;
     if (C < 1 || C > PYLC_MAX_CLASSES) return PYLC_ERR_CLASSES;
     if (!(S == T || 2 * S == T)) return PYLC_ERR_GEOMETRY;
     // this form covers the network's geometry: a x4 up-sample, rows of 2-pixel units that fill a CTA evenly
     if (C > kUpCpad || hs * 4 != T || ws * 4 != T || S % kUpR || (S / 2) > kThreads || kThreads % (S / 2) || (S & (S - 1))) return PYLC_ERR_GEOMETRY;
-    if ((stitched && (uintptr_t)stitched % 8) || (labels && (uintptr_t)labels % 2) || (rgb && (uintptr_t)rgb % 2)) return PYLC_ERR_ALIGN;
+    if ((stitched && (uintptr_t)stitched % 8) || (labels && (uintptr_t)labels % 2) || (rgb && (uintptr_t)rgb % 2) ||
+        (confidence && (uintptr_t)confidence % 2))
+        return PYLC_ERR_ALIGN;
     StitchUpArgs a;
     a.batches = decoder_batches;
     a.tiles_per_batch = tiles_per_batch;
@@ -537,17 +654,24 @@ extern "C" int pylc_stitch_upsample_argmax_colour(const float *const *decoder_ba
     const size_t smem = (size_t)4 * kUpSrcRows * a.cols_max * kUpCpad * sizeof(float);
     const unsigned grid = (unsigned)((long long)a.nbx * a.nby * a.slabs);
     cudaStream_t st = (cudaStream_t)stream;
-#define LAUNCH_UP(CT, CM)                                                                                                  \
-    do {                                                                                                                   \
-        cudaError_t e = cudaFuncSetAttribute(stitch_up_kernel<CT, CM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-        if (e != cudaSuccess) return (int)e;                                                                               \
-        stitch_up_kernel<CT, CM><<<grid, kThreads, smem, st>>>(a, lut);                                                   \
-    } while (0)
-    if (C == 9) LAUNCH_UP(9, 9);
-    else if (C == 11) LAUNCH_UP(11, 11);
-    else if (C <= 4) LAUNCH_UP(0, 4);
-    else if (C <= 8) LAUNCH_UP(0, 8);
-    else LAUNCH_UP(0, 12);
-#undef LAUNCH_UP
+    int rc;
+    if (mode == PYLC_STITCH_MEAN) rc = confidence ? launch_stitch_up<1, true>(C, grid, smem, st, a, lut, confidence)
+                                                  : launch_stitch_up<1, false>(C, grid, smem, st, a, lut, nullptr);
+    else rc = confidence ? launch_stitch_up<0, true>(C, grid, smem, st, a, lut, confidence) : launch_stitch_up<0, false>(C, grid, smem, st, a, lut, nullptr);
+    if (rc) return rc;
     return finish_launch();
+}
+
+extern "C" int pylc_stitch_upsample_argmax_colour(const float *const *decoder_batches, int tiles_per_batch, int nr, int nc, int C,
+                                                  int T, int S, int hs, int ws, const uint8_t *lut_rgb, uint8_t *labels,
+                                                  uint8_t *rgb, float *stitched, pylc_stream_t stream) {
+    return stitch_up_launch(decoder_batches, tiles_per_batch, nr, nc, C, T, S, hs, ws, PYLC_STITCH_REFERENCE, lut_rgb, labels,
+                            rgb, nullptr, stitched, stream);
+}
+
+extern "C" int pylc_stitch_upsample_probs(const float *const *decoder_batches, int tiles_per_batch, int nr, int nc, int C,
+                                          int T, int S, int hs, int ws, int mode, const uint8_t *lut_rgb, uint8_t *labels,
+                                          uint8_t *rgb, uint8_t *confidence, float *stitched, pylc_stream_t stream) {
+    return stitch_up_launch(decoder_batches, tiles_per_batch, nr, nc, C, T, S, hs, ws, mode, lut_rgb, labels, rgb, confidence,
+                            stitched, stream);
 }

@@ -289,13 +289,9 @@ def stitch_dims(nr, nc, T, S):
     return ((nr + 1) * S, (nc + 1) * S) if S < T else (nr * S, nc * S)
 
 
-def stitch_argmax_colour(logits, nr, nc, T, S, lut_rgb=None, want_labels=True, want_rgb=False,
-                         want_stitched=False, tiles_per_batch=None):
-    """pylc_stitch_argmax_colour.  `logits` is one contiguous CUDA [nr*nc,C,T,T] f32 tensor, or a list
-    of per-batch tensors [<=b,C,T,T] (the reference's `model_outputs` list).
-    Returns (labels [h,w] u8 | None, rgb [h,w,3] u8 | None, stitched [C,h,w] f32 | None)."""
-    lib = _lib.load()
-    batch_table = None
+def _tile_source(logits, nr, nc, tiles_per_batch):
+    """(logits pointer, batch-table pointer, tiles per batch, C, device, batch table | None) of the stitch
+    kernels' input: one contiguous [nr*nc,C,T,T] f32 tensor or a list of per-batch tensors."""
     if isinstance(logits, (list, tuple)):
         _need_cuda(*logits)
         C = logits[0].shape[1]
@@ -310,40 +306,17 @@ def stitch_argmax_colour(logits, nr, nc, T, S, lut_rgb=None, want_labels=True, w
             raise PylcError("expected %d tiles, got %d" % (nr * nc, sum(t.shape[0] for t in logits)))
         ptrs = torch.tensor([t.data_ptr() for t in logits], dtype=torch.int64)
         batch_table = ptrs.to(dev, non_blocking=True)
-        lp, bp = ctypes.c_void_p(0), _p(batch_table)
-    else:
-        _need_cuda(logits)
-        if logits.dtype != torch.float32 or not logits.is_contiguous():
-            raise PylcError("logits must be contiguous float32")
-        if logits.shape[0] != nr * nc:
-            raise PylcError("expected %d tiles, got %d" % (nr * nc, logits.shape[0]))
-        C = logits.shape[1]
-        dev = logits.device
-        tpb = nr * nc
-        lp, bp = _p(logits), ctypes.c_void_p(0)
-    h, w = stitch_dims(nr, nc, T, S)
-    labels = torch.empty((h, w), dtype=torch.uint8, device=dev) if want_labels else None
-    rgb = torch.empty((h, w, 3), dtype=torch.uint8, device=dev) if want_rgb else None
-    stitched = torch.empty((C, h, w), dtype=torch.float32, device=dev) if want_stitched else None
-    pal = None
-    if lut_rgb is not None:
-        pal, c2 = _lib.palette_array(lut_rgb)
-        if c2 != C:
-            raise PylcError("lut_rgb has %d colours, logits have %d classes" % (c2, C))
-    check(lib.pylc_stitch_argmax_colour(lp, bp, tpb, nr, nc, C, T, S, pal, _p(labels), _p(rgb), _p(stitched),
-                                        _stream()), "pylc_stitch_argmax_colour")
-    if batch_table is not None:
-        batch_table.record_stream(torch.cuda.current_stream())
-    return labels, rgb, stitched
+        return ctypes.c_void_p(0), _p(batch_table), tpb, C, dev, batch_table
+    _need_cuda(logits)
+    if logits.dtype != torch.float32 or not logits.is_contiguous():
+        raise PylcError("logits must be contiguous float32")
+    if logits.shape[0] != nr * nc:
+        raise PylcError("expected %d tiles, got %d" % (nr * nc, logits.shape[0]))
+    return _p(logits), ctypes.c_void_p(0), nr * nc, logits.shape[1], logits.device, None
 
 
-def stitch_upsample_argmax_colour(decoder_batches, nr, nc, T, S, lut_rgb=None, want_labels=True, want_rgb=False,
-                                  want_stitched=False, tiles_per_batch=None):
-    """pylc_stitch_upsample_argmax_colour: stitch straight from the decoder's channels-last outputs
-    [b, C, T/4, T/4] (one tensor per network batch), the final x4 bilinear up-sample evaluated in the kernel.
-    Returns (labels [h,w] u8, rgb [h,w,3] u8 or None, stitched [C,h,w] f32 or None), bit-identical to
-    stitch_argmax_colour(upsample_nhwc_to_nchw(batch) ...)."""
-    lib = _lib.load()
+def _decoder_source(decoder_batches, nr, nc, tiles_per_batch):
+    """(batch table, tiles per batch, C, hs, ws, device) of the fused stitch's channels-last decoder outputs."""
     if torch.is_tensor(decoder_batches):
         decoder_batches = [decoder_batches]
     decoder_batches = list(decoder_batches)
@@ -359,19 +332,115 @@ def stitch_upsample_argmax_colour(decoder_batches, nr, nc, T, S, lut_rgb=None, w
     if sum(t.shape[0] for t in decoder_batches) != nr * nc:
         raise PylcError("expected %d tiles, got %d" % (nr * nc, sum(t.shape[0] for t in decoder_batches)))
     batch_table = torch.tensor([t.data_ptr() for t in decoder_batches], dtype=torch.int64).to(dev, non_blocking=True)
+    return batch_table, tpb, C, hs, ws, dev
+
+
+def _lut_for(lut_rgb, C, what):
+    if lut_rgb is None:
+        return None
+    pal, c2 = _lib.palette_array(lut_rgb)
+    if c2 != C:
+        raise PylcError("lut_rgb has %d colours, %s %d classes" % (c2, what, C))
+    return pal
+
+
+def stitch_argmax_colour(logits, nr, nc, T, S, lut_rgb=None, want_labels=True, want_rgb=False,
+                         want_stitched=False, tiles_per_batch=None):
+    """pylc_stitch_argmax_colour.  `logits` is one contiguous CUDA [nr*nc,C,T,T] f32 tensor, or a list
+    of per-batch tensors [<=b,C,T,T] (the reference's `model_outputs` list).
+    Returns (labels [h,w] u8 | None, rgb [h,w,3] u8 | None, stitched [C,h,w] f32 | None)."""
+    lib = _lib.load()
+    lp, bp, tpb, C, dev, batch_table = _tile_source(logits, nr, nc, tiles_per_batch)
     h, w = stitch_dims(nr, nc, T, S)
     labels = torch.empty((h, w), dtype=torch.uint8, device=dev) if want_labels else None
     rgb = torch.empty((h, w, 3), dtype=torch.uint8, device=dev) if want_rgb else None
     stitched = torch.empty((C, h, w), dtype=torch.float32, device=dev) if want_stitched else None
-    pal = None
-    if lut_rgb is not None:
-        pal, c2 = _lib.palette_array(lut_rgb)
-        if c2 != C:
-            raise PylcError("lut_rgb has %d colours, the decoder output has %d classes" % (c2, C))
+    pal = _lut_for(lut_rgb, C, "logits have")
+    check(lib.pylc_stitch_argmax_colour(lp, bp, tpb, nr, nc, C, T, S, pal, _p(labels), _p(rgb), _p(stitched),
+                                        _stream()), "pylc_stitch_argmax_colour")
+    if batch_table is not None:
+        batch_table.record_stream(torch.cuda.current_stream())
+    return labels, rgb, stitched
+
+
+def stitch_upsample_argmax_colour(decoder_batches, nr, nc, T, S, lut_rgb=None, want_labels=True, want_rgb=False,
+                                  want_stitched=False, tiles_per_batch=None):
+    """pylc_stitch_upsample_argmax_colour: stitch straight from the decoder's channels-last outputs
+    [b, C, T/4, T/4] (one tensor per network batch), the final x4 bilinear up-sample evaluated in the kernel.
+    Returns (labels [h,w] u8, rgb [h,w,3] u8 or None, stitched [C,h,w] f32 or None), bit-identical to
+    stitch_argmax_colour(upsample_nhwc_to_nchw(batch) ...)."""
+    lib = _lib.load()
+    batch_table, tpb, C, hs, ws, dev = _decoder_source(decoder_batches, nr, nc, tiles_per_batch)
+    h, w = stitch_dims(nr, nc, T, S)
+    labels = torch.empty((h, w), dtype=torch.uint8, device=dev) if want_labels else None
+    rgb = torch.empty((h, w, 3), dtype=torch.uint8, device=dev) if want_rgb else None
+    stitched = torch.empty((C, h, w), dtype=torch.float32, device=dev) if want_stitched else None
+    pal = _lut_for(lut_rgb, C, "the decoder output has")
     check(lib.pylc_stitch_upsample_argmax_colour(_p(batch_table), tpb, nr, nc, C, T, S, hs, ws, pal, _p(labels), _p(rgb),
                                                  _p(stitched), _stream()), "pylc_stitch_upsample_argmax_colour")
     batch_table.record_stream(torch.cuda.current_stream())
     return labels, rgb, stitched
+
+
+STITCH_MODES = {"reference": 0, "mean": 1}     # PYLC_STITCH_REFERENCE, PYLC_STITCH_MEAN
+
+
+def _stitch_mode(mode):
+    if mode not in STITCH_MODES:
+        raise PylcError("stitch mode must be one of %s, got %r" % (sorted(STITCH_MODES), mode))
+    return STITCH_MODES[mode]
+
+
+def _prob_outputs(C, h, w, dev, want_labels, want_rgb, want_confidence, want_probs, out):
+    out = dict(out or {})
+
+    def get(key, shape, dtype, want):
+        if out.get(key) is not None:
+            return out[key]
+        return torch.empty(shape, dtype=dtype, device=dev) if want else None
+    return {"labels": get("labels", (h, w), torch.uint8, want_labels),
+            "rgb": get("rgb", (h, w, 3), torch.uint8, want_rgb),
+            "confidence": get("confidence", (h, w), torch.uint8, want_confidence),
+            "probs": get("probs", (C, h, w), torch.float32, want_probs)}
+
+
+def stitch_probs(logits, nr, nc, T, S, mode="reference", lut_rgb=None, want_labels=True, want_rgb=False,
+                 want_confidence=True, want_probs=False, tiles_per_batch=None, out=None):
+    """pylc_stitch_probs: the stitch of stitch_argmax_colour with per-pixel probabilities.
+    P = the mean over the covering tiles of their softmaxes.  mode "reference": labels / rgb are those of
+    stitch_argmax_colour and `probs` is the reference's merged map M; mode "mean": labels = argmax P and
+    `probs` = P.  `confidence` is the u8 plane round(P[label] * 255) in both modes.
+    `out`: optional dict of preallocated outputs (any of labels / rgb / confidence / probs).
+    Returns dict(labels, rgb, confidence, probs), entries None where not wanted."""
+    lib = _lib.load()
+    m = _stitch_mode(mode)
+    lp, bp, tpb, C, dev, batch_table = _tile_source(logits, nr, nc, tiles_per_batch)
+    h, w = stitch_dims(nr, nc, T, S)
+    res = _prob_outputs(C, h, w, dev, want_labels, want_rgb, want_confidence, want_probs, out)
+    pal = _lut_for(lut_rgb, C, "logits have")
+    check(lib.pylc_stitch_probs(lp, bp, tpb, nr, nc, C, T, S, m, pal, _p(res["labels"]), _p(res["rgb"]),
+                                _p(res["confidence"]), _p(res["probs"]), _stream()), "pylc_stitch_probs")
+    if batch_table is not None:
+        batch_table.record_stream(torch.cuda.current_stream())
+    return res
+
+
+def stitch_upsample_probs(decoder_batches, nr, nc, T, S, mode="reference", lut_rgb=None, want_labels=True,
+                          want_rgb=False, want_confidence=True, want_probs=False, tiles_per_batch=None, out=None):
+    """pylc_stitch_upsample_probs: stitch_probs straight from the decoder's channels-last outputs (the fused
+    x4 up-sample of stitch_upsample_argmax_colour), bit-identical to
+    stitch_probs(upsample_nhwc_to_nchw(batch) ...).  Returns dict(labels, rgb, confidence, probs)."""
+    lib = _lib.load()
+    m = _stitch_mode(mode)
+    batch_table, tpb, C, hs, ws, dev = _decoder_source(decoder_batches, nr, nc, tiles_per_batch)
+    h, w = stitch_dims(nr, nc, T, S)
+    res = _prob_outputs(C, h, w, dev, want_labels, want_rgb, want_confidence, want_probs, out)
+    pal = _lut_for(lut_rgb, C, "the decoder output has")
+    check(lib.pylc_stitch_upsample_probs(_p(batch_table), tpb, nr, nc, C, T, S, hs, ws, m, pal, _p(res["labels"]),
+                                         _p(res["rgb"]), _p(res["confidence"]), _p(res["probs"]), _stream()),
+          "pylc_stitch_upsample_probs")
+    batch_table.record_stream(torch.cuda.current_stream())
+    return res
 
 
 def stitch_upsample_supported(C, T, S, hs, ws):
@@ -454,6 +523,37 @@ def confusion_u8(y_true, y_pred, n_classes, n_inject=0, conf=None):
     check(_lib.load().pylc_confusion_u8(_p(y_true), _p(y_pred), y_true.numel(), n_classes, n_inject, _p(conf),
                                         _stream()), "pylc_confusion_u8")
     return conf
+
+
+def confidence_resample(confidence, w_full, h_full, y_pred_full=None, y_true_full=None, n_classes=None,
+                        reliability=None, want_full=True, maps=None):
+    """pylc_confidence_resample: the fitted u8 confidence [h,w] to full resolution with the label map's
+    INTER_NEAREST index maps, and, given the full-resolution predicted and true classes, the reliability table
+    [C,256,2] i64 (pred, confidence level, correct) ADDED INTO `reliability` (allocated zeroed when None).
+    Returns dict(confidence_full, reliability)."""
+    _need_cuda(confidence, y_pred_full, y_true_full)
+    confidence = confidence.contiguous()
+    h, w = confidence.shape
+    dev = confidence.device
+    if maps is None:
+        maps = device_index_maps(w, h, w_full, h_full, dev)
+    x_ofs, y_ofs = maps
+    counting = y_pred_full is not None or y_true_full is not None
+    if counting:
+        if y_pred_full is None or y_true_full is None or n_classes is None:
+            raise PylcError("confidence_resample: the reliability table needs y_pred_full, y_true_full and n_classes")
+        y_pred_full, y_true_full = y_pred_full.contiguous(), y_true_full.contiguous()
+        if y_pred_full.numel() != h_full * w_full or y_true_full.numel() != h_full * w_full:
+            raise PylcError("confidence_resample: label planes must hold h_full * w_full pixels")
+        if reliability is None:
+            reliability = torch.zeros((n_classes, 256, 2), dtype=torch.int64, device=dev)
+    else:
+        reliability = None
+    full = torch.empty((h_full, w_full), dtype=torch.uint8, device=dev) if want_full else None
+    check(_lib.load().pylc_confidence_resample(_p(confidence), h, w, _p(x_ofs), _p(y_ofs), h_full, w_full, _p(y_pred_full),
+                                               _p(y_true_full), int(n_classes or 0), _p(full), _p(reliability), _stream()),
+          "pylc_confidence_resample")
+    return {"confidence_full": full, "reliability": reliability}
 
 
 # ---- multi-loss ---------------------------------------------------------------------------------

@@ -14,6 +14,9 @@ Here, per image (device_fit, the default whenever OpenCV's general area filter a
            DeepLabv3+/ResNet-101         stock PyTorch / cuDNN, batches of `batch_tiles`
            pylc_stitch_argmax_colour     logits -> label map, reference band semantics (1 launch)
            pylc_resample_encode_confusion  NN resample + GT encode + [C,C] counts    (1 launch)
+With `stitch="mean"` or `confidence=True` the stitch is pylc_stitch_probs / pylc_stitch_upsample_probs
+instead: labels from the mean of the covering tiles' softmaxes ("mean") and / or the u8 confidence plane
+of that mean; with keep_masks the plane is also resampled to full resolution (pylc_confidence_resample).
     D2H    nothing per image; the [C,C] i64 matrix (and optional masks) at the end
 With device_fit off (or for geometries OpenCV resizes with another filter) the fit-resize runs on
 host worker threads with cv2 itself and the fitted image is uploaded instead.
@@ -40,7 +43,8 @@ class FittedImage(object):
 
 class TiledSegmenter(object):
     def __init__(self, model, batch_tiles=32, channels_last=True, autocast_dtype=None, host_workers=4,
-                 n_inject=None, keep_masks=False, fuse_network=False, device_fit=True, fuse_upsample=True):
+                 n_inject=None, keep_masks=False, fuse_network=False, device_fit=True, fuse_upsample=True,
+                 stitch="reference", confidence=False):
         self.model = model
         self.meta = model.meta
         self.net = model.net.eval()
@@ -74,6 +78,9 @@ class TiledSegmenter(object):
         self.lut = tools.colourize_lut(self.C, self.palette)
         self.n_inject = min(len(defaults.class_codes), self.C) if n_inject is None else n_inject
         self.keep_masks = keep_masks
+        ops._stitch_mode(stitch)
+        self.stitch = stitch                      # "reference": the reference's labels; "mean": argmax of P
+        self.confidence = bool(confidence)        # adds res["confidence"] (and res["confidence_full"])
         self.device_fit = device_fit
         self.copy_stream = torch.cuda.Stream(device=self.device)
         self.pool = cf.ThreadPoolExecutor(max_workers=host_workers)
@@ -180,7 +187,18 @@ class TiledSegmenter(object):
             tiles = ops.tile_gather_norm_f32(img, f.h, f.w, self.ch, pitch, self.T, self.S, self.mean, self.std,
                                              self.post_div, self.out_ch)
         nr, nc = f.h // self.S - 1, f.w // self.S - 1
-        if self.fuse_upsample:
+        conf_fit = None
+        if self.stitch != "reference" or self.confidence:
+            probs = ops.stitch_upsample_probs if self.fuse_upsample else ops.stitch_probs
+            if self.fuse_upsample:
+                src = self.forward_tiles(tiles, s2d=self.s2d, decoder_only=True)
+            else:
+                src = self.forward_tiles(tiles, s2d=self.s2d)
+                src = src if len(src) > 1 else src[0]
+            out = probs(src, nr, nc, self.T, self.S, mode=self.stitch, want_confidence=self.confidence,
+                        tiles_per_batch=self.batch_tiles)
+            labels, conf_fit = out["labels"], out["confidence"]
+        elif self.fuse_upsample:
             dec = self.forward_tiles(tiles, s2d=self.s2d, decoder_only=True)
             labels, _, _ = ops.stitch_upsample_argmax_colour(dec, nr, nc, self.T, self.S, tiles_per_batch=self.batch_tiles)
         else:
@@ -193,6 +211,10 @@ class TiledSegmenter(object):
             n_classes=self.C, n_inject=n_inject if f.gt is not None else 0, conf=self.conf if f.gt is not None else None,
             want_pred=self.keep_masks, want_rgb=self.keep_masks)
         res["labels"] = labels
+        if conf_fit is not None:
+            res["confidence"] = conf_fit
+            if self.keep_masks:
+                res["confidence_full"] = ops.confidence_resample(conf_fit, f.w_full, f.h_full)["confidence_full"]
         return res
 
     # ---- drivers ------------------------------------------------------------------------------

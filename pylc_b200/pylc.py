@@ -9,7 +9,7 @@ train.py:22-174), same sub-commands and flags for the tiled-segmentation path:
     python -m pylc_b200.pylc augment --db FILE            (sample-rate search + over-sampling of rare classes)
     python -m pylc_b200.pylc train   --db FILE [--batch_size N --n_epochs E --lr LR --weighted ...]
     python -m pylc_b200.pylc test    --model M --img I [--mask G] [--scale S] [--save_logits]
-                                     [--aggregate_metrics]
+                                     [--aggregate_metrics] [--stitch reference|mean] [--save_confidence]
 
 Launched under torchrun (WORLD_SIZE > 1), `extract`/`profile`/`test` shard images or tiles across
 the GPUs and all-reduce only histograms / confusion matrices (pylc_b200.dist).  `merge` and `grayscale`
@@ -178,7 +178,9 @@ def test(args):
     extractor.verbose = False
     evaluator = Evaluator(model.meta)
     evaluator.aggregate_inject = 0 in mine           # the concatenated vectors carry ONE injection
-    seg = TiledSegmenter(model, batch_tiles=getattr(args, 'batch_tiles', 32), keep_masks=True)
+    save_confidence = bool(getattr(args, 'save_confidence', False))
+    seg = TiledSegmenter(model, batch_tiles=getattr(args, 'batch_tiles', 32), keep_masks=True,
+                         stitch=getattr(args, 'stitch', 'reference'), confidence=save_confidence)
     def decode(i):
         fpair = files[i]
         img_file, mask_file = (fpair['img'], fpair['mask']) if isinstance(fpair, dict) else (fpair, None)
@@ -199,6 +201,8 @@ def test(args):
                         'n': (f.h // seg.S - 1) * (f.w // seg.S - 1), 'w_full': w_full, 'h_full': h_full,
                         'w_scaled': w_scaled, 'h_scaled': h_scaled, 'w_fitted': f.w, 'h_fitted': f.h, 'offset': 0}
         evaluator.load(res, meta, mask_true_path=mask_file, scale=params.scale, mask_true=gt).save_image()
+        if save_confidence:
+            evaluator.save_confidence()
         if mask_file and not params.aggregate_metrics:
             print("\nStarting evaluation ... ")
             evaluator.evaluate().save_metrics()
@@ -281,6 +285,12 @@ def get_parser():
     p.add_argument('--save_logits', action='store_true')
     p.add_argument('--aggregate_metrics', action='store_true')
     p.add_argument('--batch_tiles', type=int, default=32)
+    # extensions: per-pixel probabilities (the mean of the covering tiles' softmaxes) and calibration
+    p.add_argument('--stitch', type=str, default='reference', choices=['reference', 'mean'],
+                   help="Labels from the reference's merge ('reference', default) or from the mean of the covering "
+                        "tiles' softmaxes ('mean').")
+    p.add_argument('--save_confidence', action='store_true',
+                   help='Write full-resolution confidence PNGs (255 = 1.0); with masks, add calibration (ECE) to the metrics.')
     return parser
 
 

@@ -16,6 +16,13 @@ aggregate, exactly where the concatenated vectors would carry it.
 
 `mask_pred` may be the reference's np.float32 [H,W,3] RGB array (it is re-encoded on the GPU) or
 the dict returned by tools.reconstruct_device (labels stay on the device; no RGB round trip).
+
+Confidence (an extension): when that dict also carries the fitted u8 confidence plane
+(TiledSegmenter(confidence=True)), load() resamples it to full resolution and counts the reliability
+table [C,256,2] (predicted class, confidence level, correct) in the same kernel call,
+pylc_confidence_resample -- per image and in aggregate, without the coverage injection.  evaluate()
+then adds a `calibration` entry (ECE, MCE, reliability bins, per-class confidence / accuracy) to the
+metrics, and save_confidence() writes the full-resolution plane as an 8-bit PNG (255 = 1.0).
 """
 import json
 import os
@@ -28,7 +35,7 @@ from .. import dist as pdist
 from .. import ops
 from ..config import Parameters, defaults
 from . import tools as utils
-from .metrics import Metrics
+from .metrics import Metrics, calibration_from_reliability
 
 
 class Evaluator:
@@ -50,6 +57,9 @@ class Evaluator:
         self.conf_aggregate = None    # device i64 [C,C]: all images, injection on the first only
         self.n_aggregated = 0
         self.aggregate_inject = True  # data-parallel: only the rank owning image 0 injects
+        self.reliability = None       # device i64 [C,256,2]: this image (confidence runs only)
+        self.reliability_aggregate = None
+        self.confidence_full = None   # device u8 [H,W]: this image's full-resolution confidence
         self.model_path = None
         self.output_dir = os.path.join(defaults.output_dir, str(self.meta.id))
         if make_dirs:
@@ -116,6 +126,14 @@ class Evaluator:
             raw = self.conf - count(1, n_inject)["conf"] + count(1, 0)["conf"]
             self.conf_aggregate = raw if self.conf_aggregate is None else self.conf_aggregate + raw
         self.n_aggregated += 1
+        if isinstance(pred, dict) and pred.get("confidence") is not None:
+            have_full = pred.get("confidence_full") is not None
+            cres = ops.confidence_resample(pred["confidence"], w_full, h_full, y_pred_full=res["pred_full"],
+                                           y_true_full=res["gt_full"], n_classes=C, want_full=not have_full, maps=maps)
+            self.confidence_full = pred["confidence_full"] if have_full else cres["confidence_full"]
+            self.reliability = cres["reliability"]
+            self.reliability_aggregate = self.reliability.clone() if self.reliability_aggregate is None \
+                else self.reliability_aggregate + self.reliability
         self.y_true_aggregate += [None]                   # placeholders: length = number of masks
         self.y_pred_aggregate += [None]
 
@@ -137,6 +155,12 @@ class Evaluator:
         self.metrics.mcc(None, None)
         self.metrics.confusion_matrix(None, None, labels=self.labels)
         self.metrics.report(None, None, labels=self.labels)
+        table = self.reliability_aggregate if aggregate else self.reliability
+        if table is not None:
+            if aggregate and distributed:
+                table = pdist.all_reduce_(table.clone())
+            self.metrics.results['calibration'] = calibration_from_reliability(table.cpu().numpy(), self.labels)
+            print('{:30s}{}'.format('ECE', self.metrics.results['calibration']['ece']))
         return self
 
     def validate(self):
@@ -159,6 +183,8 @@ class Evaluator:
         self.y_true = None
         self.y_pred = None
         self.conf = None
+        self.reliability = None
+        self.confidence_full = None
 
     def save_logits(self, logits):
         logits_file = os.path.join(self.logits_dir, self.fid + '_output.pth')
@@ -180,6 +206,26 @@ class Evaluator:
             np.save(cmap_data_file, self.metrics.cmatrix)
         self.metrics.plt.clf()
         return metrics_file, cmap_img_file, cmap_data_file
+
+    def save_confidence(self):
+        """Write the full-resolution confidence of the last loaded prediction as an 8-bit gray PNG
+        (255 = probability 1.0) to <output>/confidence/<fid>.png; the directory is created on first use."""
+        pred = self.mask_pred
+        conf = self.confidence_full
+        if conf is None and isinstance(pred, dict):
+            conf = pred.get("confidence_full")
+            if conf is None and pred.get("confidence") is not None:
+                ex = self.meta.extract
+                conf = ops.confidence_resample(pred["confidence"], ex['w_scaled'], ex['h_scaled'])["confidence_full"]
+        if conf is None:
+            print("No confidence map was computed. Confidence save cancelled.")
+            return
+        conf_file = os.path.join(utils.mk_path(os.path.join(self.output_dir, 'confidence')), self.fid + '.png')
+        if utils.confirm_write_file(conf_file):
+            cv2.imwrite(conf_file, conf.cpu().numpy())
+            print("Confidence map saved to: \n\t{}.".format(conf_file))
+            return conf_file
+        return
 
     def save_image(self):
         """Write the predicted RGB mask as PNG (reference evaluate.py:262-284)."""

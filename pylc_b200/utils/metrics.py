@@ -63,6 +63,49 @@ def scores_from_confusion(M, labels=None):
     return out
 
 
+def calibration_from_reliability(table, class_codes=None, n_bins=15):
+    """Calibration figures from a reliability table [C, 256, 2] of pixel counts (predicted class, confidence
+    level q, prediction correct) -- pylc_confidence_resample's table, summed over images and ranks.
+
+    The confidence of level q is q / 255.  Bin b of `n_bins` equal-width bins holds the levels with
+    b <= q / 255 * n_bins < b + 1 (the last bin also holds 1.0).  In float64:
+        ECE = sum_b n_b / N * |accuracy_b - confidence_b|,   MCE = max over non-empty bins of |accuracy_b - confidence_b|
+    and, per predicted class, the mean confidence and the accuracy of its pixels.  Empty bins / classes report
+    0.0 with a count of 0.  Returns a JSON-ready dict."""
+    t = np.asarray(table, dtype=np.int64)
+    if t.ndim != 3 or t.shape[1:] != (256, 2):
+        raise ValueError("reliability table must be [C, 256, 2], got %s" % (t.shape,))
+    C = t.shape[0]
+    level = np.arange(256, dtype=np.float64) / 255.0
+    bin_of = np.minimum((level * n_bins).astype(np.int64), n_bins - 1)
+    per_q = t.sum(axis=0)                                   # [256, 2] over classes
+    n_q = per_q.sum(axis=1).astype(np.float64)
+    hit_q = per_q[:, 1].astype(np.float64)
+    count = np.bincount(bin_of, weights=n_q, minlength=n_bins)
+    hits = np.bincount(bin_of, weights=hit_q, minlength=n_bins)
+    conf_sum = np.bincount(bin_of, weights=n_q * level, minlength=n_bins)
+
+    def ratio(a, b):
+        out = np.zeros_like(a, dtype=np.float64)
+        np.divide(a, b, out=out, where=b > 0)
+        return out
+    acc_b, conf_b = ratio(hits, count), ratio(conf_sum, count)
+    N = count.sum()
+    gap = np.abs(acc_b - conf_b)
+    ece = float((count * gap).sum() / N) if N > 0 else 0.0
+    mce = float(gap[count > 0].max()) if N > 0 else 0.0
+    n_c = t.sum(axis=(1, 2)).astype(np.float64)
+    hit_c = t[:, :, 1].sum(axis=1).astype(np.float64)
+    conf_c = ratio((t.sum(axis=2) * level[None, :]).sum(axis=1), n_c)
+    acc_c = ratio(hit_c, n_c)
+    names = list(class_codes) if class_codes is not None and len(class_codes) >= C else [str(i) for i in range(C)]
+    return {'ece': ece, 'mce': mce, 'n_bins': int(n_bins), 'n_pixels': int(N),
+            'bins': {'count': [int(v) for v in count], 'accuracy': [float(v) for v in acc_b],
+                     'confidence': [float(v) for v in conf_b]},
+            'classes': {str(names[c]): {'count': int(n_c[c]), 'confidence': float(conf_c[c]), 'accuracy': float(acc_c[c])}
+                        for c in range(C)}}
+
+
 def format_report(report):
     """Plain-text table of a classification report dict (what the reference prints, metrics.py:58-64)."""
     rows = [k for k in report if k not in ('accuracy', 'macro avg', 'weighted avg')]

@@ -276,7 +276,16 @@ def main():
     # the bench.py geometry: one fitted 2560x1536 image = 45 tiles (5 x 9)
     report("stitch_argmax_colour 45 tiles C9 labels (bench.py image)", 45 * C * T * T * 4 + 2560 * 1536,
            lambda: ops.stitch_argmax_colour(logits[:45], 5, 9, T, 256), "every logit once + 1 B label")
-    del logits
+    # per-pixel probabilities: labels + the u8 confidence plane, reference labels or the argmax of the mean
+    c_out = {"labels": torch.empty((Hf, Wf), dtype=torch.uint8, device="cuda"),
+             "confidence": torch.empty((Hf, Wf), dtype=torch.uint8, device="cuda")}
+    for mode in ("reference", "mean"):
+        report("stitch_probs 273 tiles C9 %s+confidence" % mode, logits.numel() * 4 + hw * 2,
+               lambda mode=mode: ops.stitch_probs(logits, nr, nc, T, 256, mode=mode, out=c_out),
+               "every logit once + 1 B label + 1 B confidence")
+        report("stitch_probs 45 tiles C9 %s+confidence (bench.py image)" % mode, 45 * C * T * T * 4 + 2560 * 1536 * 2,
+               lambda mode=mode: ops.stitch_probs(logits[:45], 5, 9, T, 256, mode=mode), "every logit once + 2 B per px")
+    del logits, c_out
     # §8f-1: the same image stitched straight from the decoder's [45, 9, 128, 128] channels-last output, the
     # final x4 bilinear up-sample evaluated in the kernel (no 424 MB logits round trip)
     dec = (torch.randn((45, C, T // 4, T // 4), generator=g, device="cuda") * 3).contiguous(memory_format=torch.channels_last)
@@ -284,6 +293,11 @@ def main():
            lambda: ops.stitch_upsample_argmax_colour(dec, 5, 9, T, 256),
            "decoder output once + 1 B label; replaces upsample_nhwc_to_nchw + stitch_argmax_colour (2 x 424.7 MB + 26.5 MB of traffic); "
            "exp- and blend-bound, not HBM-bound: compare its time with the sum of those two rows")
+    for mode in ("mean", "reference"):
+        report("stitch_upsample_probs 45 tiles C9 %s+confidence (bench.py image)" % mode, dec.numel() * 4 + 2560 * 1536 * 2,
+               lambda mode=mode: ops.stitch_upsample_probs(dec, 5, 9, T, 256, mode=mode),
+               "decoder output once + 2 B per px; mean mode skips the interior's second softmax (36 instead of 54 "
+               "exponentials per interior pixel at C = 9), compare with the row above")
     del dec
 
     # ---- evaluation --------------------------------------------------------------------------
@@ -336,6 +350,24 @@ def main():
     palc, _ = ops._lib.palette_array(pal)
     report("resample_encode_confusion 6000x4000 C9 + label outputs", H * W * 6, with_outputs,
            "3 B GT + 1 B label in, 2 x 1 B label maps out")
+
+    # confidence plane to full resolution + reliability table (fitted u8 plane, full-res predicted / true classes)
+    for (Wc, Hc) in ((3000, 2000), (6000, 4000)):
+        wc, hc = orc.fit_dims(Wc, Hc, T)
+        c_fit = torch.from_numpy(orc.synth_labels(5, wc, hc, 256, block=37)).cuda()
+        c_pred = torch.from_numpy(orc.synth_labels(6, Wc, Hc, C, skew=True, block=37)).cuda()
+        c_true = torch.from_numpy(orc.synth_labels(7, Wc, Hc, C, skew=True, block=37)).cuda()
+        c_maps = ops.device_index_maps(wc, hc, Wc, Hc, c_fit.device)
+        rel = torch.zeros((C, 256, 2), dtype=torch.int64, device="cuda")
+        c_full = torch.empty((Hc, Wc), dtype=torch.uint8, device="cuda")
+
+        def conf_resample(c_fit=c_fit, c_pred=c_pred, c_true=c_true, c_maps=c_maps, rel=rel, c_full=c_full, Wc=Wc, Hc=Hc, wc=wc, hc=hc):
+            ops._lib.check(ops._lib.load().pylc_confidence_resample(
+                ops._p(c_fit), hc, wc, ops._p(c_maps[0]), ops._p(c_maps[1]), Hc, Wc, ops._p(c_pred), ops._p(c_true), C,
+                ops._p(c_full), ops._p(rel), ops._stream()), "pylc_confidence_resample")
+        report("confidence_resample %dx%d C9 + reliability" % (Wc, Hc), Hc * Wc * 3, conf_resample,
+               "1 B pred + 1 B truth in, 1 B confidence out per full-res px; 37-px blocks")
+        del c_fit, c_pred, c_true, c_full
 
     # ---- multi-loss --------------------------------------------------------------------------
     B = 64
