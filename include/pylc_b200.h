@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define PYLC_ABI_VERSION 3
+#define PYLC_ABI_VERSION 4
 #define PYLC_MAX_CLASSES 32
 
 #define PYLC_OK 0
@@ -355,6 +355,28 @@ PYLC_API int pylc_confidence_resample(const uint8_t *confidence, int h, int w, c
                              const int32_t *y_ofs, int h_full, int w_full, const uint8_t *y_pred_full,
                              const uint8_t *y_true_full, int C, uint8_t *confidence_full, int64_t *reliability,
                              pylc_stream_t stream);
+
+/*
+ * Multi-scale combine (an extension): the mean-mode probability maps of K image scales averaged on one output grid.
+ *   probs         HOST [K] array of DEVICE pointers, member k = [C, h[k], w[k]] f32 (pylc_stitch_probs' `stitched`
+ *                 in PYLC_STITCH_MEAN mode for the image resized by s_k and fitted to the tiles)
+ *   x_ofs / y_ofs HOST [K] arrays of DEVICE pointers, x_ofs[k] = [w_full] i32, y_ofs[k] = [h_full] i32: OpenCV's
+ *                 INTER_NEAREST source index per output index from (w[k], h[k]) to (w_full, h_full), as
+ *                 pylc_resample_encode_confusion takes them.  PRECONDITION, not checked on the device: every value
+ *                 lies in [0, w[k]) / [0, h[k]); the host layer checks its maps once per geometry
+ *   h / w         HOST [K] member plane sizes
+ * Per output pixel and class, in f32 and in this order: sum = P_1[c] + ... + P_K[c] (scale order),
+ * Pbar[c] = sum * f32(1/K); label = first argmax of Pbar; confidence = min(255, round-to-nearest(Pbar[label] * 255)).
+ * With K = 1 these are the member's mean-mode labels and confidence, resampled with the maps.
+ *   labels        nullable [h_full, w_full] u8 ; rgb nullable [h_full, w_full, 3] u8 (lut_rgb HOST [C, 3], needed iff
+ *                 rgb) ; confidence nullable [h_full, w_full] u8.  At least one output.
+ * Any width and any output alignment; rows are dense.  PYLC_ERR_ARG for K outside [1, PYLC_MAX_SCALES], a null
+ * plane or map, a non-positive size or no output; PYLC_ERR_CLASSES for C outside [1, 32].
+ */
+#define PYLC_MAX_SCALES 8
+PYLC_API int pylc_multiscale_combine(const float *const *probs, const int32_t *const *x_ofs, const int32_t *const *y_ofs,
+                            const int *h, const int *w, int K, int C, int h_full, int w_full, const uint8_t *lut_rgb,
+                            uint8_t *labels, uint8_t *rgb, uint8_t *confidence, pylc_stream_t stream);
 
 /* ---- multi-loss --------------------------------------------------------------------------- */
 

@@ -15,7 +15,8 @@ LIB_PATH = os.path.join(_HERE, "lib", "libpylc_b200.so")
 
 MAX_CLASSES = 32
 AREA_TAPS = 6
-ABI_VERSION = 3
+ABI_VERSION = 4
+MAX_SCALES = 8
 
 
 class PylcError(RuntimeError):
@@ -78,6 +79,8 @@ SIGNATURES = {
                                                _u8p, _u8p, _u8p, _ptr]),
     "pylc_confusion_u8": (c_int, [_u8p, _u8p, c_int64, c_int, c_int, _ptr, _ptr]),
     "pylc_confidence_resample": (c_int, [_u8p, c_int, c_int, _ptr, _ptr, c_int, c_int, _u8p, _u8p, c_int, _u8p, _ptr, _ptr]),
+    "pylc_multiscale_combine": (c_int, [_ptr, _ptr, _ptr, POINTER(c_int), POINTER(c_int), c_int, c_int, c_int, c_int,
+                                        POINTER(c_uint8), _u8p, _u8p, _u8p, _ptr]),
     "pylc_multiloss_reduce": (c_int, [_ptr, _ptr, c_int, c_int, c_int, c_int64, _ptr, POINTER(LossCfg),
                                       _ptr, _u8p, _ptr]),
     "pylc_multiloss_finalize": (c_int, [_ptr, c_int, c_int64, POINTER(LossCfg), _ptr, _ptr]),

@@ -556,6 +556,51 @@ def confidence_resample(confidence, w_full, h_full, y_pred_full=None, y_true_ful
     return {"confidence_full": full, "reliability": reliability}
 
 
+_CHECKED_MAPS = set()
+
+
+def _checked_index_maps(w, h, w_full, h_full, device):
+    """device_index_maps, with every index checked to lie inside the (w, h) plane once per geometry (the C ABI
+    takes that as a precondition)."""
+    key = (w, h, w_full, h_full)
+    if key not in _CHECKED_MAPS:
+        for src, dst in ((w, w_full), (h, h_full)):
+            m = nn_index_map(src, dst)
+            if m.min() < 0 or m.max() >= src:
+                raise PylcError("index map %d -> %d leaves its plane" % (src, dst))
+        _CHECKED_MAPS.add(key)
+    return device_index_maps(w, h, w_full, h_full, device)
+
+
+def multiscale_combine(probs, w_full, h_full, lut_rgb=None, want_labels=True, want_rgb=False, want_confidence=True,
+                       out=None):
+    """pylc_multiscale_combine: the probability maps of K <= 8 image scales, a list of [C, h_k, w_k] f32 CUDA tensors
+    (mean-mode `probs` of stitch_probs / stitch_upsample_probs), sampled onto the [h_full, w_full] grid with the label
+    map's INTER_NEAREST index maps and averaged in scale order: labels = first argmax of the mean, confidence =
+    min(255, round(mean[label] * 255)).  `out`: optional dict of preallocated outputs (labels / rgb / confidence).
+    Returns dict(labels, rgb, confidence), entries None where not wanted."""
+    probs = list(probs)
+    if not 1 <= len(probs) <= _lib.MAX_SCALES:
+        raise PylcError("multiscale_combine takes 1 to %d probability maps, got %d" % (_lib.MAX_SCALES, len(probs)))
+    _need_cuda(*probs)
+    C, dev = probs[0].shape[0], probs[0].device
+    for p in probs:
+        if p.dtype != torch.float32 or p.dim() != 3 or not p.is_contiguous() or p.shape[0] != C or p.device != dev:
+            raise PylcError("multiscale_combine takes contiguous [C, h, w] float32 maps of one class count and device")
+    K = len(probs)
+    maps = [_checked_index_maps(p.shape[2], p.shape[1], w_full, h_full, dev) for p in probs]
+    res = _prob_outputs(C, h_full, w_full, dev, want_labels, want_rgb, want_confidence, False, out)
+    res.pop("probs")
+    pal = _lut_for(lut_rgb, C, "the probability maps have")
+    ptrs = lambda ts: (ctypes.c_void_p * K)(*[t.data_ptr() for t in ts])     # noqa: E731
+    ints = lambda vals: (ctypes.c_int * K)(*vals)                             # noqa: E731
+    check(_lib.load().pylc_multiscale_combine(ptrs(probs), ptrs([m[0] for m in maps]), ptrs([m[1] for m in maps]),
+                                              ints([p.shape[1] for p in probs]), ints([p.shape[2] for p in probs]), K, C,
+                                              int(h_full), int(w_full), pal, _p(res["labels"]), _p(res["rgb"]),
+                                              _p(res["confidence"]), _stream()), "pylc_multiscale_combine")
+    return res
+
+
 # ---- multi-loss ---------------------------------------------------------------------------------
 
 

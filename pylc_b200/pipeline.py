@@ -18,6 +18,11 @@ With `stitch="mean"` or `confidence=True` the stitch is pylc_stitch_probs / pylc
 instead: labels from the mean of the covering tiles' softmaxes ("mean") and / or the u8 confidence plane
 of that mean; with keep_masks the plane is also resampled to full resolution (pylc_confidence_resample).
     D2H    nothing per image; the [C,C] i64 matrix (and optional masks) at the end
+With `scales` (multi-scale inference, mean stitch only) every image is segmented once per scale s_k: the decoded
+image resized by s_k (INTER_AREA) and fitted to the tiles, on the device when both resizes are OpenCV's general
+area filter, otherwise with cv2 on the host threads.  Each member's mean-mode probability map P_k stays on the
+device; pylc_multiscale_combine samples every P_k onto the full-resolution grid, averages them and writes the
+full-resolution labels and confidence, and pylc_resample_encode_confusion counts the confusion from those.
 With device_fit off (or for geometries OpenCV resizes with another filter) the fit-resize runs on
 host worker threads with cv2 itself and the fitted image is uploaded instead.
 Logits never leave the device.  Images are independent, so data-parallel ranks take images
@@ -37,14 +42,51 @@ from .utils.metrics import scores_from_confusion
 
 
 class FittedImage(object):
-    """A fitted u8 image (and optional RGB ground truth) resident on the device."""
-    __slots__ = ("img", "pitch", "h", "w", "gt", "gt_pitch", "h_full", "w_full", "index", "ready", "raw", "raw_pitch")
+    """A fitted u8 image (and optional RGB ground truth) resident on the device.  Multi-scale: `members` holds one
+    (geometry, fitted image, pitch) triple per scale (multiscale_geometry); a fitted image of None means the member
+    is fitted from `raw` on the device."""
+    __slots__ = ("img", "pitch", "h", "w", "gt", "gt_pitch", "h_full", "w_full", "index", "ready", "raw", "raw_pitch",
+                 "members")
+
+
+MAX_SCALES = 8
+
+
+def check_scales(scales):
+    """The scale list of a multi-scale run, sorted; ValueError for an empty or too long list, a duplicate or a
+    non-positive scale."""
+    vals = sorted(float(s) for s in scales)
+    if not 1 <= len(vals) <= MAX_SCALES:
+        raise ValueError("multi-scale inference takes 1 to %d scales, got %d" % (MAX_SCALES, len(vals)))
+    if vals[0] <= 0:
+        raise ValueError("scales must be positive, got %g" % vals[0])
+    if len(set(vals)) != len(vals):
+        raise ValueError("duplicate scale in %s" % (vals,))
+    return tuple(vals)
+
+
+def multiscale_geometry(W, H, T, scales):
+    """Per scale s of a W x H decoded image: dict(scale, resized=(w, h), fitted=(w, h), device).  The member image is
+    cv2.resize(img, (int(s*W), int(s*H)), INTER_AREA) (no resize at s == 1) fitted by adjust_to_tile; `device` is True
+    when OpenCV does both resizes with the general area filter that pylc_fit_resize_area_u8 reproduces.  Raises
+    ValueError, naming the scale and the size, for a member whose fitted image is less than two tiles high or wide:
+    the reference's stitch leaves rows of a one-tile-row image unset, so such a fit is outside its contract."""
+    out = []
+    for s in check_scales(scales):
+        wr, hr = (W, H) if s == 1.0 else (int(s * W), int(s * H))
+        wf, hf = tools.fit_dims(wr, hr, T) if wr >= 1 and hr >= 1 else (0, 0)
+        if wf < 2 * T or hf < 2 * T:
+            raise ValueError("scale %g: the %dx%d image resizes to %dx%d, which fits to %dx%d, less than two %d-pixel "
+                             "tiles in a direction" % (s, W, H, wr, hr, wf, hf, T))
+        device = (s == 1.0 or ops.area_supported(W, H, wr, hr)) and ops.area_supported(wr, hr, wf, hf)
+        out.append({"scale": s, "resized": (wr, hr), "fitted": (wf, hf), "device": bool(device)})
+    return out
 
 
 class TiledSegmenter(object):
     def __init__(self, model, batch_tiles=32, channels_last=True, autocast_dtype=None, host_workers=4,
                  n_inject=None, keep_masks=False, fuse_network=False, device_fit=True, fuse_upsample=True,
-                 stitch="reference", confidence=False):
+                 stitch="reference", confidence=False, scales=None):
         self.model = model
         self.meta = model.meta
         self.net = model.net.eval()
@@ -81,6 +123,12 @@ class TiledSegmenter(object):
         ops._stitch_mode(stitch)
         self.stitch = stitch                      # "reference": the reference's labels; "mean": argmax of P
         self.confidence = bool(confidence)        # adds res["confidence"] (and res["confidence_full"])
+        # multi-scale: labels and confidence from the mean of the members' mean-mode probabilities
+        self.scales = None
+        if scales is not None:
+            if stitch != "mean":
+                raise ValueError("multi-scale inference averages the mean stitch's probabilities: it needs stitch='mean'")
+            self.scales = check_scales(scales)
         self.device_fit = device_fit
         self.copy_stream = torch.cuda.Stream(device=self.device)
         self.pool = cf.ThreadPoolExecutor(max_workers=host_workers)
@@ -99,6 +147,8 @@ class TiledSegmenter(object):
         wait on `f.ready` before touching its tensors."""
         if torch.is_tensor(img):
             img = img.numpy()
+        if self.scales is not None:
+            return self._stage_multiscale(img, gt, index, None)
         buf, pitch, h, w = self.fit_host(img)
         f = FittedImage()
         f.index = index
@@ -128,6 +178,8 @@ class TiledSegmenter(object):
         """Device fit: pitched H2D of the DECODED image (and ground truth) on the copy stream; the
         INTER_AREA resize itself is launched by segment_fitted on the compute stream.  `after`: an event
         the copy stream waits for first (bounds how far uploads run ahead of the compute stream)."""
+        if self.scales is not None:
+            return self._stage_multiscale(img, gt, index, after)
         t_img = img if torch.is_tensor(img) else torch.from_numpy(np.ascontiguousarray(img))
         f = FittedImage()
         f.index = index
@@ -146,6 +198,52 @@ class TiledSegmenter(object):
             f.ready = torch.cuda.Event()
             f.ready.record(self.copy_stream)
         return f
+
+    def _stage_multiscale(self, img, gt, index, after):
+        """Multi-scale staging on the copy stream: one upload of the decoded image when a member is fitted on the
+        device, and for every other member cv2.resize + adjust_to_tile here (a host worker thread under run_host)
+        and the upload of the fitted image."""
+        img = img.numpy() if torch.is_tensor(img) else np.asarray(img)
+        f = FittedImage()
+        f.index = index
+        f.h_full, f.w_full = img.shape[0], img.shape[1]
+        f.w, f.h = tools.fit_dims(f.w_full, f.h_full, self.T)
+        f.img, f.pitch = None, 0
+        geo = multiscale_geometry(f.w_full, f.h_full, self.T, self.scales)
+        on_device = [self.device_fit and g["device"] for g in geo]
+        hosted = []
+        for g, dev in zip(geo, on_device):
+            if dev:
+                hosted.append((None, 0))
+                continue
+            x = img if g["scale"] == 1.0 else cv2.resize(img, g["resized"], interpolation=cv2.INTER_AREA)
+            hosted.append(self.fit_host(x)[:2])
+        with torch.cuda.stream(self.copy_stream):
+            if after is not None:
+                self.copy_stream.wait_event(after)
+            f.raw, f.raw_pitch = None, 0
+            if any(on_device):
+                buf, f.raw_pitch = ops.pinned_pitched(img)
+                f.raw = buf.to(self.device, non_blocking=True)
+            f.members = [(g, None if buf is None else buf.to(self.device, non_blocking=True), pitch)
+                         for g, (buf, pitch) in zip(geo, hosted)]
+            if gt is not None:
+                if torch.is_tensor(gt) and gt.ndim == 2:      # already a pitched [H, pitch] buffer
+                    gbuf, f.gt_pitch = gt, gt.shape[1]
+                else:
+                    gbuf, f.gt_pitch = ops.pinned_pitched(gt.numpy() if torch.is_tensor(gt) else gt)
+                f.gt = gbuf.to(self.device, non_blocking=True)
+            else:
+                f.gt, f.gt_pitch = None, 0
+            f.ready = torch.cuda.Event()
+            f.ready.record(self.copy_stream)
+        return f
+
+    def _release(self, f, stream):
+        """Tie the staged buffers of `f` to `stream`, where the device work that reads them was enqueued."""
+        for t in [f.img, f.raw, f.gt] + [m[1] for m in (getattr(f, "members", None) or [])]:
+            if t is not None:
+                t.record_stream(stream)
 
     # ---- device stage -------------------------------------------------------------------------
     def forward_tiles(self, tiles, s2d=False, decoder_only=False):
@@ -175,28 +273,35 @@ class TiledSegmenter(object):
                 outs.append(torch.nn.functional.interpolate(y, size=x.shape[2:], mode='bilinear', align_corners=True))
         return outs
 
+    def _tiles(self, img, pitch, h, w):
+        if self.s2d:
+            return ops.tile_gather_norm_s2d(img, h, w, self.ch, pitch, self.T, self.S, self.mean, self.std, self.post_div)
+        return ops.tile_gather_norm_f32(img, h, w, self.ch, pitch, self.T, self.S, self.mean, self.std, self.post_div,
+                                        self.out_ch)
+
+    def _stitch_probs(self, tiles, nr, nc, **kw):
+        """Network + pylc_stitch_probs (or its fused up-sample form) over one fitted image's tiles."""
+        probs = ops.stitch_upsample_probs if self.fuse_upsample else ops.stitch_probs
+        if self.fuse_upsample:
+            src = self.forward_tiles(tiles, s2d=self.s2d, decoder_only=True)
+        else:
+            src = self.forward_tiles(tiles, s2d=self.s2d)
+            src = src if len(src) > 1 else src[0]
+        return probs(src, nr, nc, self.T, self.S, mode=self.stitch, tiles_per_batch=self.batch_tiles, **kw)
+
     def segment_fitted(self, f, inject=None):
         """All device work for one fitted image; accumulates into self.conf when f.gt is set.
         Returns the fitted-resolution label map (and full-res masks when keep_masks)."""
+        if self.scales is not None:
+            return self._segment_multiscale(f, inject)
         img, pitch = f.img, f.pitch
         if img is None:        # device fit: INTER_AREA resize of the uploaded decoded image
             img, pitch = ops.fit_resize_area(f.raw, f.h_full, f.w_full, self.ch, f.raw_pitch, f.h, f.w)
-        if self.s2d:
-            tiles = ops.tile_gather_norm_s2d(img, f.h, f.w, self.ch, pitch, self.T, self.S, self.mean, self.std, self.post_div)
-        else:
-            tiles = ops.tile_gather_norm_f32(img, f.h, f.w, self.ch, pitch, self.T, self.S, self.mean, self.std,
-                                             self.post_div, self.out_ch)
+        tiles = self._tiles(img, pitch, f.h, f.w)
         nr, nc = f.h // self.S - 1, f.w // self.S - 1
         conf_fit = None
         if self.stitch != "reference" or self.confidence:
-            probs = ops.stitch_upsample_probs if self.fuse_upsample else ops.stitch_probs
-            if self.fuse_upsample:
-                src = self.forward_tiles(tiles, s2d=self.s2d, decoder_only=True)
-            else:
-                src = self.forward_tiles(tiles, s2d=self.s2d)
-                src = src if len(src) > 1 else src[0]
-            out = probs(src, nr, nc, self.T, self.S, mode=self.stitch, want_confidence=self.confidence,
-                        tiles_per_batch=self.batch_tiles)
+            out = self._stitch_probs(tiles, nr, nc, want_confidence=self.confidence)
             labels, conf_fit = out["labels"], out["confidence"]
         elif self.fuse_upsample:
             dec = self.forward_tiles(tiles, s2d=self.s2d, decoder_only=True)
@@ -215,6 +320,37 @@ class TiledSegmenter(object):
             res["confidence"] = conf_fit
             if self.keep_masks:
                 res["confidence_full"] = ops.confidence_resample(conf_fit, f.w_full, f.h_full)["confidence_full"]
+        return res
+
+    def member_probs(self, f):
+        """The mean-mode probability map [C, h_k, w_k] of every scale of a multi-scale FittedImage, in scale order."""
+        planes = []
+        for g, img, pitch in f.members:
+            (wr, hr), (wf, hf) = g["resized"], g["fitted"]
+            if img is None and g["scale"] == 1.0:
+                img, pitch = ops.fit_resize_area(f.raw, f.h_full, f.w_full, self.ch, f.raw_pitch, hf, wf)
+            elif img is None:
+                r, rp = ops.fit_resize_area(f.raw, f.h_full, f.w_full, self.ch, f.raw_pitch, hr, wr)
+                img, pitch = ops.fit_resize_area(r, hr, wr, self.ch, rp, hf, wf)
+            tiles = self._tiles(img, pitch, hf, wf)
+            out = self._stitch_probs(tiles, hf // self.S - 1, wf // self.S - 1, want_labels=False, want_confidence=False,
+                                     want_probs=True)
+            planes.append(out["probs"])
+        return planes
+
+    def _segment_multiscale(self, f, inject):
+        planes = self.member_probs(f)
+        comb = ops.multiscale_combine(planes, f.w_full, f.h_full, want_confidence=self.confidence)
+        del planes                     # one image's members are live at a time
+        n_inject = self.n_inject if inject is None else inject
+        labels = comb["labels"]
+        res = ops.resample_encode_confusion(
+            labels, f.w_full, f.h_full, gt_rgb=f.gt, gt_pitch=f.gt_pitch, palette=self.palette, lut_rgb=self.lut,
+            n_classes=self.C, n_inject=n_inject if f.gt is not None else 0, conf=self.conf if f.gt is not None else None,
+            want_pred=self.keep_masks, want_rgb=self.keep_masks)
+        res["labels"] = labels
+        if comb["confidence"] is not None:
+            res["confidence"] = res["confidence_full"] = comb["confidence"]
         return res
 
     # ---- drivers ------------------------------------------------------------------------------
@@ -251,7 +387,7 @@ class TiledSegmenter(object):
             self._gidx = [int(global_offset) + i for i in range(len(images))]
         compute = torch.cuda.current_stream(self.device)
         prefetch = 3
-        if idx and all(self.can_fit_on_device(images[i]) for i in idx):
+        if self.scales is None and idx and all(self.can_fit_on_device(images[i]) for i in idx):
             return self._run_host_device_fit(images, masks, idx, compute, prefetch, distributed)
 
         def submit(k):
@@ -266,9 +402,7 @@ class TiledSegmenter(object):
                 pending.append(submit(k + prefetch))
             compute.wait_event(f.ready)
             res = self.segment_fitted(f, inject=self.n_inject if f.index == 0 else 0)
-            f.img.record_stream(compute)
-            if f.gt is not None:
-                f.gt.record_stream(compute)
+            self._release(f, compute)
             if self.keep_masks:
                 results.append(res)
         conf = self.conf

@@ -10,6 +10,7 @@ train.py:22-174), same sub-commands and flags for the tiled-segmentation path:
     python -m pylc_b200.pylc train   --db FILE [--batch_size N --n_epochs E --lr LR --weighted ...]
     python -m pylc_b200.pylc test    --model M --img I [--mask G] [--scale S] [--save_logits]
                                      [--aggregate_metrics] [--stitch reference|mean] [--save_confidence]
+                                     [--multiscale S1 S2 ...]   (with --stitch mean)
 
 Launched under torchrun (WORLD_SIZE > 1), `extract`/`profile`/`test` shard images or tiles across
 the GPUs and all-reduce only histograms / confusion matrices (pylc_b200.dist).  `merge` and `grayscale`
@@ -166,6 +167,16 @@ def test(args):
     from .utils import tools
     from .utils.evaluate import Evaluator
     from .utils.extract import Extractor
+    from .pipeline import check_scales
+    multiscale = getattr(args, 'multiscale', None)
+    if multiscale and getattr(args, 'stitch', 'reference') != 'mean':
+        print('--multiscale averages the probabilities of the mean stitch: add --stitch mean.', file=sys.stderr)
+        sys.exit(2)
+    try:
+        multiscale = check_scales(multiscale) if multiscale else None
+    except ValueError as exc:
+        print('--multiscale: %s' % exc, file=sys.stderr)
+        sys.exit(2)
     params = Parameters(args)
     rank, world, _ = pdist.init_from_env()
     model = Model().load(args.model)
@@ -180,7 +191,14 @@ def test(args):
     evaluator.aggregate_inject = 0 in mine           # the concatenated vectors carry ONE injection
     save_confidence = bool(getattr(args, 'save_confidence', False))
     seg = TiledSegmenter(model, batch_tiles=getattr(args, 'batch_tiles', 32), keep_masks=True,
-                         stitch=getattr(args, 'stitch', 'reference'), confidence=save_confidence)
+                         stitch=getattr(args, 'stitch', 'reference'), confidence=save_confidence,
+                         scales=multiscale)
+
+    def save_metrics():
+        if seg.scales is not None:                    # a multi-scale run records its scales with the scores
+            evaluator.metrics.results['multiscale'] = list(seg.scales)
+        evaluator.save_metrics()
+
     def decode(i):
         fpair = files[i]
         img_file, mask_file = (fpair['img'], fpair['mask']) if isinstance(fpair, dict) else (fpair, None)
@@ -205,7 +223,8 @@ def test(args):
             evaluator.save_confidence()
         if mask_file and not params.aggregate_metrics:
             print("\nStarting evaluation ... ")
-            evaluator.evaluate().save_metrics()
+            evaluator.evaluate()
+            save_metrics()
         if getattr(args, 'save_logits', False):
             print('--save_logits: logits stay on the device in this implementation; saving the label map instead.')
             evaluator.save_logits([res["labels"].cpu()])
@@ -213,7 +232,7 @@ def test(args):
     if getattr(args, 'aggregate_metrics', False):
         evaluator.evaluate(aggregate=True, distributed=world > 1)
         if rank == 0:
-            evaluator.save_metrics()
+            save_metrics()
     return evaluator
 
 
@@ -291,6 +310,9 @@ def get_parser():
                         "tiles' softmaxes ('mean').")
     p.add_argument('--save_confidence', action='store_true',
                    help='Write full-resolution confidence PNGs (255 = 1.0); with masks, add calibration (ECE) to the metrics.')
+    p.add_argument('--multiscale', type=float, nargs='+', default=None, metavar='S',
+                   help='Average the class probabilities over these image scales (relative to the --scale image, at '
+                        'most 8, no duplicates); needs --stitch mean.')
     return parser
 
 
