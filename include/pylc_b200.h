@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define PYLC_ABI_VERSION 4
+#define PYLC_ABI_VERSION 5
 #define PYLC_MAX_CLASSES 32
 
 #define PYLC_OK 0
@@ -309,6 +309,27 @@ PYLC_API int pylc_stitch_upsample_probs(const float *const *decoder_batches, int
                                int C, int T, int S, int hs, int ws, int mode, const uint8_t *lut_rgb,
                                uint8_t *labels, uint8_t *rgb, uint8_t *confidence, float *stitched, pylc_stream_t stream);
 
+/*
+ * Temperature-scaled probabilities (post-hoc calibration): pylc_stitch_probs / pylc_stitch_upsample_probs with every
+ * tile softmax taken of L / temperature.  In PYLC_STITCH_MEAN mode every softmax of the stitch is a softmax of raw
+ * tile logits, so the kernels evaluate it with k_T = f32(log2(e) / f32(temperature)) in place of log2(e):
+ *     P_T(y, x) = the mean over the covering tiles of softmax(L / T),  labels = first argmax of P_T,
+ *     confidence = min(255, round-to-nearest(P_T[label] * 255)),  stitched = P_T.
+ * At temperature 1 every output equals the untempered call bit for bit.  Labels in overlap zones may change with T:
+ * the argmax of a mean of softmaxes depends on the temperature.
+ * PYLC_ERR_ARG for a temperature that is not finite and > 0, or other than 1 in PYLC_STITCH_REFERENCE mode (that
+ * mode mixes raw-logit corners, a second softmax of probability sums and labels from M: a temperature has no single
+ * meaning there).  Other arguments and return codes as the untempered calls.
+ */
+PYLC_API int pylc_stitch_probs_t(const float *logits, const float *const *tile_batches, int tiles_per_batch,
+                        int nr, int nc, int C, int T, int S, int mode, const uint8_t *lut_rgb,
+                        uint8_t *labels, uint8_t *rgb, uint8_t *confidence, float *stitched, float temperature,
+                        pylc_stream_t stream);
+PYLC_API int pylc_stitch_upsample_probs_t(const float *const *decoder_batches, int tiles_per_batch, int nr, int nc,
+                                 int C, int T, int S, int hs, int ws, int mode, const uint8_t *lut_rgb,
+                                 uint8_t *labels, uint8_t *rgb, uint8_t *confidence, float *stitched, float temperature,
+                                 pylc_stream_t stream);
+
 /* ---- evaluation --------------------------------------------------------------------------- */
 
 /*
@@ -355,6 +376,27 @@ PYLC_API int pylc_confidence_resample(const uint8_t *confidence, int h, int w, c
                              const int32_t *y_ofs, int h_full, int w_full, const uint8_t *y_pred_full,
                              const uint8_t *y_true_full, int C, uint8_t *confidence_full, int64_t *reliability,
                              pylc_stream_t stream);
+
+/*
+ * Proper scores of mean-mode probabilities against the ground truth at full resolution (temperature fitting).
+ *   probs         [C, h, w] f32, the `stitched` output of a PYLC_STITCH_MEAN stitch
+ *   x_ofs / y_ofs [w_full] / [h_full] i32, the label map's INTER_NEAREST index maps (as pylc_resample_encode_confusion
+ *                 takes them).  PRECONDITION, not checked on the device: every value lies in [0, w) / [0, h)
+ *   y_true_full   [h_full, w_full] u8 encoded true classes (gt_full of pylc_resample_encode_confusion: unmatched
+ *                 colours are class 1), any alignment.  A class >= C is scored as probability 0 for it.
+ *   want_brier    0: NLL only (one plane read per pixel); 1: also the Brier score (all C planes)
+ *   workspace     [PYLC_SCORES_WS_DOUBLES] f64 scratch
+ *   sums          [2] f64, OVERWRITTEN: {sum of nll, sum of brier (0 without want_brier)} over all h_full * w_full
+ *                 pixels, where per pixel, in f32, with g its class and q = P[g][y_ofs[y]][x_ofs[x]]:
+ *                     nll = -logf(fmaxf(q, 1e-12f)),  brier = sum over c in class order of (P[c] - [c == g])^2
+ * Each pixel is added in f64 and the sums are reduced in a fixed order: the same inputs give the same bits on every
+ * call.  Two launches.  PYLC_ERR_ARG for a null pointer or a non-positive size; PYLC_ERR_CLASSES for C outside [1, 32].
+ */
+#define PYLC_SCORES_BLOCKS 1024
+#define PYLC_SCORES_WS_DOUBLES (2 * PYLC_SCORES_BLOCKS)
+PYLC_API int pylc_prob_scores(const float *probs, int C, int h, int w, const int32_t *x_ofs, const int32_t *y_ofs,
+                     int h_full, int w_full, const uint8_t *y_true_full, int want_brier, double *workspace,
+                     double *sums, pylc_stream_t stream);
 
 /*
  * Multi-scale combine (an extension): the mean-mode probability maps of K image scales averaged on one output grid.

@@ -16,6 +16,12 @@
 // PYLC_STITCH_REFERENCE (0) takes the first argmax of M (the reference's labels), PYLC_STITCH_MEAN (1) that
 // of P, and then `stitched` holds P instead of M.  CONF adds the u8 plane q = min(255, rn(P[label] * 255)).
 // MODE = 0 without CONF is the code the argmax / colour entry points have always run.
+//
+// Temperature (pylc_stitch_probs_t): in mean mode every softmax the kernels evaluate is a softmax of raw tile
+// logits, so softmax(L / T) is exp_cls with k = fl32(log2(e) / T) in place of log2(e).  The mean-mode
+// instantiations take k from the kernel's trailing argument `k`; the reference-mode instantiations ignore it
+// and keep the compile-time constant.  `k` is a kernel argument after the existing ones rather than a field
+// of StitchArgs, so every parameter the reference-mode kernels read keeps its offset.
 #include "common.cuh"
 
 namespace pylc {
@@ -171,13 +177,13 @@ __device__ __forceinline__ void emit_unit(const StitchArgs &a, const uint32_t *s
 
 // P of a corner block (or of any block when S == T): softmax of the raw logits, e[c] * (1 / sum).
 template <int CMAX, int PX>
-__device__ __forceinline__ void softmax_copy(const float (&v)[CMAX][PX], int C, float (&p)[CMAX][PX]) {
+__device__ __forceinline__ void softmax_copy(const float (&v)[CMAX][PX], int C, float k, float (&p)[CMAX][PX]) {
 #pragma unroll
     for (int c = 0; c < CMAX; ++c)
 #pragma unroll
         for (int j = 0; j < PX; ++j) p[c][j] = v[c][j];
     float r[PX];
-    exp_cls<CMAX, PX, true>(p, C, kLog2e, r);
+    exp_cls<CMAX, PX, true>(p, C, k, r);
 #pragma unroll
     for (int c = 0; c < CMAX; ++c)
 #pragma unroll
@@ -197,9 +203,10 @@ __device__ __forceinline__ void quarter_sum(const float (&s0)[CMAX][PX], const f
 
 // NH: tiles per strip (1 border / 2 interior columns); NV: strips (1 border / 2 interior rows)
 template <int C_T, int CMAX, int PX, int NH, int NV, int MODE, bool CONF>
-__device__ __forceinline__ void stitch_units(const StitchArgs &a, const uint32_t *s_lut, uint8_t *conf, int ky, int kx, int row0,
-                                             int nrows) {
+__device__ __forceinline__ void stitch_units(const StitchArgs &a, const uint32_t *s_lut, uint8_t *conf, float k, int ky, int kx,
+                                             int row0, int nrows) {
     const int C = C_T > 0 ? C_T : a.C;
+    const float kl = MODE == 1 ? k : kLog2e;     // scale of every raw-logit softmax: log2(e) / temperature
     const int T = a.T, S = a.S;
     const size_t cstride = (size_t)T * T;
     // source tiles: strip s in {0,1} x column q in {0,1}
@@ -252,23 +259,23 @@ __device__ __forceinline__ void stitch_units(const StitchArgs &a, const uint32_t
 #pragma unroll
             for (int s = 0; s < NV; ++s) {
                 float r0[PX], r1[PX];
-                exp_cls<CMAX, PX, true>(v[s][0], C, kLog2e, r0);
-                exp_cls<CMAX, PX, true>(v[s][1], C, kLog2e, r1);
+                exp_cls<CMAX, PX, true>(v[s][0], C, kl, r0);
+                exp_cls<CMAX, PX, true>(v[s][1], C, kl, r1);
                 combine_cls<CMAX, PX>(v[s][0], r0, v[s][1], r1, C, NV == 2 ? 1.f : 0.5f);
             }
         }
         constexpr bool NEED_P = MODE == 1 || CONF;
         float p[CMAX][PX];          // P where it is not M itself (interior and corner blocks)
         if constexpr (NEED_P && NV == 2 && NH == 2) quarter_sum<CMAX, PX>(v[0][0], v[NV - 1][0], C, p);
-        if constexpr (NEED_P && NV == 1 && NH == 1) softmax_copy<CMAX, PX>(v[0][0], C, p);
+        if constexpr (NEED_P && NV == 1 && NH == 1) softmax_copy<CMAX, PX>(v[0][0], C, kl, p);
         if (NV == 2 && !(MODE == 1 && NH == 2)) {     // mean mode needs no second softmax in the interior
             float r0[PX], r1[PX];
             if (NH == 2) {   // inputs: sums of two probability vectors, in [0, 2]
                 exp_cls<CMAX, PX, false>(v[0][0], C, 0.5f * kLog2e, r0);
                 exp_cls<CMAX, PX, false>(v[NV - 1][0], C, 0.5f * kLog2e, r1);
             } else {         // left / right border: raw logits
-                exp_cls<CMAX, PX, true>(v[0][0], C, kLog2e, r0);
-                exp_cls<CMAX, PX, true>(v[NV - 1][0], C, kLog2e, r1);
+                exp_cls<CMAX, PX, true>(v[0][0], C, kl, r0);
+                exp_cls<CMAX, PX, true>(v[NV - 1][0], C, kl, r1);
             }
             combine_cls<CMAX, PX>(v[0][0], r0, v[NV - 1][0], r1, C, 0.5f);
         }
@@ -282,7 +289,8 @@ __device__ __forceinline__ void stitch_units(const StitchArgs &a, const uint32_t
 }
 
 template <int C_T, int CMAX, int PX, int MODE = 0, bool CONF = false>
-__global__ void __launch_bounds__(kThreads, 2) stitch_kernel(StitchArgs a, const __grid_constant__ ColourLut lut, uint8_t *conf) {
+__global__ void __launch_bounds__(kThreads, 2) stitch_kernel(StitchArgs a, const __grid_constant__ ColourLut lut, uint8_t *conf,
+                                                             float k) {
     __shared__ uint32_t s_lut[PYLC_MAX_CLASSES];
     if (threadIdx.x < PYLC_MAX_CLASSES) s_lut[threadIdx.x] = lut.rgb[threadIdx.x];
     __syncthreads();
@@ -299,11 +307,11 @@ __global__ void __launch_bounds__(kThreads, 2) stitch_kernel(StitchArgs a, const
     const bool two_h = a.overlap && kx > 0 && kx < a.nc;
     const bool two_v = a.overlap && ky > 0 && ky < a.nr;
     if (two_h) {
-        if (two_v) stitch_units<C_T, CMAX, PX, 2, 2, MODE, CONF>(a, s_lut, conf, ky, kx, slab * a.rows_per_cta, a.rows_per_cta);
-        else stitch_units<C_T, CMAX, PX, 2, 1, MODE, CONF>(a, s_lut, conf, ky, kx, slab * a.rows_per_cta, a.rows_per_cta);
+        if (two_v) stitch_units<C_T, CMAX, PX, 2, 2, MODE, CONF>(a, s_lut, conf, k, ky, kx, slab * a.rows_per_cta, a.rows_per_cta);
+        else stitch_units<C_T, CMAX, PX, 2, 1, MODE, CONF>(a, s_lut, conf, k, ky, kx, slab * a.rows_per_cta, a.rows_per_cta);
     } else {
-        if (two_v) stitch_units<C_T, CMAX, PX, 1, 2, MODE, CONF>(a, s_lut, conf, ky, kx, slab * a.rows_per_cta, a.rows_per_cta);
-        else stitch_units<C_T, CMAX, PX, 1, 1, MODE, CONF>(a, s_lut, conf, ky, kx, slab * a.rows_per_cta, a.rows_per_cta);
+        if (two_v) stitch_units<C_T, CMAX, PX, 1, 2, MODE, CONF>(a, s_lut, conf, k, ky, kx, slab * a.rows_per_cta, a.rows_per_cta);
+        else stitch_units<C_T, CMAX, PX, 1, 1, MODE, CONF>(a, s_lut, conf, k, ky, kx, slab * a.rows_per_cta, a.rows_per_cta);
     }
 }
 
@@ -338,10 +346,11 @@ struct StitchUpArgs {
 };
 
 template <int C_T, int CMAX, int NH, int NV, int MODE, bool CONF>
-__device__ __forceinline__ void stitch_up_units(const StitchUpArgs &a, const uint32_t *s_lut, uint8_t *conf, float *s_src, int ky, int kx,
-                                                int row0) {
+__device__ __forceinline__ void stitch_up_units(const StitchUpArgs &a, const uint32_t *s_lut, uint8_t *conf, float k, float *s_src, int ky,
+                                                int kx, int row0) {
     constexpr int PX = 2;
     const int C = C_T > 0 ? C_T : a.C;
+    const float kl = MODE == 1 ? k : kLog2e;     // as in stitch_units
     const int T = a.T, S = a.S, hs = a.hs, ws = a.ws;
     const float rh = (float)(hs - 1) / (float)(T - 1), rw = (float)(ws - 1) / (float)(T - 1);
     int ti[2], ty0[2], tj[2], tx0[2];
@@ -463,8 +472,8 @@ __device__ __forceinline__ void stitch_up_units(const StitchUpArgs &a, const uin
             }
             if (NH == 2) {
                 float r0[PX], r1[PX];
-                exp_cls<CMAX, PX, true>(v[0], C, kLog2e, r0);
-                exp_cls<CMAX, PX, true>(v[NH - 1], C, kLog2e, r1);
+                exp_cls<CMAX, PX, true>(v[0], C, kl, r0);
+                exp_cls<CMAX, PX, true>(v[NH - 1], C, kl, r1);
                 combine_cls<CMAX, PX>(v[0], r0, v[NH - 1], r1, C, NV == 2 ? 1.f : 0.5f);
             }
 #pragma unroll
@@ -475,15 +484,15 @@ __device__ __forceinline__ void stitch_up_units(const StitchUpArgs &a, const uin
         constexpr bool NEED_P = MODE == 1 || CONF;     // P as in stitch_units
         float p[CMAX][PX];
         if constexpr (NEED_P && NV == 2 && NH == 2) quarter_sum<CMAX, PX>(strip[0], strip[NV - 1], C, p);
-        if constexpr (NEED_P && NV == 1 && NH == 1) softmax_copy<CMAX, PX>(strip[0], C, p);
+        if constexpr (NEED_P && NV == 1 && NH == 1) softmax_copy<CMAX, PX>(strip[0], C, kl, p);
         if (NV == 2 && !(MODE == 1 && NH == 2)) {
             float r0[PX], r1[PX];
             if (NH == 2) {
                 exp_cls<CMAX, PX, false>(strip[0], C, 0.5f * kLog2e, r0);
                 exp_cls<CMAX, PX, false>(strip[NV - 1], C, 0.5f * kLog2e, r1);
             } else {
-                exp_cls<CMAX, PX, true>(strip[0], C, kLog2e, r0);
-                exp_cls<CMAX, PX, true>(strip[NV - 1], C, kLog2e, r1);
+                exp_cls<CMAX, PX, true>(strip[0], C, kl, r0);
+                exp_cls<CMAX, PX, true>(strip[NV - 1], C, kl, r1);
             }
             combine_cls<CMAX, PX>(strip[0], r0, strip[NV - 1], r1, C, 0.5f);
         }
@@ -499,7 +508,8 @@ __device__ __forceinline__ void stitch_up_units(const StitchUpArgs &a, const uin
 }
 
 template <int C_T, int CMAX, int MODE = 0, bool CONF = false>
-__global__ void __launch_bounds__(kThreads, 2) stitch_up_kernel(StitchUpArgs a, const __grid_constant__ ColourLut lut, uint8_t *conf) {
+__global__ void __launch_bounds__(kThreads, 2) stitch_up_kernel(StitchUpArgs a, const __grid_constant__ ColourLut lut, uint8_t *conf,
+                                                                float k) {
     extern __shared__ __align__(16) float s_up[];
     __shared__ uint32_t s_lut[PYLC_MAX_CLASSES];
     if (threadIdx.x < PYLC_MAX_CLASSES) s_lut[threadIdx.x] = lut.rgb[threadIdx.x];
@@ -512,11 +522,11 @@ __global__ void __launch_bounds__(kThreads, 2) stitch_up_kernel(StitchUpArgs a, 
     const bool two_h = a.overlap && kx > 0 && kx < a.nc;
     const bool two_v = a.overlap && ky > 0 && ky < a.nr;
     if (two_h) {
-        if (two_v) stitch_up_units<C_T, CMAX, 2, 2, MODE, CONF>(a, s_lut, conf, s_up, ky, kx, slab * kUpR);
-        else stitch_up_units<C_T, CMAX, 2, 1, MODE, CONF>(a, s_lut, conf, s_up, ky, kx, slab * kUpR);
+        if (two_v) stitch_up_units<C_T, CMAX, 2, 2, MODE, CONF>(a, s_lut, conf, k, s_up, ky, kx, slab * kUpR);
+        else stitch_up_units<C_T, CMAX, 2, 1, MODE, CONF>(a, s_lut, conf, k, s_up, ky, kx, slab * kUpR);
     } else {
-        if (two_v) stitch_up_units<C_T, CMAX, 1, 2, MODE, CONF>(a, s_lut, conf, s_up, ky, kx, slab * kUpR);
-        else stitch_up_units<C_T, CMAX, 1, 1, MODE, CONF>(a, s_lut, conf, s_up, ky, kx, slab * kUpR);
+        if (two_v) stitch_up_units<C_T, CMAX, 1, 2, MODE, CONF>(a, s_lut, conf, k, s_up, ky, kx, slab * kUpR);
+        else stitch_up_units<C_T, CMAX, 1, 1, MODE, CONF>(a, s_lut, conf, k, s_up, ky, kx, slab * kUpR);
     }
 }
 
@@ -528,24 +538,32 @@ using namespace pylc;
 // mode 0 without confidence, the kernels they have always launched.
 template <int MODE, bool CONF>
 static void launch_stitch(bool px2, int C, unsigned grid, cudaStream_t st, const StitchArgs &a, const ColourLut &lut,
-                          uint8_t *conf) {
+                          uint8_t *conf, float k) {
     if (px2) {
-        if (C == 9) stitch_kernel<9, 9, 2, MODE, CONF><<<grid, kThreads, 0, st>>>(a, lut, conf);
-        else if (C == 11) stitch_kernel<11, 11, 2, MODE, CONF><<<grid, kThreads, 0, st>>>(a, lut, conf);
-        else if (C <= 4) stitch_kernel<0, 4, 2, MODE, CONF><<<grid, kThreads, 0, st>>>(a, lut, conf);
-        else if (C <= 8) stitch_kernel<0, 8, 2, MODE, CONF><<<grid, kThreads, 0, st>>>(a, lut, conf);
-        else stitch_kernel<0, 12, 2, MODE, CONF><<<grid, kThreads, 0, st>>>(a, lut, conf);
+        if (C == 9) stitch_kernel<9, 9, 2, MODE, CONF><<<grid, kThreads, 0, st>>>(a, lut, conf, k);
+        else if (C == 11) stitch_kernel<11, 11, 2, MODE, CONF><<<grid, kThreads, 0, st>>>(a, lut, conf, k);
+        else if (C <= 4) stitch_kernel<0, 4, 2, MODE, CONF><<<grid, kThreads, 0, st>>>(a, lut, conf, k);
+        else if (C <= 8) stitch_kernel<0, 8, 2, MODE, CONF><<<grid, kThreads, 0, st>>>(a, lut, conf, k);
+        else stitch_kernel<0, 12, 2, MODE, CONF><<<grid, kThreads, 0, st>>>(a, lut, conf, k);
     } else {
-        if (C <= 12) stitch_kernel<0, 12, 1, MODE, CONF><<<grid, kThreads, 0, st>>>(a, lut, conf);
-        else if (C <= 16) stitch_kernel<0, 16, 1, MODE, CONF><<<grid, kThreads, 0, st>>>(a, lut, conf);
-        else stitch_kernel<0, 32, 1, MODE, CONF><<<grid, kThreads, 0, st>>>(a, lut, conf);
+        if (C <= 12) stitch_kernel<0, 12, 1, MODE, CONF><<<grid, kThreads, 0, st>>>(a, lut, conf, k);
+        else if (C <= 16) stitch_kernel<0, 16, 1, MODE, CONF><<<grid, kThreads, 0, st>>>(a, lut, conf, k);
+        else stitch_kernel<0, 32, 1, MODE, CONF><<<grid, kThreads, 0, st>>>(a, lut, conf, k);
     }
+}
+
+// A temperature is finite and > 0, and other than 1 only for the mean stitch: reference mode mixes raw-logit
+// corners, a second softmax of probability sums and labels from M, so a temperature has no single meaning there.
+static bool temperature_ok(float temperature, int mode) {
+    if (!(temperature > 0.f) || !isfinite(temperature)) return false;
+    return mode == PYLC_STITCH_MEAN || temperature == 1.f;
 }
 
 static int stitch_launch(const float *logits, const float *const *tile_batches, int tiles_per_batch, int nr, int nc, int C,
                          int T, int S, int mode, const uint8_t *lut_rgb, uint8_t *labels, uint8_t *rgb, uint8_t *confidence,
-                         float *stitched, pylc_stream_t stream) {
+                         float *stitched, float temperature, pylc_stream_t stream) {
     if ((!logits && !tile_batches) || nr < 1 || nc < 1 || T < 1 || S < 1) return PYLC_ERR_ARG;
+    if (!temperature_ok(temperature, mode)) return PYLC_ERR_ARG;
     if (!logits && tiles_per_batch < 1) return PYLC_ERR_ARG;
     if (rgb && !lut_rgb) return PYLC_ERR_ARG;
     if (mode != PYLC_STITCH_REFERENCE && mode != PYLC_STITCH_MEAN) return PYLC_ERR_ARG;
@@ -582,11 +600,12 @@ static int stitch_launch(const float *logits, const float *const *tile_batches, 
     const unsigned grid = (unsigned)((long long)a.nbx * a.nby * a.slabs);
     cudaStream_t st = (cudaStream_t)stream;
     if (mode == PYLC_STITCH_MEAN) {
-        if (confidence) launch_stitch<1, true>(px2, C, grid, st, a, lut, confidence);
-        else launch_stitch<1, false>(px2, C, grid, st, a, lut, nullptr);
+        const float k = kLog2e / temperature;
+        if (confidence) launch_stitch<1, true>(px2, C, grid, st, a, lut, confidence, k);
+        else launch_stitch<1, false>(px2, C, grid, st, a, lut, nullptr, k);
     } else {
-        if (confidence) launch_stitch<0, true>(px2, C, grid, st, a, lut, confidence);
-        else launch_stitch<0, false>(px2, C, grid, st, a, lut, nullptr);
+        if (confidence) launch_stitch<0, true>(px2, C, grid, st, a, lut, confidence, kLog2e);
+        else launch_stitch<0, false>(px2, C, grid, st, a, lut, nullptr, kLog2e);
     }
     return finish_launch();
 }
@@ -595,24 +614,31 @@ extern "C" int pylc_stitch_argmax_colour(const float *logits, const float *const
                                          int nr, int nc, int C, int T, int S, const uint8_t *lut_rgb,
                                          uint8_t *labels, uint8_t *rgb, float *stitched, pylc_stream_t stream) {
     return stitch_launch(logits, tile_batches, tiles_per_batch, nr, nc, C, T, S, PYLC_STITCH_REFERENCE, lut_rgb, labels, rgb,
-                         nullptr, stitched, stream);
+                         nullptr, stitched, 1.f, stream);
 }
 
 extern "C" int pylc_stitch_probs(const float *logits, const float *const *tile_batches, int tiles_per_batch, int nr, int nc,
                                  int C, int T, int S, int mode, const uint8_t *lut_rgb, uint8_t *labels, uint8_t *rgb,
                                  uint8_t *confidence, float *stitched, pylc_stream_t stream) {
     return stitch_launch(logits, tile_batches, tiles_per_batch, nr, nc, C, T, S, mode, lut_rgb, labels, rgb, confidence,
-                         stitched, stream);
+                         stitched, 1.f, stream);
+}
+
+extern "C" int pylc_stitch_probs_t(const float *logits, const float *const *tile_batches, int tiles_per_batch, int nr, int nc,
+                                   int C, int T, int S, int mode, const uint8_t *lut_rgb, uint8_t *labels, uint8_t *rgb,
+                                   uint8_t *confidence, float *stitched, float temperature, pylc_stream_t stream) {
+    return stitch_launch(logits, tile_batches, tiles_per_batch, nr, nc, C, T, S, mode, lut_rgb, labels, rgb, confidence,
+                         stitched, temperature, stream);
 }
 
 template <int MODE, bool CONF>
 static int launch_stitch_up(int C, unsigned grid, size_t smem, cudaStream_t st, const StitchUpArgs &a, const ColourLut &lut,
-                            uint8_t *conf) {
+                            uint8_t *conf, float k) {
 #define LAUNCH_UP(CT, CM)                                                                                                  \
     do {                                                                                                                   \
         cudaError_t e = cudaFuncSetAttribute(stitch_up_kernel<CT, CM, MODE, CONF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
         if (e != cudaSuccess) return (int)e;                                                                               \
-        stitch_up_kernel<CT, CM, MODE, CONF><<<grid, kThreads, smem, st>>>(a, lut, conf);                                     \
+        stitch_up_kernel<CT, CM, MODE, CONF><<<grid, kThreads, smem, st>>>(a, lut, conf, k);                                  \
     } while (0)
     if (C == 9) LAUNCH_UP(9, 9);
     else if (C == 11) LAUNCH_UP(11, 11);
@@ -625,8 +651,9 @@ static int launch_stitch_up(int C, unsigned grid, size_t smem, cudaStream_t st, 
 
 static int stitch_up_launch(const float *const *decoder_batches, int tiles_per_batch, int nr, int nc, int C, int T, int S,
                             int hs, int ws, int mode, const uint8_t *lut_rgb, uint8_t *labels, uint8_t *rgb,
-                            uint8_t *confidence, float *stitched, pylc_stream_t stream) {
+                            uint8_t *confidence, float *stitched, float temperature, pylc_stream_t stream) {
     if (!decoder_batches || tiles_per_batch < 1 || nr < 1 || nc < 1 || T < 1 || S < 1 || hs < 2 || ws < 2) return PYLC_ERR_ARG;
+    if (!temperature_ok(temperature, mode)) return PYLC_ERR_ARG;
     if (rgb && !lut_rgb) return PYLC_ERR_ARG;
     if (mode != PYLC_STITCH_REFERENCE && mode != PYLC_STITCH_MEAN) return PYLC_ERR_ARG;
     if (C < 1 || C > PYLC_MAX_CLASSES) return PYLC_ERR_CLASSES;
@@ -655,9 +682,11 @@ static int stitch_up_launch(const float *const *decoder_batches, int tiles_per_b
     const unsigned grid = (unsigned)((long long)a.nbx * a.nby * a.slabs);
     cudaStream_t st = (cudaStream_t)stream;
     int rc;
-    if (mode == PYLC_STITCH_MEAN) rc = confidence ? launch_stitch_up<1, true>(C, grid, smem, st, a, lut, confidence)
-                                                  : launch_stitch_up<1, false>(C, grid, smem, st, a, lut, nullptr);
-    else rc = confidence ? launch_stitch_up<0, true>(C, grid, smem, st, a, lut, confidence) : launch_stitch_up<0, false>(C, grid, smem, st, a, lut, nullptr);
+    const float k = kLog2e / temperature;           // exactly kLog2e at T = 1; unused in reference mode
+    if (mode == PYLC_STITCH_MEAN) rc = confidence ? launch_stitch_up<1, true>(C, grid, smem, st, a, lut, confidence, k)
+                                                  : launch_stitch_up<1, false>(C, grid, smem, st, a, lut, nullptr, k);
+    else rc = confidence ? launch_stitch_up<0, true>(C, grid, smem, st, a, lut, confidence, kLog2e)
+                         : launch_stitch_up<0, false>(C, grid, smem, st, a, lut, nullptr, kLog2e);
     if (rc) return rc;
     return finish_launch();
 }
@@ -666,12 +695,20 @@ extern "C" int pylc_stitch_upsample_argmax_colour(const float *const *decoder_ba
                                                   int T, int S, int hs, int ws, const uint8_t *lut_rgb, uint8_t *labels,
                                                   uint8_t *rgb, float *stitched, pylc_stream_t stream) {
     return stitch_up_launch(decoder_batches, tiles_per_batch, nr, nc, C, T, S, hs, ws, PYLC_STITCH_REFERENCE, lut_rgb, labels,
-                            rgb, nullptr, stitched, stream);
+                            rgb, nullptr, stitched, 1.f, stream);
 }
 
 extern "C" int pylc_stitch_upsample_probs(const float *const *decoder_batches, int tiles_per_batch, int nr, int nc, int C,
                                           int T, int S, int hs, int ws, int mode, const uint8_t *lut_rgb, uint8_t *labels,
                                           uint8_t *rgb, uint8_t *confidence, float *stitched, pylc_stream_t stream) {
     return stitch_up_launch(decoder_batches, tiles_per_batch, nr, nc, C, T, S, hs, ws, mode, lut_rgb, labels, rgb, confidence,
-                            stitched, stream);
+                            stitched, 1.f, stream);
+}
+
+extern "C" int pylc_stitch_upsample_probs_t(const float *const *decoder_batches, int tiles_per_batch, int nr, int nc, int C,
+                                            int T, int S, int hs, int ws, int mode, const uint8_t *lut_rgb, uint8_t *labels,
+                                            uint8_t *rgb, uint8_t *confidence, float *stitched, float temperature,
+                                            pylc_stream_t stream) {
+    return stitch_up_launch(decoder_batches, tiles_per_batch, nr, nc, C, T, S, hs, ws, mode, lut_rgb, labels, rgb, confidence,
+                            stitched, temperature, stream);
 }

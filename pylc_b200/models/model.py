@@ -127,6 +127,7 @@ class Model:
             else torch.device(self.meta.device)
         self.net = None
         self.model_path = None
+        self.calibration = None     # the model file's "calibration" entry (pylc calibrate), None when it has none
         self.iter = 0
         self.crit = None
         self.loss = None
@@ -162,6 +163,7 @@ class Model:
         assert 'meta' in model_data, '\nLoaded model missing metadata attribute.'
         self.meta.update(model_data["meta"] if isinstance(model_data["meta"], dict) else vars(model_data["meta"]))
         self.meta.pretrained = False
+        self.calibration = model_data.get("calibration")
         self.build()
         self.net.load_state_dict(strip_module_prefix(model_data["model"]))
         return self

@@ -405,11 +405,13 @@ def _prob_outputs(C, h, w, dev, want_labels, want_rgb, want_confidence, want_pro
 
 
 def stitch_probs(logits, nr, nc, T, S, mode="reference", lut_rgb=None, want_labels=True, want_rgb=False,
-                 want_confidence=True, want_probs=False, tiles_per_batch=None, out=None):
-    """pylc_stitch_probs: the stitch of stitch_argmax_colour with per-pixel probabilities.
+                 want_confidence=True, want_probs=False, tiles_per_batch=None, out=None, temperature=1.0):
+    """pylc_stitch_probs_t: the stitch of stitch_argmax_colour with per-pixel probabilities.
     P = the mean over the covering tiles of their softmaxes.  mode "reference": labels / rgb are those of
     stitch_argmax_colour and `probs` is the reference's merged map M; mode "mean": labels = argmax P and
     `probs` = P.  `confidence` is the u8 plane round(P[label] * 255) in both modes.
+    `temperature` (mean mode only; PylcError otherwise unless 1): every tile softmax is softmax(L / temperature);
+    1 gives the untempered outputs bit for bit.
     `out`: optional dict of preallocated outputs (any of labels / rgb / confidence / probs).
     Returns dict(labels, rgb, confidence, probs), entries None where not wanted."""
     lib = _lib.load()
@@ -418,27 +420,29 @@ def stitch_probs(logits, nr, nc, T, S, mode="reference", lut_rgb=None, want_labe
     h, w = stitch_dims(nr, nc, T, S)
     res = _prob_outputs(C, h, w, dev, want_labels, want_rgb, want_confidence, want_probs, out)
     pal = _lut_for(lut_rgb, C, "logits have")
-    check(lib.pylc_stitch_probs(lp, bp, tpb, nr, nc, C, T, S, m, pal, _p(res["labels"]), _p(res["rgb"]),
-                                _p(res["confidence"]), _p(res["probs"]), _stream()), "pylc_stitch_probs")
+    check(lib.pylc_stitch_probs_t(lp, bp, tpb, nr, nc, C, T, S, m, pal, _p(res["labels"]), _p(res["rgb"]),
+                                  _p(res["confidence"]), _p(res["probs"]), float(temperature), _stream()),
+          "pylc_stitch_probs_t")
     if batch_table is not None:
         batch_table.record_stream(torch.cuda.current_stream())
     return res
 
 
 def stitch_upsample_probs(decoder_batches, nr, nc, T, S, mode="reference", lut_rgb=None, want_labels=True,
-                          want_rgb=False, want_confidence=True, want_probs=False, tiles_per_batch=None, out=None):
-    """pylc_stitch_upsample_probs: stitch_probs straight from the decoder's channels-last outputs (the fused
+                          want_rgb=False, want_confidence=True, want_probs=False, tiles_per_batch=None, out=None,
+                          temperature=1.0):
+    """pylc_stitch_upsample_probs_t: stitch_probs straight from the decoder's channels-last outputs (the fused
     x4 up-sample of stitch_upsample_argmax_colour), bit-identical to
-    stitch_probs(upsample_nhwc_to_nchw(batch) ...).  Returns dict(labels, rgb, confidence, probs)."""
+    stitch_probs(upsample_nhwc_to_nchw(batch) ..., temperature=...).  Returns dict(labels, rgb, confidence, probs)."""
     lib = _lib.load()
     m = _stitch_mode(mode)
     batch_table, tpb, C, hs, ws, dev = _decoder_source(decoder_batches, nr, nc, tiles_per_batch)
     h, w = stitch_dims(nr, nc, T, S)
     res = _prob_outputs(C, h, w, dev, want_labels, want_rgb, want_confidence, want_probs, out)
     pal = _lut_for(lut_rgb, C, "the decoder output has")
-    check(lib.pylc_stitch_upsample_probs(_p(batch_table), tpb, nr, nc, C, T, S, hs, ws, m, pal, _p(res["labels"]),
-                                         _p(res["rgb"]), _p(res["confidence"]), _p(res["probs"]), _stream()),
-          "pylc_stitch_upsample_probs")
+    check(lib.pylc_stitch_upsample_probs_t(_p(batch_table), tpb, nr, nc, C, T, S, hs, ws, m, pal, _p(res["labels"]),
+                                           _p(res["rgb"]), _p(res["confidence"]), _p(res["probs"]), float(temperature),
+                                           _stream()), "pylc_stitch_upsample_probs_t")
     batch_table.record_stream(torch.cuda.current_stream())
     return res
 
@@ -570,6 +574,30 @@ def _checked_index_maps(w, h, w_full, h_full, device):
                 raise PylcError("index map %d -> %d leaves its plane" % (src, dst))
         _CHECKED_MAPS.add(key)
     return device_index_maps(w, h, w_full, h_full, device)
+
+
+def prob_scores(probs, y_true_full, w_full, h_full, want_brier=True, maps=None, workspace=None):
+    """pylc_prob_scores: [2] f64 CUDA tensor {sum of -log(max(P[g], 1e-12)), sum of the Brier score} over the
+    h_full x w_full pixels of `y_true_full` (u8 encoded classes), P = the mean-mode `probs` [C, h, w] sampled with
+    the label map's INTER_NEAREST index maps (`maps`, default device_index_maps).  The Brier entry is 0 without
+    `want_brier`.  Deterministic: the same inputs give the same bits.  `workspace`: optional f64 scratch of
+    _lib.SCORES_WS_DOUBLES entries, reused across calls on one stream."""
+    _need_cuda(probs, y_true_full)
+    if probs.dtype != torch.float32 or probs.dim() != 3 or not probs.is_contiguous():
+        raise PylcError("prob_scores takes a contiguous [C, h, w] float32 map")
+    if y_true_full.dtype != torch.uint8 or y_true_full.numel() != h_full * w_full or not y_true_full.is_contiguous():
+        raise PylcError("prob_scores: y_true_full must be a contiguous u8 plane of h_full * w_full pixels")
+    C, h, w = probs.shape
+    dev = probs.device
+    x_ofs, y_ofs = _checked_index_maps(w, h, w_full, h_full, dev) if maps is None else maps
+    if x_ofs.numel() != w_full or y_ofs.numel() != h_full:
+        raise PylcError("prob_scores: index maps must hold w_full / h_full entries")
+    if workspace is None:
+        workspace = torch.empty((_lib.SCORES_WS_DOUBLES,), dtype=torch.float64, device=dev)
+    sums = torch.empty((2,), dtype=torch.float64, device=dev)
+    check(_lib.load().pylc_prob_scores(_p(probs), C, h, w, _p(x_ofs), _p(y_ofs), int(h_full), int(w_full), _p(y_true_full),
+                                       1 if want_brier else 0, _p(workspace), _p(sums), _stream()), "pylc_prob_scores")
+    return sums
 
 
 def multiscale_combine(probs, w_full, h_full, lut_rgb=None, want_labels=True, want_rgb=False, want_confidence=True,

@@ -23,12 +23,15 @@ image resized by s_k (INTER_AREA) and fitted to the tiles, on the device when bo
 area filter, otherwise with cv2 on the host threads.  Each member's mean-mode probability map P_k stays on the
 device; pylc_multiscale_combine samples every P_k onto the full-resolution grid, averages them and writes the
 full-resolution labels and confidence, and pylc_resample_encode_confusion counts the confusion from those.
+With `temperature` T (post-hoc calibration, mean stitch only) every tile softmax of the mean stitch is softmax(L / T),
+in the single-scale stitch and in every multi-scale member alike (pylc_stitch_probs_t).
 With device_fit off (or for geometries OpenCV resizes with another filter) the fit-resize runs on
 host worker threads with cv2 itself and the fitted image is uploaded instead.
 Logits never leave the device.  Images are independent, so data-parallel ranks take images
 round-robin and all-reduce only the [C,C] matrix (pylc_b200.dist).
 """
 import concurrent.futures as cf
+import math
 
 import cv2
 import numpy as np
@@ -86,7 +89,7 @@ def multiscale_geometry(W, H, T, scales):
 class TiledSegmenter(object):
     def __init__(self, model, batch_tiles=32, channels_last=True, autocast_dtype=None, host_workers=4,
                  n_inject=None, keep_masks=False, fuse_network=False, device_fit=True, fuse_upsample=True,
-                 stitch="reference", confidence=False, scales=None):
+                 stitch="reference", confidence=False, scales=None, temperature=1.0):
         self.model = model
         self.meta = model.meta
         self.net = model.net.eval()
@@ -129,6 +132,11 @@ class TiledSegmenter(object):
             if stitch != "mean":
                 raise ValueError("multi-scale inference averages the mean stitch's probabilities: it needs stitch='mean'")
             self.scales = check_scales(scales)
+        self.temperature = float(temperature)     # softmax(L / T) of every tile in the mean stitch
+        if not (math.isfinite(self.temperature) and self.temperature > 0):
+            raise ValueError("temperature must be finite and > 0, got %r" % (temperature,))
+        if self.temperature != 1.0 and stitch != "mean":
+            raise ValueError("temperature scaling applies to the mean stitch's probabilities: it needs stitch='mean'")
         self.device_fit = device_fit
         self.copy_stream = torch.cuda.Stream(device=self.device)
         self.pool = cf.ThreadPoolExecutor(max_workers=host_workers)
@@ -279,26 +287,44 @@ class TiledSegmenter(object):
         return ops.tile_gather_norm_f32(img, h, w, self.ch, pitch, self.T, self.S, self.mean, self.std, self.post_div,
                                         self.out_ch)
 
-    def _stitch_probs(self, tiles, nr, nc, **kw):
-        """Network + pylc_stitch_probs (or its fused up-sample form) over one fitted image's tiles."""
-        probs = ops.stitch_upsample_probs if self.fuse_upsample else ops.stitch_probs
+    def network_output(self, tiles):
+        """The network's output for one fitted image's tiles, in the form the probability stitch reads: the list of
+        channels-last decoder batches on the fused route, else the logit batches (one tensor for a single batch)."""
         if self.fuse_upsample:
-            src = self.forward_tiles(tiles, s2d=self.s2d, decoder_only=True)
-        else:
-            src = self.forward_tiles(tiles, s2d=self.s2d)
-            src = src if len(src) > 1 else src[0]
-        return probs(src, nr, nc, self.T, self.S, mode=self.stitch, tiles_per_batch=self.batch_tiles, **kw)
+            return self.forward_tiles(tiles, s2d=self.s2d, decoder_only=True)
+        src = self.forward_tiles(tiles, s2d=self.s2d)
+        return src if len(src) > 1 else src[0]
+
+    def retained_bytes(self, nr, nc):
+        """Device bytes of network_output for an nr x nc tile grid: C * T^2 f32 per tile, 16x less on the fused
+        route, which keeps the decoder's T/4 x T/4 output."""
+        per_tile = self.C * self.T * self.T * 4
+        return nr * nc * (per_tile // 16 if self.fuse_upsample else per_tile)
+
+    def stitch_output(self, src, nr, nc, temperature=None, **kw):
+        """pylc_stitch_probs_t (or its fused up-sample form) of a network_output at `temperature` (default: the
+        segmenter's)."""
+        probs = ops.stitch_upsample_probs if self.fuse_upsample else ops.stitch_probs
+        t = self.temperature if temperature is None else temperature
+        return probs(src, nr, nc, self.T, self.S, mode=self.stitch, tiles_per_batch=self.batch_tiles, temperature=t, **kw)
+
+    def _stitch_probs(self, tiles, nr, nc, **kw):
+        """Network + probability stitch over one fitted image's tiles."""
+        return self.stitch_output(self.network_output(tiles), nr, nc, **kw)
+
+    def fitted_tiles(self, f):
+        """(tiles, nr, nc) of a single-scale FittedImage; a device-fitted image is resized here first."""
+        img, pitch = f.img, f.pitch
+        if img is None:        # device fit: INTER_AREA resize of the uploaded decoded image
+            img, pitch = ops.fit_resize_area(f.raw, f.h_full, f.w_full, self.ch, f.raw_pitch, f.h, f.w)
+        return self._tiles(img, pitch, f.h, f.w), f.h // self.S - 1, f.w // self.S - 1
 
     def segment_fitted(self, f, inject=None):
         """All device work for one fitted image; accumulates into self.conf when f.gt is set.
         Returns the fitted-resolution label map (and full-res masks when keep_masks)."""
         if self.scales is not None:
             return self._segment_multiscale(f, inject)
-        img, pitch = f.img, f.pitch
-        if img is None:        # device fit: INTER_AREA resize of the uploaded decoded image
-            img, pitch = ops.fit_resize_area(f.raw, f.h_full, f.w_full, self.ch, f.raw_pitch, f.h, f.w)
-        tiles = self._tiles(img, pitch, f.h, f.w)
-        nr, nc = f.h // self.S - 1, f.w // self.S - 1
+        tiles, nr, nc = self.fitted_tiles(f)
         conf_fit = None
         if self.stitch != "reference" or self.confidence:
             out = self._stitch_probs(tiles, nr, nc, want_confidence=self.confidence)

@@ -10,13 +10,17 @@ train.py:22-174), same sub-commands and flags for the tiled-segmentation path:
     python -m pylc_b200.pylc train   --db FILE [--batch_size N --n_epochs E --lr LR --weighted ...]
     python -m pylc_b200.pylc test    --model M --img I [--mask G] [--scale S] [--save_logits]
                                      [--aggregate_metrics] [--stitch reference|mean] [--save_confidence]
-                                     [--multiscale S1 S2 ...]   (with --stitch mean)
+                                     [--multiscale S1 S2 ...]   (with --stitch mean) [--temperature T]
+    python -m pylc_b200.pylc calibrate -l M -i I -m G [--scale S] [--batch_tiles N] [-o OUT] [--max_resident_gb G]
+                                     (fits the mean stitch's softmax temperature; writes a calibrated model copy)
 
 Launched under torchrun (WORLD_SIZE > 1), `extract`/`profile`/`test` shard images or tiles across
 the GPUs and all-reduce only histograms / confusion matrices (pylc_b200.dist).  `merge` and `grayscale`
 are stubs in the reference itself (preprocess.py:94-122: commented-out body / bare return) and are not provided.
 """
 import argparse
+import json
+import math
 import os
 import sys
 
@@ -169,7 +173,15 @@ def test(args):
     from .utils.extract import Extractor
     from .pipeline import check_scales
     multiscale = getattr(args, 'multiscale', None)
-    if multiscale and getattr(args, 'stitch', 'reference') != 'mean':
+    stitch = getattr(args, 'stitch', 'reference')
+    temperature = getattr(args, 'temperature', None)
+    if temperature is not None and not (math.isfinite(temperature) and temperature > 0):
+        print('--temperature must be finite and > 0, got %r.' % temperature, file=sys.stderr)
+        sys.exit(2)
+    if temperature is not None and stitch != 'mean':
+        print("--temperature scales the mean stitch's probabilities: add --stitch mean.", file=sys.stderr)
+        sys.exit(2)
+    if multiscale and stitch != 'mean':
         print('--multiscale averages the probabilities of the mean stitch: add --stitch mean.', file=sys.stderr)
         sys.exit(2)
     try:
@@ -183,6 +195,12 @@ def test(args):
     if rank == 0:
         model.print_settings()
     model.net.eval()
+    stored = (model.calibration or {}).get('temperature')
+    if temperature is None:              # a calibrated model file applies its temperature to the mean stitch
+        temperature = float(stored) if stored is not None and stitch == 'mean' else 1.0
+        if stored is not None and stitch != 'mean' and rank == 0:
+            print('The model is calibrated (temperature %g); the temperature is not applied with --stitch reference.'
+                  % stored)
     files = tools.collate(args.img, args.mask)
     mine = pdist.shard_indices(len(files))
     extractor = Extractor(model.meta)
@@ -191,12 +209,13 @@ def test(args):
     evaluator.aggregate_inject = 0 in mine           # the concatenated vectors carry ONE injection
     save_confidence = bool(getattr(args, 'save_confidence', False))
     seg = TiledSegmenter(model, batch_tiles=getattr(args, 'batch_tiles', 32), keep_masks=True,
-                         stitch=getattr(args, 'stitch', 'reference'), confidence=save_confidence,
-                         scales=multiscale)
+                         stitch=stitch, confidence=save_confidence, scales=multiscale, temperature=temperature)
 
     def save_metrics():
         if seg.scales is not None:                    # a multi-scale run records its scales with the scores
             evaluator.metrics.results['multiscale'] = list(seg.scales)
+        if seg.temperature != 1.0:
+            evaluator.metrics.results['temperature'] = seg.temperature
         evaluator.save_metrics()
 
     def decode(i):
@@ -234,6 +253,62 @@ def test(args):
         if rank == 0:
             save_metrics()
     return evaluator
+
+
+def calibrate(args):
+    """Fit the softmax temperature of the mean stitch on labelled images (utils/calibrate.py) and write a copy of the
+    model file with a "calibration" entry, plus <output>/<id>/metrics/calibration_fit.json."""
+    from .models.model import Model
+    from .pipeline import TiledSegmenter
+    from .utils import tools
+    from .utils.calibrate import ResidentBudgetError, TemperatureFit, write_calibrated_copy
+    if int(os.environ.get('WORLD_SIZE', '1')) > 1:
+        print('pylc calibrate runs on one GPU: launch it without torchrun.', file=sys.stderr)
+        sys.exit(2)
+    stem, _ = os.path.splitext(args.model)
+    out_file = args.output or stem + '_calibrated.pth'
+    if os.path.abspath(out_file) == os.path.abspath(args.model):
+        print('pylc calibrate writes a copy: the output %s is the input model.' % out_file, file=sys.stderr)
+        sys.exit(2)
+    params = Parameters(args)
+    model = Model().load(args.model)
+    model.net.eval()
+    free = torch.cuda.mem_get_info()[0]
+    budget = args.max_resident_gb * 1e9 if args.max_resident_gb is not None else free / 2
+    seg = TiledSegmenter(model, batch_tiles=args.batch_tiles, stitch='mean')
+    fit = TemperatureFit(seg, budget)
+    files = tools.collate(args.img, args.mask)
+    for fpair in files:
+        img_file, mask_file = (fpair['img'], fpair['mask']) if isinstance(fpair, dict) else (fpair, None)
+        if not mask_file:
+            print('pylc calibrate needs a mask for every image; none for %s.' % img_file, file=sys.stderr)
+            sys.exit(2)
+        img = tools.get_image(img_file, model.meta.ch, scale=params.scale)[0]
+        gt = tools.get_image(mask_file, ch=3, scale=params.scale, interpolate=cv2.INTER_NEAREST)[0]
+        try:
+            fit.add(img, gt)
+        except ResidentBudgetError as exc:
+            print('pylc calibrate: %s' % exc, file=sys.stderr)
+            sys.exit(2)
+    before = fit.report(1.0)
+    res = fit.fit()
+    after = fit.report(res['temperature'])
+    if res['at_bound']:
+        print('Warning: the best temperature %g lies at the end of the searched range [0.05, 20]; the minimum may lie '
+              'outside it.' % res['temperature'])
+    calibration = {'temperature': res['temperature'], 'n_images': len(fit.retained), 'n_px': fit.n_px,
+                   'nll_before': before['nll'], 'nll_after': after['nll']}
+    write_calibrated_copy(args.model, out_file, calibration)
+    metrics_dir = tools.mk_path(os.path.join(defaults.output_dir, str(model.meta.id), 'metrics'))
+    fit_file = os.path.join(metrics_dir, 'calibration_fit.json')
+    with open(fit_file, 'w') as fp:
+        json.dump({'temperature': res['temperature'], 'at_bound': res['at_bound'],
+                   'evaluations': [[t, v] for t, v in res['evals']], 'before': before, 'after': after}, fp, indent=4)
+    print('Temperature %.6g: NLL %.6g -> %.6g, ECE %.4g -> %.4g, accuracy %.4f -> %.4f' % (
+        res['temperature'], before['nll'], after['nll'], before['ece'], after['ece'], before['accuracy'],
+        after['accuracy']))
+    print('Calibrated model saved to:\n\t%s\nFit report:\n\t%s' % (out_file, fit_file))
+    return calibration
 
 
 # ---- parser -----------------------------------------------------------------------------------
@@ -313,6 +388,22 @@ def get_parser():
     p.add_argument('--multiscale', type=float, nargs='+', default=None, metavar='S',
                    help='Average the class probabilities over these image scales (relative to the --scale image, at '
                         'most 8, no duplicates); needs --stitch mean.')
+    p.add_argument('--temperature', type=float, default=None,
+                   help="Softmax temperature of the mean stitch (default: the model file's fitted temperature, else "
+                        "1; 1 turns a fitted temperature off); needs --stitch mean.")
+
+    p = sub.add_parser('calibrate', help="Fit the mean stitch's softmax temperature on labelled images.")
+    common(p)
+    p.set_defaults(func=calibrate)
+    p.add_argument('-l', '--model', type=str, required=True, help='Path to trained PyLC model.')
+    p.add_argument('-i', '--img', type=str, required=True, help='Path to images directory or file.')
+    p.add_argument('-m', '--mask', type=str, required=True, help='Path to masks directory or file.')
+    p.add_argument('--scale', type=float, default=defaults.scale)
+    p.add_argument('--batch_tiles', type=int, default=32)
+    p.add_argument('-o', '--output', type=str, default=None,
+                   help='Calibrated model file to write (default: <model stem>_calibrated.pth next to the model).')
+    p.add_argument('--max_resident_gb', type=float, default=None,
+                   help="Device memory for the retained network outputs (default: half the device's free memory).")
     return parser
 
 
