@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define PYLC_ABI_VERSION 5
+#define PYLC_ABI_VERSION 6
 #define PYLC_MAX_CLASSES 32
 
 #define PYLC_OK 0
@@ -254,81 +254,64 @@ PYLC_API int pylc_tile_gather_norm_s2d_f32(const uint8_t *src, int H, int W, int
 
 /*
  * Fused stitch + softmax + argmax + colourise, replaces tools.reconstruct up to and including
- * colourize (utils/tools.py:239-313, 322-358) with the reference's exact band semantics
- * (raw logits at the borders, one softmax-average on edges, double softmax in the interior).
+ * colourize (utils/tools.py:239-313, 322-358), and per-pixel class probabilities and confidence from the same
+ * stitch (an extension: the reference never forms a clean probability map).
  *   logits        one contiguous [nr*nc, C, T, T] f32 buffer, row-major tile order, or NULL
  *   tile_batches  (used when logits == NULL) device array of pointers, batch b =
  *                 [tiles_per_batch, C, T, T] f32 holding tiles b*tiles_per_batch ... -- the list of
  *                 per-batch network outputs the reference concatenates (utils/tools.py:221-222)
  *   S             T/2 (output (nr+1)S x (nc+1)S) or T (pure scatter, output nr*T x nc*T)
+ *   mode          PYLC_STITCH_REFERENCE: the reference's exact band semantics (raw logits at the borders, one
+ *                 softmax-average on edges, double softmax in the interior) give the merged map M;
+ *                 labels = first argmax of M, stitched = M.  With confidence == NULL these are the
+ *                 reference's labels, rgb and M, bit for bit.
+ *                 PYLC_STITCH_MEAN: labels = first argmax of P, stitched = P, where P(y, x) is the mean, over
+ *                 the 1, 2 or 4 tiles covering the pixel, of softmax_c of that tile's logits.  On edge blocks P
+ *                 is exactly M; on corners (and everywhere when S == T) the softmax of the raw logits; in the
+ *                 interior the mean of the four softmaxes.
+ *                 Any other mode is PYLC_ERR_ARG.
  *   lut_rgb       HOST [C, 3] u8 colour per label (colourize's final mapping); needed iff rgb
  *   labels        [h, w] u8 first-maximum argmax     (nullable)
  *   rgb           [h, w, 3] u8                       (nullable)
- *   stitched      [C, h, w] f32 merged map           (nullable; parity tests / save_logits)
+ *   confidence    [h, w] u8, q = min(255, round-to-nearest(P[label] * 255)); the same P in both modes (nullable)
+ *   stitched      [C, h, w] f32 M or P               (nullable; parity tests / save_logits)
+ *   temperature   post-hoc calibration: in PYLC_STITCH_MEAN mode every tile softmax is taken of L / temperature.
+ *                 Every softmax of the mean stitch is a softmax of raw tile logits, so the kernels evaluate it
+ *                 with k_T = f32(log2(e) / f32(temperature)) in place of log2(e):
+ *                     P_T(y, x) = the mean over the covering tiles of softmax(L / T),  labels = first argmax of P_T,
+ *                     confidence = min(255, round-to-nearest(P_T[label] * 255)),  stitched = P_T.
+ *                 Temperature 1 is the untempered stitch.  Labels in overlap zones may change with T: the argmax
+ *                 of a mean of softmaxes depends on the temperature.  PYLC_ERR_ARG for a temperature that is not
+ *                 finite and > 0, or other than 1 in PYLC_STITCH_REFERENCE mode (that mode mixes raw-logit
+ *                 corners, a second softmax of probability sums and labels from M: a temperature has no single
+ *                 meaning there).
  */
-PYLC_API int pylc_stitch_argmax_colour(const float *logits, const float *const *tile_batches,
-                              int tiles_per_batch, int nr, int nc, int C, int T, int S,
-                              const uint8_t *lut_rgb, uint8_t *labels, uint8_t *rgb,
-                              float *stitched, pylc_stream_t stream);
+#define PYLC_STITCH_REFERENCE 0
+#define PYLC_STITCH_MEAN 1
+PYLC_API int pylc_stitch_probs(const float *logits, const float *const *tile_batches, int tiles_per_batch,
+                      int nr, int nc, int C, int T, int S, int mode, const uint8_t *lut_rgb,
+                      uint8_t *labels, uint8_t *rgb, uint8_t *confidence, float *stitched, float temperature,
+                      pylc_stream_t stream);
 
-/* tools.colourize (utils/tools.py:322-358) on a flat u8 label array: rgb[i] = lut_rgb[labels[i]]. */
 /*
  * Fused form of the network's last step + the stitch (SURVEY.md 8f-1): takes the decoder's output
  * BEFORE the final x4 bilinear up-sample -- `decoder_batches`: device array of device pointers to
  * channels-last [b, hs, ws, C] f32 batches, hs = ws = T/4 -- evaluates
  * F.interpolate(..., size=T, mode='bilinear', align_corners=True) (models/architectures/deeplab.py:38) per
  * output pixel with the arithmetic of pylc_upsample_nhwc_to_nchw_f32, and stitches as
- * pylc_stitch_argmax_colour does.  Outputs are bit-identical to that two-call route.
+ * pylc_stitch_probs does.  Outputs are bit-identical to that two-call route.
  * PYLC_ERR_GEOMETRY for C > 12 or a geometry other than the x4 up-sample of 512-class tile sizes: the
- * caller keeps the two-call route.
+ * caller keeps the two-call route.  PYLC_ERR_ALIGN for a misaligned output (stitched not 8-byte, labels,
+ * rgb or confidence not 2-byte aligned).  Other arguments and return codes as pylc_stitch_probs.
  */
-PYLC_API int pylc_stitch_upsample_argmax_colour(const float *const *decoder_batches, int tiles_per_batch, int nr, int nc,
-                                       int C, int T, int S, int hs, int ws, const uint8_t *lut_rgb, uint8_t *labels,
-                                       uint8_t *rgb, float *stitched, pylc_stream_t stream);
-PYLC_API int pylc_colourise_u8(const uint8_t *labels, int64_t n_px, const uint8_t *lut_rgb, int C,
-                      uint8_t *rgb, pylc_stream_t stream);
-
-/*
- * Per-pixel class probabilities and confidence from the same stitch (an extension: the reference never forms a
- * clean probability map).  P(y, x) is the mean, over the 1, 2 or 4 tiles covering the pixel, of softmax_c of
- * that tile's logits.  On edge blocks it is exactly the reference's merged map M; on corners (and everywhere
- * when S == T) the softmax of the raw logits; in the interior the mean of the four softmaxes.
- *   mode          PYLC_STITCH_REFERENCE: labels / rgb / stitched are those of pylc_stitch_argmax_colour (first
- *                 argmax of M, stitched = M), bit for bit.
- *                 PYLC_STITCH_MEAN: labels = first argmax of P, stitched = P.
- *   confidence    nullable [h, w] u8, q = min(255, round-to-nearest(P[label] * 255)); the same P in both modes
- * Other arguments as pylc_stitch_argmax_colour / pylc_stitch_upsample_argmax_colour (the fused form also
- * returns PYLC_ERR_ALIGN for an odd `confidence` address).  An unknown mode is PYLC_ERR_ARG.
- */
-#define PYLC_STITCH_REFERENCE 0
-#define PYLC_STITCH_MEAN 1
-PYLC_API int pylc_stitch_probs(const float *logits, const float *const *tile_batches, int tiles_per_batch,
-                      int nr, int nc, int C, int T, int S, int mode, const uint8_t *lut_rgb,
-                      uint8_t *labels, uint8_t *rgb, uint8_t *confidence, float *stitched, pylc_stream_t stream);
 PYLC_API int pylc_stitch_upsample_probs(const float *const *decoder_batches, int tiles_per_batch, int nr, int nc,
                                int C, int T, int S, int hs, int ws, int mode, const uint8_t *lut_rgb,
-                               uint8_t *labels, uint8_t *rgb, uint8_t *confidence, float *stitched, pylc_stream_t stream);
+                               uint8_t *labels, uint8_t *rgb, uint8_t *confidence, float *stitched, float temperature,
+                               pylc_stream_t stream);
 
-/*
- * Temperature-scaled probabilities (post-hoc calibration): pylc_stitch_probs / pylc_stitch_upsample_probs with every
- * tile softmax taken of L / temperature.  In PYLC_STITCH_MEAN mode every softmax of the stitch is a softmax of raw
- * tile logits, so the kernels evaluate it with k_T = f32(log2(e) / f32(temperature)) in place of log2(e):
- *     P_T(y, x) = the mean over the covering tiles of softmax(L / T),  labels = first argmax of P_T,
- *     confidence = min(255, round-to-nearest(P_T[label] * 255)),  stitched = P_T.
- * At temperature 1 every output equals the untempered call bit for bit.  Labels in overlap zones may change with T:
- * the argmax of a mean of softmaxes depends on the temperature.
- * PYLC_ERR_ARG for a temperature that is not finite and > 0, or other than 1 in PYLC_STITCH_REFERENCE mode (that
- * mode mixes raw-logit corners, a second softmax of probability sums and labels from M: a temperature has no single
- * meaning there).  Other arguments and return codes as the untempered calls.
- */
-PYLC_API int pylc_stitch_probs_t(const float *logits, const float *const *tile_batches, int tiles_per_batch,
-                        int nr, int nc, int C, int T, int S, int mode, const uint8_t *lut_rgb,
-                        uint8_t *labels, uint8_t *rgb, uint8_t *confidence, float *stitched, float temperature,
-                        pylc_stream_t stream);
-PYLC_API int pylc_stitch_upsample_probs_t(const float *const *decoder_batches, int tiles_per_batch, int nr, int nc,
-                                 int C, int T, int S, int hs, int ws, int mode, const uint8_t *lut_rgb,
-                                 uint8_t *labels, uint8_t *rgb, uint8_t *confidence, float *stitched, float temperature,
-                                 pylc_stream_t stream);
+/* tools.colourize (utils/tools.py:322-358) on a flat u8 label array: rgb[i] = lut_rgb[labels[i]]. */
+PYLC_API int pylc_colourise_u8(const uint8_t *labels, int64_t n_px, const uint8_t *lut_rgb, int C,
+                      uint8_t *rgb, pylc_stream_t stream);
 
 /* ---- evaluation --------------------------------------------------------------------------- */
 
@@ -338,7 +321,7 @@ PYLC_API int pylc_stitch_upsample_probs_t(const float *const *decoder_batches, i
  * Evaluator.load's two class_encode passes, Evaluator.validate's coverage injection and every
  * scikit-learn confusion matrix (utils/tools.py:316-317, utils/evaluate.py:87-119,150-176,
  * utils/metrics.py:45-87).
- *   labels    [h, w] u8 fitted-resolution labels, every value < C (what pylc_stitch_*_argmax_colour and
+ *   labels    [h, w] u8 fitted-resolution labels, every value < C (what the stitch entry points and
  *             pylc_class_encode emit).  PRECONDITION, not checked: a per-pixel test costs 10-15 % of the kernel
  *             (measured); a label >= C indexes the shared-memory counters out of range
  *   x_ofs     [w_full] i32, y_ofs [h_full] i32: OpenCV nearest source index per destination index

@@ -15,7 +15,7 @@ LIB_PATH = os.path.join(_HERE, "lib", "libpylc_b200.so")
 
 MAX_CLASSES = 32
 AREA_TAPS = 6
-ABI_VERSION = 5
+ABI_VERSION = 6
 MAX_SCALES = 8
 SCORES_WS_DOUBLES = 2048      # PYLC_SCORES_WS_DOUBLES
 
@@ -66,19 +66,11 @@ SIGNATURES = {
     "pylc_upsample_nhwc_to_nchw_f32": (c_int, [_ptr, c_int, c_int, c_int, c_int, _ptr, c_int, c_int, _ptr]),
     "pylc_tile_gather_norm_s2d_f32": (c_int, [_u8p, c_int, c_int, c_int, c_size_t, c_int, c_int,
                                               POINTER(c_float), POINTER(c_float), c_float, _ptr, _ptr]),
-    "pylc_stitch_argmax_colour": (c_int, [_ptr, _ptr, c_int, c_int, c_int, c_int, c_int, c_int,
-                                          POINTER(c_uint8), _u8p, _u8p, _ptr, _ptr]),
-    "pylc_stitch_upsample_argmax_colour": (c_int, [_ptr, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
-                                                   POINTER(c_uint8), _u8p, _u8p, _ptr, _ptr]),
-    "pylc_colourise_u8": (c_int, [_u8p, c_int64, POINTER(c_uint8), c_int, _u8p, _ptr]),
     "pylc_stitch_probs": (c_int, [_ptr, _ptr, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
-                                  POINTER(c_uint8), _u8p, _u8p, _u8p, _ptr, _ptr]),
+                                  POINTER(c_uint8), _u8p, _u8p, _u8p, _ptr, c_float, _ptr]),
     "pylc_stitch_upsample_probs": (c_int, [_ptr, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
-                                           POINTER(c_uint8), _u8p, _u8p, _u8p, _ptr, _ptr]),
-    "pylc_stitch_probs_t": (c_int, [_ptr, _ptr, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
-                                    POINTER(c_uint8), _u8p, _u8p, _u8p, _ptr, c_float, _ptr]),
-    "pylc_stitch_upsample_probs_t": (c_int, [_ptr, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
-                                             POINTER(c_uint8), _u8p, _u8p, _u8p, _ptr, c_float, _ptr]),
+                                           POINTER(c_uint8), _u8p, _u8p, _u8p, _ptr, c_float, _ptr]),
+    "pylc_colourise_u8": (c_int, [_u8p, c_int64, POINTER(c_uint8), c_int, _u8p, _ptr]),
     "pylc_prob_scores": (c_int, [_ptr, c_int, c_int, c_int, _ptr, _ptr, c_int, c_int, _u8p, c_int, _ptr, _ptr, _ptr]),
     "pylc_resample_encode_confusion": (c_int, [_u8p, c_int, c_int, _ptr, _ptr, c_int, c_int, _u8p, c_size_t,
                                                POINTER(c_uint8), POINTER(c_uint8), c_int, c_int, _ptr,

@@ -15,13 +15,14 @@
 // the two strip sums x 1/4 in the interior, taken before the second softmax.  MODE selects the labels:
 // PYLC_STITCH_REFERENCE (0) takes the first argmax of M (the reference's labels), PYLC_STITCH_MEAN (1) that
 // of P, and then `stitched` holds P instead of M.  CONF adds the u8 plane q = min(255, rn(P[label] * 255)).
-// MODE = 0 without CONF is the code the argmax / colour entry points have always run.
+// MODE = 0 without CONF is the reference's stitch: labels, rgb and M.
 //
-// Temperature (pylc_stitch_probs_t): in mean mode every softmax the kernels evaluate is a softmax of raw tile
-// logits, so softmax(L / T) is exp_cls with k = fl32(log2(e) / T) in place of log2(e).  The mean-mode
-// instantiations take k from the kernel's trailing argument `k`; the reference-mode instantiations ignore it
-// and keep the compile-time constant.  `k` is a kernel argument after the existing ones rather than a field
-// of StitchArgs, so every parameter the reference-mode kernels read keeps its offset.
+// Temperature: in mean mode every softmax the kernels evaluate is a softmax of raw tile logits, so
+// softmax(L / T) is exp_cls with k = fl32(log2(e) / T) in place of log2(e).  The mean-mode instantiations
+// take k from the kernel argument `k`; the reference-mode instantiations ignore it and keep the
+// compile-time constant.
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace pylc {
@@ -38,6 +39,22 @@ struct StitchArgs {
     uint8_t *rgb;
     float *stitched;
 };
+
+// What emit_unit writes, the same for both kernel forms; every pointer is nullable.
+struct StitchOut {
+    int h, w;                       // output map size
+    uint8_t *labels;                // [h, w]
+    uint8_t *rgb;                   // [h, w, 3]
+    float *stitched;                // [C, h, w]: M, or P in mean mode
+    uint8_t *confidence;            // [h, w], written by the CONF instantiations
+};
+
+// The output fields are kept in the argument structs rather than in a StitchOut member: moving them changes the
+// kernels' parameter layout, and with it the code ptxas generates for every stitch_kernel instantiation.
+template <class Args>
+__device__ __forceinline__ StitchOut stitch_out(const Args &a, uint8_t *conf) {
+    return {a.h, a.w, a.labels, a.rgb, a.stitched, conf};
+}
 
 __device__ __forceinline__ const float *tile_base(const StitchArgs &a, int i, int j) {
     const int k = i * a.nc + j;
@@ -122,8 +139,8 @@ __device__ __forceinline__ void load_cls(const float *p, size_t cstride, int C, 
 // Writes one unit: optional f32 map, first-maximum argmax (np.argmax), label bytes, optional RGB and, with
 // CONF, the confidence byte of P at the label.
 template <int CMAX, int PX, bool CONF = false>
-__device__ __forceinline__ void emit_unit(const StitchArgs &a, const uint32_t *s_lut, int C, const float (&m)[CMAX][PX],
-                                          const float (&p)[CMAX][PX], uint8_t *conf, size_t o) {
+__device__ __forceinline__ void emit_unit(const StitchOut &a, const uint32_t *s_lut, int C, const float (&m)[CMAX][PX],
+                                          const float (&p)[CMAX][PX], size_t o) {
     if (a.stitched) {
 #pragma unroll
         for (int c = 0; c < CMAX; ++c)
@@ -150,12 +167,12 @@ __device__ __forceinline__ void emit_unit(const StitchArgs &a, const uint32_t *s
         else a.labels[o] = (uint8_t)lab[0];
     }
     if constexpr (CONF) {
-        if (conf) {
+        if (a.confidence) {
             uint32_t q[PX];
 #pragma unroll
             for (int j = 0; j < PX; ++j) q[j] = min(255u, __float2uint_rn(pl[j] * 255.f));
-            if (PX == 2) *reinterpret_cast<uint16_t *>(conf + o) = (uint16_t)(q[0] | (q[PX - 1] << 8));
-            else conf[o] = (uint8_t)q[0];
+            if (PX == 2) *reinterpret_cast<uint16_t *>(a.confidence + o) = (uint16_t)(q[0] | (q[PX - 1] << 8));
+            else a.confidence[o] = (uint8_t)q[0];
         }
     }
     if (a.rgb) {
@@ -201,16 +218,13 @@ __device__ __forceinline__ void quarter_sum(const float (&s0)[CMAX][PX], const f
             if (c < C) p[c][j] = (s0[c][j] + s1[c][j]) * 0.25f;
 }
 
-// NH: tiles per strip (1 border / 2 interior columns); NV: strips (1 border / 2 interior rows)
-template <int C_T, int CMAX, int PX, int NH, int NV, int MODE, bool CONF>
-__device__ __forceinline__ void stitch_units(const StitchArgs &a, const uint32_t *s_lut, uint8_t *conf, float k, int ky, int kx,
-                                             int row0, int nrows) {
-    const int C = C_T > 0 ? C_T : a.C;
-    const float kl = MODE == 1 ? k : kLog2e;     // scale of every raw-logit softmax: log2(e) / temperature
-    const int T = a.T, S = a.S;
-    const size_t cstride = (size_t)T * T;
-    // source tiles: strip s in {0,1} x column q in {0,1}
-    int ti[2], ty0[2], tj[2], tx0[2];
+// Source tiles of output block (ky, kx): strip s in {0,1} reads tile row ti[s] from tile row ty0[s] on, column
+// q in {0,1} tile column tj[q] from tile column tx0[q] on.  NH: tiles per strip (1 border / 2 interior
+// columns); NV: strips (1 border / 2 interior rows).
+template <int NH, int NV, class Args>
+__device__ __forceinline__ void select_tiles(const Args &a, int ky, int kx, int (&ti)[2], int (&ty0)[2], int (&tj)[2],
+                                             int (&tx0)[2]) {
+    const int S = a.S;
     if (!a.overlap) {
         ti[0] = ky; ty0[0] = 0; tj[0] = kx; tx0[0] = 0;
     } else {
@@ -229,6 +243,58 @@ __device__ __forceinline__ void stitch_units(const StitchArgs &a, const uint32_t
             tj[1] = kx;     tx0[1] = 0;
         }
     }
+}
+
+// Column merge of one strip at interior columns: the two tiles' softmaxes averaged into v0.  When a second
+// softmax follows (NV == 2) the strip keeps the SUM of the two and the 1/2 moves into that softmax's scale.
+template <int CMAX, int PX, int NV>
+__device__ __forceinline__ void merge_columns(float (&v0)[CMAX][PX], float (&v1)[CMAX][PX], int C, float kl) {
+    float r0[PX], r1[PX];
+    exp_cls<CMAX, PX, true>(v0, C, kl, r0);
+    exp_cls<CMAX, PX, true>(v1, C, kl, r1);
+    combine_cls<CMAX, PX>(v0, r0, v1, r1, C, NV == 2 ? 1.f : 0.5f);
+}
+
+// Everything after the column merge, given the merged strips s0 and s1 (the same array when NV == 1): P where it
+// is not M itself, the row merge into s0 (mean mode needs no second softmax in the interior) and the write of
+// output pixel (y0 + yl, x0 + xl): block origin and the unit's place in the block.  The offset is formed after the
+// merge, as the kernels have always done; computing it before changes the generated code.
+template <int CMAX, int PX, int NH, int NV, int MODE, bool CONF>
+__device__ __forceinline__ void merge_rows_emit(const StitchOut &out, const uint32_t *s_lut, int C, float kl,
+                                                float (&s0)[CMAX][PX], float (&s1)[CMAX][PX], int y0, int yl, int x0, int xl) {
+    constexpr bool NEED_P = MODE == 1 || CONF;
+    float p[CMAX][PX];          // P where it is not M itself (interior and corner blocks)
+    if constexpr (NEED_P && NV == 2 && NH == 2) quarter_sum<CMAX, PX>(s0, s1, C, p);
+    if constexpr (NEED_P && NV == 1 && NH == 1) softmax_copy<CMAX, PX>(s0, C, kl, p);
+    if (NV == 2 && !(MODE == 1 && NH == 2)) {
+        float r0[PX], r1[PX];
+        if (NH == 2) {   // inputs: sums of two probability vectors, in [0, 2]
+            exp_cls<CMAX, PX, false>(s0, C, 0.5f * kLog2e, r0);
+            exp_cls<CMAX, PX, false>(s1, C, 0.5f * kLog2e, r1);
+        } else {         // left / right border: raw logits
+            exp_cls<CMAX, PX, true>(s0, C, kl, r0);
+            exp_cls<CMAX, PX, true>(s1, C, kl, r1);
+        }
+        combine_cls<CMAX, PX>(s0, r0, s1, r1, C, 0.5f);
+    }
+    const size_t o = (size_t)(y0 + yl) * out.w + (size_t)(x0 + xl);
+    constexpr bool P_IS_M = NH + NV == 3;         // edge blocks: P is the reference's M
+    if constexpr (!NEED_P) emit_unit<CMAX, PX>(out, s_lut, C, s0, s0, o);
+    else if constexpr (P_IS_M) emit_unit<CMAX, PX, CONF>(out, s_lut, C, s0, s0, o);
+    else if constexpr (MODE == 1) emit_unit<CMAX, PX, CONF>(out, s_lut, C, p, p, o);
+    else emit_unit<CMAX, PX, CONF>(out, s_lut, C, s0, p, o);
+}
+
+template <int C_T, int CMAX, int PX, int NH, int NV, int MODE, bool CONF>
+__device__ __forceinline__ void stitch_units(const StitchArgs &a, const uint32_t *s_lut, uint8_t *conf, float k, int ky, int kx, int row0,
+                                             int nrows) {
+    const int C = C_T > 0 ? C_T : a.C;
+    const float kl = MODE == 1 ? k : kLog2e;     // scale of every raw-logit softmax: log2(e) / temperature
+    const int T = a.T, S = a.S;
+    const size_t cstride = (size_t)T * T;
+    int ti[2], ty0[2], tj[2], tx0[2];
+    select_tiles<NH, NV>(a, ky, kx, ti, ty0, tj, tx0);
+    const StitchOut out = stitch_out(a, conf);
     const float *base[NV][NH];
 #pragma unroll
     for (int s = 0; s < NV; ++s)
@@ -252,39 +318,11 @@ __device__ __forceinline__ void stitch_units(const StitchArgs &a, const uint32_t
         for (int s = 0; s < NV; ++s)
 #pragma unroll
             for (int q = 0; q < NH; ++q) load_cls<CMAX, PX>(base[s][q] + off, cstride, C, v[s][q]);
-
-        // strips: at interior columns the two tiles' softmaxes are averaged.  When a second softmax
-        // follows (NV == 2) the strip keeps the SUM of the two and the 1/2 moves into that softmax's scale.
-        if (NH == 2) {
+        if constexpr (NH == 2) {
 #pragma unroll
-            for (int s = 0; s < NV; ++s) {
-                float r0[PX], r1[PX];
-                exp_cls<CMAX, PX, true>(v[s][0], C, kl, r0);
-                exp_cls<CMAX, PX, true>(v[s][1], C, kl, r1);
-                combine_cls<CMAX, PX>(v[s][0], r0, v[s][1], r1, C, NV == 2 ? 1.f : 0.5f);
-            }
+            for (int s = 0; s < NV; ++s) merge_columns<CMAX, PX, NV>(v[s][0], v[s][1], C, kl);
         }
-        constexpr bool NEED_P = MODE == 1 || CONF;
-        float p[CMAX][PX];          // P where it is not M itself (interior and corner blocks)
-        if constexpr (NEED_P && NV == 2 && NH == 2) quarter_sum<CMAX, PX>(v[0][0], v[NV - 1][0], C, p);
-        if constexpr (NEED_P && NV == 1 && NH == 1) softmax_copy<CMAX, PX>(v[0][0], C, kl, p);
-        if (NV == 2 && !(MODE == 1 && NH == 2)) {     // mean mode needs no second softmax in the interior
-            float r0[PX], r1[PX];
-            if (NH == 2) {   // inputs: sums of two probability vectors, in [0, 2]
-                exp_cls<CMAX, PX, false>(v[0][0], C, 0.5f * kLog2e, r0);
-                exp_cls<CMAX, PX, false>(v[NV - 1][0], C, 0.5f * kLog2e, r1);
-            } else {         // left / right border: raw logits
-                exp_cls<CMAX, PX, true>(v[0][0], C, kl, r0);
-                exp_cls<CMAX, PX, true>(v[NV - 1][0], C, kl, r1);
-            }
-            combine_cls<CMAX, PX>(v[0][0], r0, v[NV - 1][0], r1, C, 0.5f);
-        }
-        const size_t o = (size_t)(ky * S + yl) * a.w + (size_t)(kx * S + xl);
-        constexpr bool P_IS_M = NH + NV == 3;         // edge blocks: P is the reference's M
-        if constexpr (!NEED_P) emit_unit<CMAX, PX>(a, s_lut, C, v[0][0], v[0][0], conf, o);
-        else if constexpr (P_IS_M) emit_unit<CMAX, PX, CONF>(a, s_lut, C, v[0][0], v[0][0], conf, o);
-        else if constexpr (MODE == 1) emit_unit<CMAX, PX, CONF>(a, s_lut, C, p, p, conf, o);
-        else emit_unit<CMAX, PX, CONF>(a, s_lut, C, v[0][0], p, conf, o);
+        merge_rows_emit<CMAX, PX, NH, NV, MODE, CONF>(out, s_lut, C, kl, v[0][0], v[NV - 1][0], ky * S, yl, kx * S, xl);
     }
 }
 
@@ -346,32 +384,16 @@ struct StitchUpArgs {
 };
 
 template <int C_T, int CMAX, int NH, int NV, int MODE, bool CONF>
-__device__ __forceinline__ void stitch_up_units(const StitchUpArgs &a, const uint32_t *s_lut, uint8_t *conf, float k, float *s_src, int ky,
-                                                int kx, int row0) {
+__device__ __forceinline__ void stitch_up_units(const StitchUpArgs &a, const uint32_t *s_lut, uint8_t *conf, float k, float *s_src, int ky, int kx,
+                                                int row0) {
     constexpr int PX = 2;
     const int C = C_T > 0 ? C_T : a.C;
     const float kl = MODE == 1 ? k : kLog2e;     // as in stitch_units
     const int T = a.T, S = a.S, hs = a.hs, ws = a.ws;
     const float rh = (float)(hs - 1) / (float)(T - 1), rw = (float)(ws - 1) / (float)(T - 1);
     int ti[2], ty0[2], tj[2], tx0[2];
-    if (!a.overlap) {
-        ti[0] = ky; ty0[0] = 0; tj[0] = kx; tx0[0] = 0;
-    } else {
-        if (NV == 1) {
-            ti[0] = ky == 0 ? 0 : a.nr - 1;
-            ty0[0] = ky == 0 ? 0 : S;
-        } else {
-            ti[0] = ky - 1; ty0[0] = S;
-            ti[1] = ky;     ty0[1] = 0;
-        }
-        if (NH == 1) {
-            tj[0] = kx == 0 ? 0 : a.nc - 1;
-            tx0[0] = kx == 0 ? 0 : S;
-        } else {
-            tj[0] = kx - 1; tx0[0] = S;
-            tj[1] = kx;     tx0[1] = 0;
-        }
-    }
+    select_tiles<NH, NV>(a, ky, kx, ti, ty0, tj, tx0);
+    const StitchOut out = stitch_out(a, conf);
     // ---- stage ---------------------------------------------------------------------------------------
     int ys0[NV], xs0[NH], ncol[NH];
 #pragma unroll
@@ -470,40 +492,13 @@ __device__ __forceinline__ void stitch_up_units(const StitchUpArgs &a, const uin
                     for (int j = 0; j < PX; ++j)
                         v[q][c][j] = fmaf(cw[q][j][0], col[0][c], fmaf(cw[q][j][1], col[1][c], cw[q][j][2] * col[2][c]));
             }
-            if (NH == 2) {
-                float r0[PX], r1[PX];
-                exp_cls<CMAX, PX, true>(v[0], C, kl, r0);
-                exp_cls<CMAX, PX, true>(v[NH - 1], C, kl, r1);
-                combine_cls<CMAX, PX>(v[0], r0, v[NH - 1], r1, C, NV == 2 ? 1.f : 0.5f);
-            }
+            if constexpr (NH == 2) merge_columns<CMAX, PX, NV>(v[0], v[1], C, kl);
 #pragma unroll
             for (int c = 0; c < CMAX; ++c)
 #pragma unroll
                 for (int j = 0; j < PX; ++j) strip[s][c][j] = v[0][c][j];
         }
-        constexpr bool NEED_P = MODE == 1 || CONF;     // P as in stitch_units
-        float p[CMAX][PX];
-        if constexpr (NEED_P && NV == 2 && NH == 2) quarter_sum<CMAX, PX>(strip[0], strip[NV - 1], C, p);
-        if constexpr (NEED_P && NV == 1 && NH == 1) softmax_copy<CMAX, PX>(strip[0], C, kl, p);
-        if (NV == 2 && !(MODE == 1 && NH == 2)) {
-            float r0[PX], r1[PX];
-            if (NH == 2) {
-                exp_cls<CMAX, PX, false>(strip[0], C, 0.5f * kLog2e, r0);
-                exp_cls<CMAX, PX, false>(strip[NV - 1], C, 0.5f * kLog2e, r1);
-            } else {
-                exp_cls<CMAX, PX, true>(strip[0], C, kl, r0);
-                exp_cls<CMAX, PX, true>(strip[NV - 1], C, kl, r1);
-            }
-            combine_cls<CMAX, PX>(strip[0], r0, strip[NV - 1], r1, C, 0.5f);
-        }
-        StitchArgs e;                    // emit_unit only reads the output pointers and the map size
-        e.labels = a.labels; e.rgb = a.rgb; e.stitched = a.stitched; e.h = a.h; e.w = a.w;
-        const size_t o = (size_t)(ky * S + yl) * a.w + (size_t)(kx * S + X);
-        constexpr bool P_IS_M = NH + NV == 3;
-        if constexpr (!NEED_P) emit_unit<CMAX, PX>(e, s_lut, C, strip[0], strip[0], conf, o);
-        else if constexpr (P_IS_M) emit_unit<CMAX, PX, CONF>(e, s_lut, C, strip[0], strip[0], conf, o);
-        else if constexpr (MODE == 1) emit_unit<CMAX, PX, CONF>(e, s_lut, C, p, p, conf, o);
-        else emit_unit<CMAX, PX, CONF>(e, s_lut, C, strip[0], p, conf, o);
+        merge_rows_emit<CMAX, PX, NH, NV, MODE, CONF>(out, s_lut, C, kl, strip[0], strip[NV - 1], ky * S, yl, kx * S, X);
     }
 }
 
@@ -534,11 +529,60 @@ __global__ void __launch_bounds__(kThreads, 2) stitch_up_kernel(StitchUpArgs a, 
 
 using namespace pylc;
 
-// Launch of the stitch kernel instantiation for (mode, confidence); the argmax / colour entry points take
-// mode 0 without confidence, the kernels they have always launched.
+// Checks both forms make, after their own checks of the tile source (PYLC_ERR_ARG too).  A temperature is finite and
+// > 0, and other than 1 only for the mean stitch: reference mode mixes raw-logit corners, a second softmax of
+// probability sums and labels from M, so a temperature has no single meaning there.
+static int check_stitch(int nr, int nc, int C, int T, int S, int mode, float temperature, const uint8_t *lut_rgb,
+                        const uint8_t *rgb) {
+    if (nr < 1 || nc < 1 || T < 1 || S < 1) return PYLC_ERR_ARG;
+    if (!(temperature > 0.f) || !isfinite(temperature)) return PYLC_ERR_ARG;
+    if (mode != PYLC_STITCH_MEAN && temperature != 1.f) return PYLC_ERR_ARG;
+    if (rgb && !lut_rgb) return PYLC_ERR_ARG;
+    if (mode != PYLC_STITCH_REFERENCE && mode != PYLC_STITCH_MEAN) return PYLC_ERR_ARG;
+    if (C < 1 || C > PYLC_MAX_CLASSES) return PYLC_ERR_CLASSES;
+    if (!(S == T || 2 * S == T)) return PYLC_ERR_GEOMETRY;  // the reference is only correct for these (tools.py:235-236)
+    return PYLC_OK;
+}
+
+// The block grid and the outputs, the fields both argument structs share.
+template <class Args>
+static void set_blocks(Args &a, int nr, int nc, int C, int T, int S, uint8_t *labels, uint8_t *rgb, float *stitched) {
+    a.nr = nr; a.nc = nc; a.C = C; a.T = T; a.S = S;
+    a.overlap = S < T;
+    a.nbx = a.overlap ? nc + 1 : nc;
+    a.nby = a.overlap ? nr + 1 : nr;
+    a.h = a.nby * S;
+    a.w = a.nbx * S;
+    a.labels = labels; a.rgb = rgb; a.stitched = stitched;
+}
+
+static ColourLut stitch_lut(const uint8_t *lut_rgb, int C) {
+    ColourLut lut;
+    if (lut_rgb) build_colour_lut(lut_rgb, C, &lut);
+    else for (int i = 0; i < PYLC_MAX_CLASSES; ++i) lut.rgb[i] = 0;
+    return lut;
+}
+
+// Calls launch(std::integral_constant<int, MODE>, std::bool_constant<CONF>, k) for the instantiation (mode, confidence)
+// selects; k = log2(e) / temperature is the softmax scale of the mean-mode kernels, exactly log2(e) at T = 1.
+template <class Launch>
+static int launch_mode(int mode, bool confidence, float temperature, Launch launch) {
+    using Ref = std::integral_constant<int, 0>;
+    using Mean = std::integral_constant<int, 1>;
+    int rc;
+    if (mode == PYLC_STITCH_MEAN) {
+        const float k = kLog2e / temperature;
+        rc = confidence ? launch(Mean{}, std::true_type{}, k) : launch(Mean{}, std::false_type{}, k);
+    } else {
+        rc = confidence ? launch(Ref{}, std::true_type{}, kLog2e) : launch(Ref{}, std::false_type{}, kLog2e);
+    }
+    if (rc) return rc;
+    return finish_launch();
+}
+
 template <int MODE, bool CONF>
-static void launch_stitch(bool px2, int C, unsigned grid, cudaStream_t st, const StitchArgs &a, const ColourLut &lut,
-                          uint8_t *conf, float k) {
+static int launch_stitch(bool px2, int C, unsigned grid, cudaStream_t st, const StitchArgs &a, const ColourLut &lut,
+                         uint8_t *conf, float k) {
     if (px2) {
         if (C == 9) stitch_kernel<9, 9, 2, MODE, CONF><<<grid, kThreads, 0, st>>>(a, lut, conf, k);
         else if (C == 11) stitch_kernel<11, 11, 2, MODE, CONF><<<grid, kThreads, 0, st>>>(a, lut, conf, k);
@@ -550,36 +594,19 @@ static void launch_stitch(bool px2, int C, unsigned grid, cudaStream_t st, const
         else if (C <= 16) stitch_kernel<0, 16, 1, MODE, CONF><<<grid, kThreads, 0, st>>>(a, lut, conf, k);
         else stitch_kernel<0, 32, 1, MODE, CONF><<<grid, kThreads, 0, st>>>(a, lut, conf, k);
     }
+    return 0;
 }
 
-// A temperature is finite and > 0, and other than 1 only for the mean stitch: reference mode mixes raw-logit
-// corners, a second softmax of probability sums and labels from M, so a temperature has no single meaning there.
-static bool temperature_ok(float temperature, int mode) {
-    if (!(temperature > 0.f) || !isfinite(temperature)) return false;
-    return mode == PYLC_STITCH_MEAN || temperature == 1.f;
-}
-
-static int stitch_launch(const float *logits, const float *const *tile_batches, int tiles_per_batch, int nr, int nc, int C,
-                         int T, int S, int mode, const uint8_t *lut_rgb, uint8_t *labels, uint8_t *rgb, uint8_t *confidence,
-                         float *stitched, float temperature, pylc_stream_t stream) {
-    if ((!logits && !tile_batches) || nr < 1 || nc < 1 || T < 1 || S < 1) return PYLC_ERR_ARG;
-    if (!temperature_ok(temperature, mode)) return PYLC_ERR_ARG;
-    if (!logits && tiles_per_batch < 1) return PYLC_ERR_ARG;
-    if (rgb && !lut_rgb) return PYLC_ERR_ARG;
-    if (mode != PYLC_STITCH_REFERENCE && mode != PYLC_STITCH_MEAN) return PYLC_ERR_ARG;
-    if (C < 1 || C > PYLC_MAX_CLASSES) return PYLC_ERR_CLASSES;
-    if (!(S == T || 2 * S == T)) return PYLC_ERR_GEOMETRY;  // the reference is only correct for these (tools.py:235-236)
+extern "C" int pylc_stitch_probs(const float *logits, const float *const *tile_batches, int tiles_per_batch, int nr, int nc,
+                                 int C, int T, int S, int mode, const uint8_t *lut_rgb, uint8_t *labels, uint8_t *rgb,
+                                 uint8_t *confidence, float *stitched, float temperature, pylc_stream_t stream) {
+    if (!logits && (!tile_batches || tiles_per_batch < 1)) return PYLC_ERR_ARG;
+    if (int rc = check_stitch(nr, nc, C, T, S, mode, temperature, lut_rgb, rgb)) return rc;
     StitchArgs a;
     a.logits = logits;
     a.batches = tile_batches;
     a.tiles_per_batch = logits ? nr * nc : tiles_per_batch;
-    a.nr = nr; a.nc = nc; a.C = C; a.T = T; a.S = S;
-    a.overlap = S < T;
-    a.nbx = a.overlap ? nc + 1 : nc;
-    a.nby = a.overlap ? nr + 1 : nr;
-    a.h = a.nby * S;
-    a.w = a.nbx * S;
-    a.labels = labels; a.rgb = rgb; a.stitched = stitched;
+    set_blocks(a, nr, nc, C, T, S, labels, rgb, stitched);
     const bool px2 = (S % 2 == 0) && C <= 12 && ((uintptr_t)logits % 8 == 0) &&
                      (!stitched || (uintptr_t)stitched % 8 == 0) && (!labels || (uintptr_t)labels % 2 == 0) &&
                      (!rgb || (uintptr_t)rgb % 2 == 0) && (!confidence || (uintptr_t)confidence % 2 == 0);
@@ -594,41 +621,12 @@ static int stitch_launch(const float *logits, const float *const *tile_batches, 
     while (rows > 1 && rows * a.upr > kThreads * 8 && rows % 2 == 0) rows /= 2;
     a.rows_per_cta = rows;
     a.slabs = S / rows;
-    ColourLut lut;
-    if (lut_rgb) build_colour_lut(lut_rgb, C, &lut);
-    else for (int i = 0; i < PYLC_MAX_CLASSES; ++i) lut.rgb[i] = 0;
+    const ColourLut lut = stitch_lut(lut_rgb, C);
     const unsigned grid = (unsigned)((long long)a.nbx * a.nby * a.slabs);
     cudaStream_t st = (cudaStream_t)stream;
-    if (mode == PYLC_STITCH_MEAN) {
-        const float k = kLog2e / temperature;
-        if (confidence) launch_stitch<1, true>(px2, C, grid, st, a, lut, confidence, k);
-        else launch_stitch<1, false>(px2, C, grid, st, a, lut, nullptr, k);
-    } else {
-        if (confidence) launch_stitch<0, true>(px2, C, grid, st, a, lut, confidence, kLog2e);
-        else launch_stitch<0, false>(px2, C, grid, st, a, lut, nullptr, kLog2e);
-    }
-    return finish_launch();
-}
-
-extern "C" int pylc_stitch_argmax_colour(const float *logits, const float *const *tile_batches, int tiles_per_batch,
-                                         int nr, int nc, int C, int T, int S, const uint8_t *lut_rgb,
-                                         uint8_t *labels, uint8_t *rgb, float *stitched, pylc_stream_t stream) {
-    return stitch_launch(logits, tile_batches, tiles_per_batch, nr, nc, C, T, S, PYLC_STITCH_REFERENCE, lut_rgb, labels, rgb,
-                         nullptr, stitched, 1.f, stream);
-}
-
-extern "C" int pylc_stitch_probs(const float *logits, const float *const *tile_batches, int tiles_per_batch, int nr, int nc,
-                                 int C, int T, int S, int mode, const uint8_t *lut_rgb, uint8_t *labels, uint8_t *rgb,
-                                 uint8_t *confidence, float *stitched, pylc_stream_t stream) {
-    return stitch_launch(logits, tile_batches, tiles_per_batch, nr, nc, C, T, S, mode, lut_rgb, labels, rgb, confidence,
-                         stitched, 1.f, stream);
-}
-
-extern "C" int pylc_stitch_probs_t(const float *logits, const float *const *tile_batches, int tiles_per_batch, int nr, int nc,
-                                   int C, int T, int S, int mode, const uint8_t *lut_rgb, uint8_t *labels, uint8_t *rgb,
-                                   uint8_t *confidence, float *stitched, float temperature, pylc_stream_t stream) {
-    return stitch_launch(logits, tile_batches, tiles_per_batch, nr, nc, C, T, S, mode, lut_rgb, labels, rgb, confidence,
-                         stitched, temperature, stream);
+    return launch_mode(mode, confidence, temperature, [&](auto m, auto conf, float k) {
+        return launch_stitch<decltype(m)::value, decltype(conf)::value>(px2, C, grid, st, a, lut, confidence, k);
+    });
 }
 
 template <int MODE, bool CONF>
@@ -638,7 +636,7 @@ static int launch_stitch_up(int C, unsigned grid, size_t smem, cudaStream_t st, 
     do {                                                                                                                   \
         cudaError_t e = cudaFuncSetAttribute(stitch_up_kernel<CT, CM, MODE, CONF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
         if (e != cudaSuccess) return (int)e;                                                                               \
-        stitch_up_kernel<CT, CM, MODE, CONF><<<grid, kThreads, smem, st>>>(a, lut, conf, k);                                  \
+        stitch_up_kernel<CT, CM, MODE, CONF><<<grid, kThreads, smem, st>>>(a, lut, conf, k);                                     \
     } while (0)
     if (C == 9) LAUNCH_UP(9, 9);
     else if (C == 11) LAUNCH_UP(11, 11);
@@ -649,15 +647,12 @@ static int launch_stitch_up(int C, unsigned grid, size_t smem, cudaStream_t st, 
     return 0;
 }
 
-static int stitch_up_launch(const float *const *decoder_batches, int tiles_per_batch, int nr, int nc, int C, int T, int S,
-                            int hs, int ws, int mode, const uint8_t *lut_rgb, uint8_t *labels, uint8_t *rgb,
-                            uint8_t *confidence, float *stitched, float temperature, pylc_stream_t stream) {
-    if (!decoder_batches || tiles_per_batch < 1 || nr < 1 || nc < 1 || T < 1 || S < 1 || hs < 2 || ws < 2) return PYLC_ERR_ARG;
-    if (!temperature_ok(temperature, mode)) return PYLC_ERR_ARG;
-    if (rgb && !lut_rgb) return PYLC_ERR_ARG;
-    if (mode != PYLC_STITCH_REFERENCE && mode != PYLC_STITCH_MEAN) return PYLC_ERR_ARG;
-    if (C < 1 || C > PYLC_MAX_CLASSES) return PYLC_ERR_CLASSES;
-    if (!(S == T || 2 * S == T)) return PYLC_ERR_GEOMETRY;
+extern "C" int pylc_stitch_upsample_probs(const float *const *decoder_batches, int tiles_per_batch, int nr, int nc, int C,
+                                          int T, int S, int hs, int ws, int mode, const uint8_t *lut_rgb, uint8_t *labels,
+                                          uint8_t *rgb, uint8_t *confidence, float *stitched, float temperature,
+                                          pylc_stream_t stream) {
+    if (!decoder_batches || tiles_per_batch < 1 || hs < 2 || ws < 2) return PYLC_ERR_ARG;
+    if (int rc = check_stitch(nr, nc, C, T, S, mode, temperature, lut_rgb, rgb)) return rc;
     // this form covers the network's geometry: a x4 up-sample, rows of 2-pixel units that fill a CTA evenly
     if (C > kUpCpad || hs * 4 != T || ws * 4 != T || S % kUpR || (S / 2) > kThreads || kThreads % (S / 2) || (S & (S - 1))) return PYLC_ERR_GEOMETRY;
     if ((stitched && (uintptr_t)stitched % 8) || (labels && (uintptr_t)labels % 2) || (rgb && (uintptr_t)rgb % 2) ||
@@ -666,49 +661,15 @@ static int stitch_up_launch(const float *const *decoder_batches, int tiles_per_b
     StitchUpArgs a;
     a.batches = decoder_batches;
     a.tiles_per_batch = tiles_per_batch;
-    a.nr = nr; a.nc = nc; a.C = C; a.T = T; a.S = S; a.hs = hs; a.ws = ws;
-    a.overlap = S < T;
-    a.nbx = a.overlap ? nc + 1 : nc;
-    a.nby = a.overlap ? nr + 1 : nr;
-    a.h = a.nby * S;
-    a.w = a.nbx * S;
+    a.hs = hs; a.ws = ws;
+    set_blocks(a, nr, nc, C, T, S, labels, rgb, stitched);
     a.slabs = S / kUpR;
     a.cols_max = (int)((double)S * (ws - 1) / (T - 1)) + 4;
-    a.labels = labels; a.rgb = rgb; a.stitched = stitched;
-    ColourLut lut;
-    if (lut_rgb) build_colour_lut(lut_rgb, C, &lut);
-    else for (int i = 0; i < PYLC_MAX_CLASSES; ++i) lut.rgb[i] = 0;
+    const ColourLut lut = stitch_lut(lut_rgb, C);
     const size_t smem = (size_t)4 * kUpSrcRows * a.cols_max * kUpCpad * sizeof(float);
     const unsigned grid = (unsigned)((long long)a.nbx * a.nby * a.slabs);
     cudaStream_t st = (cudaStream_t)stream;
-    int rc;
-    const float k = kLog2e / temperature;           // exactly kLog2e at T = 1; unused in reference mode
-    if (mode == PYLC_STITCH_MEAN) rc = confidence ? launch_stitch_up<1, true>(C, grid, smem, st, a, lut, confidence, k)
-                                                  : launch_stitch_up<1, false>(C, grid, smem, st, a, lut, nullptr, k);
-    else rc = confidence ? launch_stitch_up<0, true>(C, grid, smem, st, a, lut, confidence, kLog2e)
-                         : launch_stitch_up<0, false>(C, grid, smem, st, a, lut, nullptr, kLog2e);
-    if (rc) return rc;
-    return finish_launch();
-}
-
-extern "C" int pylc_stitch_upsample_argmax_colour(const float *const *decoder_batches, int tiles_per_batch, int nr, int nc, int C,
-                                                  int T, int S, int hs, int ws, const uint8_t *lut_rgb, uint8_t *labels,
-                                                  uint8_t *rgb, float *stitched, pylc_stream_t stream) {
-    return stitch_up_launch(decoder_batches, tiles_per_batch, nr, nc, C, T, S, hs, ws, PYLC_STITCH_REFERENCE, lut_rgb, labels,
-                            rgb, nullptr, stitched, 1.f, stream);
-}
-
-extern "C" int pylc_stitch_upsample_probs(const float *const *decoder_batches, int tiles_per_batch, int nr, int nc, int C,
-                                          int T, int S, int hs, int ws, int mode, const uint8_t *lut_rgb, uint8_t *labels,
-                                          uint8_t *rgb, uint8_t *confidence, float *stitched, pylc_stream_t stream) {
-    return stitch_up_launch(decoder_batches, tiles_per_batch, nr, nc, C, T, S, hs, ws, mode, lut_rgb, labels, rgb, confidence,
-                            stitched, 1.f, stream);
-}
-
-extern "C" int pylc_stitch_upsample_probs_t(const float *const *decoder_batches, int tiles_per_batch, int nr, int nc, int C,
-                                            int T, int S, int hs, int ws, int mode, const uint8_t *lut_rgb, uint8_t *labels,
-                                            uint8_t *rgb, uint8_t *confidence, float *stitched, float temperature,
-                                            pylc_stream_t stream) {
-    return stitch_up_launch(decoder_batches, tiles_per_batch, nr, nc, C, T, S, hs, ws, mode, lut_rgb, labels, rgb, confidence,
-                            stitched, temperature, stream);
+    return launch_mode(mode, confidence, temperature, [&](auto m, auto conf, float k) {
+        return launch_stitch_up<decltype(m)::value, decltype(conf)::value>(C, grid, smem, st, a, lut, confidence, k);
+    });
 }

@@ -344,44 +344,6 @@ def _lut_for(lut_rgb, C, what):
     return pal
 
 
-def stitch_argmax_colour(logits, nr, nc, T, S, lut_rgb=None, want_labels=True, want_rgb=False,
-                         want_stitched=False, tiles_per_batch=None):
-    """pylc_stitch_argmax_colour.  `logits` is one contiguous CUDA [nr*nc,C,T,T] f32 tensor, or a list
-    of per-batch tensors [<=b,C,T,T] (the reference's `model_outputs` list).
-    Returns (labels [h,w] u8 | None, rgb [h,w,3] u8 | None, stitched [C,h,w] f32 | None)."""
-    lib = _lib.load()
-    lp, bp, tpb, C, dev, batch_table = _tile_source(logits, nr, nc, tiles_per_batch)
-    h, w = stitch_dims(nr, nc, T, S)
-    labels = torch.empty((h, w), dtype=torch.uint8, device=dev) if want_labels else None
-    rgb = torch.empty((h, w, 3), dtype=torch.uint8, device=dev) if want_rgb else None
-    stitched = torch.empty((C, h, w), dtype=torch.float32, device=dev) if want_stitched else None
-    pal = _lut_for(lut_rgb, C, "logits have")
-    check(lib.pylc_stitch_argmax_colour(lp, bp, tpb, nr, nc, C, T, S, pal, _p(labels), _p(rgb), _p(stitched),
-                                        _stream()), "pylc_stitch_argmax_colour")
-    if batch_table is not None:
-        batch_table.record_stream(torch.cuda.current_stream())
-    return labels, rgb, stitched
-
-
-def stitch_upsample_argmax_colour(decoder_batches, nr, nc, T, S, lut_rgb=None, want_labels=True, want_rgb=False,
-                                  want_stitched=False, tiles_per_batch=None):
-    """pylc_stitch_upsample_argmax_colour: stitch straight from the decoder's channels-last outputs
-    [b, C, T/4, T/4] (one tensor per network batch), the final x4 bilinear up-sample evaluated in the kernel.
-    Returns (labels [h,w] u8, rgb [h,w,3] u8 or None, stitched [C,h,w] f32 or None), bit-identical to
-    stitch_argmax_colour(upsample_nhwc_to_nchw(batch) ...)."""
-    lib = _lib.load()
-    batch_table, tpb, C, hs, ws, dev = _decoder_source(decoder_batches, nr, nc, tiles_per_batch)
-    h, w = stitch_dims(nr, nc, T, S)
-    labels = torch.empty((h, w), dtype=torch.uint8, device=dev) if want_labels else None
-    rgb = torch.empty((h, w, 3), dtype=torch.uint8, device=dev) if want_rgb else None
-    stitched = torch.empty((C, h, w), dtype=torch.float32, device=dev) if want_stitched else None
-    pal = _lut_for(lut_rgb, C, "the decoder output has")
-    check(lib.pylc_stitch_upsample_argmax_colour(_p(batch_table), tpb, nr, nc, C, T, S, hs, ws, pal, _p(labels), _p(rgb),
-                                                 _p(stitched), _stream()), "pylc_stitch_upsample_argmax_colour")
-    batch_table.record_stream(torch.cuda.current_stream())
-    return labels, rgb, stitched
-
-
 STITCH_MODES = {"reference": 0, "mean": 1}     # PYLC_STITCH_REFERENCE, PYLC_STITCH_MEAN
 
 
@@ -406,12 +368,12 @@ def _prob_outputs(C, h, w, dev, want_labels, want_rgb, want_confidence, want_pro
 
 def stitch_probs(logits, nr, nc, T, S, mode="reference", lut_rgb=None, want_labels=True, want_rgb=False,
                  want_confidence=True, want_probs=False, tiles_per_batch=None, out=None, temperature=1.0):
-    """pylc_stitch_probs_t: the stitch of stitch_argmax_colour with per-pixel probabilities.
-    P = the mean over the covering tiles of their softmaxes.  mode "reference": labels / rgb are those of
-    stitch_argmax_colour and `probs` is the reference's merged map M; mode "mean": labels = argmax P and
-    `probs` = P.  `confidence` is the u8 plane round(P[label] * 255) in both modes.
-    `temperature` (mean mode only; PylcError otherwise unless 1): every tile softmax is softmax(L / temperature);
-    1 gives the untempered outputs bit for bit.
+    """pylc_stitch_probs.  `logits` is one contiguous CUDA [nr*nc,C,T,T] f32 tensor, or a list of per-batch tensors
+    [<=b,C,T,T] (the reference's `model_outputs` list).
+    P = the mean over the covering tiles of their softmaxes.  mode "reference": labels / rgb are the reference's
+    and `probs` is its merged map M; mode "mean": labels = argmax P and `probs` = P.  `confidence` is the u8 plane
+    round(P[label] * 255) in both modes.
+    `temperature` (mean mode only; PylcError otherwise unless 1): every tile softmax is softmax(L / temperature).
     `out`: optional dict of preallocated outputs (any of labels / rgb / confidence / probs).
     Returns dict(labels, rgb, confidence, probs), entries None where not wanted."""
     lib = _lib.load()
@@ -420,9 +382,9 @@ def stitch_probs(logits, nr, nc, T, S, mode="reference", lut_rgb=None, want_labe
     h, w = stitch_dims(nr, nc, T, S)
     res = _prob_outputs(C, h, w, dev, want_labels, want_rgb, want_confidence, want_probs, out)
     pal = _lut_for(lut_rgb, C, "logits have")
-    check(lib.pylc_stitch_probs_t(lp, bp, tpb, nr, nc, C, T, S, m, pal, _p(res["labels"]), _p(res["rgb"]),
-                                  _p(res["confidence"]), _p(res["probs"]), float(temperature), _stream()),
-          "pylc_stitch_probs_t")
+    check(lib.pylc_stitch_probs(lp, bp, tpb, nr, nc, C, T, S, m, pal, _p(res["labels"]), _p(res["rgb"]),
+                                _p(res["confidence"]), _p(res["probs"]), float(temperature), _stream()),
+          "pylc_stitch_probs")
     if batch_table is not None:
         batch_table.record_stream(torch.cuda.current_stream())
     return res
@@ -431,8 +393,8 @@ def stitch_probs(logits, nr, nc, T, S, mode="reference", lut_rgb=None, want_labe
 def stitch_upsample_probs(decoder_batches, nr, nc, T, S, mode="reference", lut_rgb=None, want_labels=True,
                           want_rgb=False, want_confidence=True, want_probs=False, tiles_per_batch=None, out=None,
                           temperature=1.0):
-    """pylc_stitch_upsample_probs_t: stitch_probs straight from the decoder's channels-last outputs (the fused
-    x4 up-sample of stitch_upsample_argmax_colour), bit-identical to
+    """pylc_stitch_upsample_probs: stitch_probs straight from the decoder's channels-last outputs [b, C, T/4, T/4]
+    (one tensor per network batch), the final x4 bilinear up-sample evaluated in the kernel.  Bit-identical to
     stitch_probs(upsample_nhwc_to_nchw(batch) ..., temperature=...).  Returns dict(labels, rgb, confidence, probs)."""
     lib = _lib.load()
     m = _stitch_mode(mode)
@@ -440,11 +402,31 @@ def stitch_upsample_probs(decoder_batches, nr, nc, T, S, mode="reference", lut_r
     h, w = stitch_dims(nr, nc, T, S)
     res = _prob_outputs(C, h, w, dev, want_labels, want_rgb, want_confidence, want_probs, out)
     pal = _lut_for(lut_rgb, C, "the decoder output has")
-    check(lib.pylc_stitch_upsample_probs_t(_p(batch_table), tpb, nr, nc, C, T, S, hs, ws, m, pal, _p(res["labels"]),
-                                           _p(res["rgb"]), _p(res["confidence"]), _p(res["probs"]), float(temperature),
-                                           _stream()), "pylc_stitch_upsample_probs_t")
+    check(lib.pylc_stitch_upsample_probs(_p(batch_table), tpb, nr, nc, C, T, S, hs, ws, m, pal, _p(res["labels"]),
+                                         _p(res["rgb"]), _p(res["confidence"]), _p(res["probs"]), float(temperature),
+                                         _stream()), "pylc_stitch_upsample_probs")
     batch_table.record_stream(torch.cuda.current_stream())
     return res
+
+
+def stitch_argmax_colour(logits, nr, nc, T, S, lut_rgb=None, want_labels=True, want_rgb=False,
+                         want_stitched=False, tiles_per_batch=None):
+    """The reference's stitch (tools.reconstruct up to colourize): stitch_probs in reference mode without confidence.
+    Returns (labels [h,w] u8 | None, rgb [h,w,3] u8 | None, stitched [C,h,w] f32 | None)."""
+    r = stitch_probs(logits, nr, nc, T, S, lut_rgb=lut_rgb, want_labels=want_labels, want_rgb=want_rgb,
+                     want_confidence=False, want_probs=want_stitched, tiles_per_batch=tiles_per_batch)
+    return r["labels"], r["rgb"], r["probs"]
+
+
+def stitch_upsample_argmax_colour(decoder_batches, nr, nc, T, S, lut_rgb=None, want_labels=True, want_rgb=False,
+                                  want_stitched=False, tiles_per_batch=None):
+    """stitch_argmax_colour straight from the decoder's channels-last outputs (stitch_upsample_probs in reference mode
+    without confidence).  Returns (labels, rgb, stitched) as stitch_argmax_colour, bit-identical to
+    stitch_argmax_colour(upsample_nhwc_to_nchw(batch) ...)."""
+    r = stitch_upsample_probs(decoder_batches, nr, nc, T, S, lut_rgb=lut_rgb, want_labels=want_labels,
+                              want_rgb=want_rgb, want_confidence=False, want_probs=want_stitched,
+                              tiles_per_batch=tiles_per_batch)
+    return r["labels"], r["rgb"], r["probs"]
 
 
 def stitch_upsample_supported(C, T, S, hs, ws):

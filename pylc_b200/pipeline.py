@@ -12,10 +12,10 @@ Here, per image (device_fit, the default whenever OpenCV's general area filter a
     GPU    pylc_fit_resize_area_u8       cv2.resize(INTER_AREA) of adjust_to_tile, bit-exact (1 launch)
            pylc_tile_gather_norm_f32     tiles, normalised, grayscale replicated   (1 launch)
            DeepLabv3+/ResNet-101         stock PyTorch / cuDNN, batches of `batch_tiles`
-           pylc_stitch_argmax_colour     logits -> label map, reference band semantics (1 launch)
+           pylc_stitch_probs             logits -> label map, reference band semantics (1 launch)
            pylc_resample_encode_confusion  NN resample + GT encode + [C,C] counts    (1 launch)
-With `stitch="mean"` or `confidence=True` the stitch is pylc_stitch_probs / pylc_stitch_upsample_probs
-instead: labels from the mean of the covering tiles' softmaxes ("mean") and / or the u8 confidence plane
+With `stitch="mean"` or `confidence=True` the same stitch (pylc_stitch_probs / pylc_stitch_upsample_probs)
+gives instead: labels from the mean of the covering tiles' softmaxes ("mean") and / or the u8 confidence plane
 of that mean; with keep_masks the plane is also resampled to full resolution (pylc_confidence_resample).
     D2H    nothing per image; the [C,C] i64 matrix (and optional masks) at the end
 With `scales` (multi-scale inference, mean stitch only) every image is segmented once per scale s_k: the decoded
@@ -24,7 +24,7 @@ area filter, otherwise with cv2 on the host threads.  Each member's mean-mode pr
 device; pylc_multiscale_combine samples every P_k onto the full-resolution grid, averages them and writes the
 full-resolution labels and confidence, and pylc_resample_encode_confusion counts the confusion from those.
 With `temperature` T (post-hoc calibration, mean stitch only) every tile softmax of the mean stitch is softmax(L / T),
-in the single-scale stitch and in every multi-scale member alike (pylc_stitch_probs_t).
+in the single-scale stitch and in every multi-scale member alike.
 With device_fit off (or for geometries OpenCV resizes with another filter) the fit-resize runs on
 host worker threads with cv2 itself and the fitted image is uploaded instead.
 Logits never leave the device.  Images are independent, so data-parallel ranks take images
@@ -302,7 +302,7 @@ class TiledSegmenter(object):
         return nr * nc * (per_tile // 16 if self.fuse_upsample else per_tile)
 
     def stitch_output(self, src, nr, nc, temperature=None, **kw):
-        """pylc_stitch_probs_t (or its fused up-sample form) of a network_output at `temperature` (default: the
+        """pylc_stitch_probs (or its fused up-sample form) of a network_output at `temperature` (default: the
         segmenter's)."""
         probs = ops.stitch_upsample_probs if self.fuse_upsample else ops.stitch_probs
         t = self.temperature if temperature is None else temperature
@@ -325,17 +325,15 @@ class TiledSegmenter(object):
         if self.scales is not None:
             return self._segment_multiscale(f, inject)
         tiles, nr, nc = self.fitted_tiles(f)
+        src = self.network_output(tiles)
         conf_fit = None
         if self.stitch != "reference" or self.confidence:
-            out = self._stitch_probs(tiles, nr, nc, want_confidence=self.confidence)
+            out = self.stitch_output(src, nr, nc, want_confidence=self.confidence)
             labels, conf_fit = out["labels"], out["confidence"]
-        elif self.fuse_upsample:
-            dec = self.forward_tiles(tiles, s2d=self.s2d, decoder_only=True)
-            labels, _, _ = ops.stitch_upsample_argmax_colour(dec, nr, nc, self.T, self.S, tiles_per_batch=self.batch_tiles)
         else:
-            logits = self.forward_tiles(tiles, s2d=self.s2d)
-            labels, _, _ = ops.stitch_argmax_colour(logits if len(logits) > 1 else logits[0], nr, nc, self.T, self.S,
-                                                    tiles_per_batch=self.batch_tiles)
+            # looked up on `ops` at call time, so that a wrapper installed there (bench.py's kernel timer) sees it
+            stitch = ops.stitch_upsample_argmax_colour if self.fuse_upsample else ops.stitch_argmax_colour
+            labels = stitch(src, nr, nc, self.T, self.S, tiles_per_batch=self.batch_tiles)[0]
         n_inject = self.n_inject if inject is None else inject
         res = ops.resample_encode_confusion(
             labels, f.w_full, f.h_full, gt_rgb=f.gt, gt_pitch=f.gt_pitch, palette=self.palette, lut_rgb=self.lut,

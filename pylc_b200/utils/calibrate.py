@@ -5,7 +5,7 @@ negative log-likelihood of the full-resolution ground truth on labelled images.
 
 The network is almost all of a segmentation step, so each image's network output is computed once and kept on the
 device (TiledSegmenter.network_output: the logit batches, or the decoder batches on the fused route); every
-evaluation of the objective re-runs only the tempered stitch (pylc_stitch_probs_t) and the score reduction
+evaluation of the objective re-runs only the tempered stitch (pylc_stitch_probs) and the score reduction
 (pylc_prob_scores), through the same TiledSegmenter.stitch_output that `pylc test` runs.
 
 Search, over u = ln T, of f(u) = sum_images nll_sum(T = exp(u)) / sum_images n_px (the kernels receive f32(exp(u))):

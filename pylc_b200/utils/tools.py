@@ -6,7 +6,7 @@ per-pixel body replaced by an sm_100a kernel call through the C ABI (pylc_b200.o
     get_image / adjust_to_tile   host (OpenCV decode + INTER_AREA fit), reference tools.py:77-206
     class_encode                 pylc_class_encode,            reference tools.py:412-449
     colourize                    pylc_colourise_u8,            reference tools.py:322-358
-    reconstruct                  pylc_stitch_argmax_colour +
+    reconstruct                  pylc_stitch_probs +
                                  pylc_resample_encode_confusion, reference tools.py:209-319
     coshuffle / collate / load_files / mk_path / confirm_write_file   host, unchanged semantics
 

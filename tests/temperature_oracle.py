@@ -1,4 +1,4 @@
-"""CPU oracle (float64) of temperature scaling for the mean stitch: pylc_stitch_probs_t, pylc_prob_scores and the
+"""CPU oracle (float64) of temperature scaling for the mean stitch: pylc_stitch_probs, pylc_prob_scores and the
 temperature search of pylc_b200/utils/calibrate.py, each written from its definition."""
 import math
 

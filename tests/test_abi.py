@@ -26,7 +26,7 @@ def lib():
 
 def test_header_declares_something():
     syms = declared_symbols()
-    assert len(syms) >= 15 and "pylc_stitch_argmax_colour" in syms
+    assert len(syms) >= 15 and "pylc_stitch_probs" in syms
 
 
 def test_every_declared_symbol_is_exported_and_bound(lib):

@@ -113,7 +113,8 @@ def test_stitch_probs_argument_errors(ops):
         ops.stitch_probs(tiles, 2, 2, 32, 16, mode="max")
     lib = ops._lib.load()
     lab = torch.empty((48, 48), dtype=torch.uint8, device="cuda")
-    rc = lib.pylc_stitch_probs(ops._p(tiles), None, 4, 2, 2, 9, 32, 16, 2, None, ops._p(lab), None, None, None, None)
+    rc = lib.pylc_stitch_probs(ops._p(tiles), None, 4, 2, 2, 9, 32, 16, 2, None, ops._p(lab), None, None, None, 1.0,
+                               None)
     assert rc == -1                                           # PYLC_ERR_ARG: unknown mode
 
 

@@ -1,4 +1,4 @@
-"""Temperature scaling of the mean stitch on the GPU (pylc_stitch_probs_t, pylc_stitch_upsample_probs_t,
+"""Temperature scaling of the mean stitch on the GPU (pylc_stitch_probs, pylc_stitch_upsample_probs,
 pylc_prob_scores, utils/calibrate.py) against the f64 oracle in tests/temperature_oracle.py, through the pipeline and
 the command line."""
 import glob
@@ -43,28 +43,27 @@ def _outputs(ops, C, h, w):
             "probs": torch.empty((C, h, w), dtype=torch.float32, device="cuda")}
 
 
-def _raw_stitch(ops, src, nr, nc, T, S, mode, temperature=None):
-    """One call of pylc_stitch_probs (temperature None) or pylc_stitch_probs_t, outputs allocated here."""
+def _raw_stitch(ops, src, nr, nc, T, S, mode, temperature):
+    """One call of pylc_stitch_probs, outputs allocated here."""
     lib = ops._lib.load()
     lp, bp, tpb, C, _, table = ops._tile_source(src, nr, nc, None)
     h, w = ops.stitch_dims(nr, nc, T, S)
     out = _outputs(ops, C, h, w)
     args = [lp, bp, tpb, nr, nc, C, T, S, mode, None, ops._p(out["labels"]), None, ops._p(out["confidence"]),
-            ops._p(out["probs"])]
-    rc = lib.pylc_stitch_probs(*args, None) if temperature is None else lib.pylc_stitch_probs_t(*args, temperature, None)
+            ops._p(out["probs"]), temperature, None]
+    rc = lib.pylc_stitch_probs(*args)
     torch.cuda.synchronize()
     return rc, out
 
 
-def _raw_stitch_up(ops, dec, nr, nc, T, S, mode, temperature=None):
+def _raw_stitch_up(ops, dec, nr, nc, T, S, mode, temperature):
     lib = ops._lib.load()
     table, tpb, C, hs, ws, _ = ops._decoder_source(dec, nr, nc, None)
     h, w = ops.stitch_dims(nr, nc, T, S)
     out = _outputs(ops, C, h, w)
     args = [ops._p(table), tpb, nr, nc, C, T, S, hs, ws, mode, None, ops._p(out["labels"]), None,
-            ops._p(out["confidence"]), ops._p(out["probs"])]
-    rc = lib.pylc_stitch_upsample_probs(*args, None) if temperature is None \
-        else lib.pylc_stitch_upsample_probs_t(*args, temperature, None)
+            ops._p(out["confidence"]), ops._p(out["probs"]), temperature, None]
+    rc = lib.pylc_stitch_upsample_probs(*args)
     torch.cuda.synchronize()
     return rc, out
 
@@ -79,26 +78,7 @@ def _decoder(C, nr, nc, T, seed):
     return [d.contiguous(memory_format=torch.channels_last)]
 
 
-# ---- 1. T = 1 anchors ------------------------------------------------------------------------------------------
-
-@pytest.mark.parametrize("C,nr,nc,T,S", GEOMS)
-def test_tempered_entry_points_at_one_equal_the_untempered_ones(ops, C, nr, nc, T, S):
-    src = torch.from_numpy(_tiles(C, nr, nc, T, C * 100 + nr * 10 + nc)).cuda()
-    for mode in (0, 1):
-        rc0, a = _raw_stitch(ops, src, nr, nc, T, S, mode)
-        rc1, b = _raw_stitch(ops, src, nr, nc, T, S, mode, 1.0)
-        assert rc0 == rc1 == 0 and _same(a, b), mode
-
-
-@pytest.mark.parametrize("C,S", [(4, 32), (9, 32), (11, 32), (12, 32), (9, 64)])
-def test_fused_tempered_entry_point_at_one_equals_the_untempered_one(ops, C, S):
-    nr, nc, T = 2, 3, 64
-    dec = _decoder(C, nr, nc, T, C + S)
-    for mode in (0, 1):
-        rc0, a = _raw_stitch_up(ops, dec, nr, nc, T, S, mode)
-        rc1, b = _raw_stitch_up(ops, dec, nr, nc, T, S, mode, 1.0)
-        assert rc0 == rc1 == 0 and _same(a, b), mode
-
+# ---- 1. argument errors ------------------------------------------------------------------------------------------
 
 def test_temperature_argument_errors(ops):
     from pylc_b200._lib import PylcError
